@@ -4,6 +4,7 @@
 Contract (see the task prompt / BASELINE.json):
   python bench.py --gpus N --steps K --warmup W            (N>1: launched under torch.distributed.run)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py ... --dump-outputs DIR   also writes the results of the last timed step as DIR/<name>.npy
 
 A "step" is one pass of the hot path (lm_detect_batch through the C ABI) over one batch of synthetic
 frames: SURVEY config 2 = 10 000 raw 400x1700 u8 frames per GPU, resident in HBM, six random-init
@@ -41,6 +42,32 @@ UNIT = "frames/s"
 FRAMES_PER_STEP = 10_000
 WORKLOAD = ("configs[1]: LocoMouse_TM batched detection, 10k synthetic 400x1700 u8 frames per GPU resident in HBM, "
             "six random-init 30x30 templates")
+# --dump-outputs writes the results of this many frames, drawn with a fixed seed: about 11 kB per frame in the dumped
+# dtypes, 45 MB in all (the full 10k-frame result set would be 110 MB)
+DUMP_FRAMES = 4096
+DUMP_SEED = 0
+
+
+def dump_outputs(res, out_dir: str) -> None:
+    """Writes every array of `res` (the Results of one detect_batch call) for a seeded sample of its frames as
+    out_dir/<name>.npy: integer fields as float32 (coordinates, counts and flags are far below 2**24, so exactly),
+    scores as float64; the candidate records are split into <name>_x, <name>_y, <name>_s.  frame_index.npy holds the
+    sampled frame numbers."""
+    from locomouse_cpp_b200.types import CAND_DTYPE
+
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(res.n, min(res.n, DUMP_FRAMES), replace=False))
+    out = {"frame_index": idx.astype(np.float64)}
+    for name in res.ARRAYS:
+        a = getattr(res, name)[idx]
+        if a.dtype == CAND_DTYPE:
+            out.update({f"{name}_x": a["x"].astype(np.float32), f"{name}_y": a["y"].astype(np.float32), f"{name}_s": a["s"].copy()})
+        elif a.dtype == np.float64:
+            out[name] = a
+        else:
+            out[name] = a.astype(np.float32)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def algorithmic_fma_per_frame(cfg, model) -> float:
@@ -126,8 +153,10 @@ def run_reference(args):
         oracle.detect(cfg, model, bkg, calib, frames, bx, bs, bb, n_threads=threads)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oracle.detect(cfg, model, bkg, calib, frames, bx, bs, bb, n_threads=threads)
+        out = oracle.detect(cfg, model, bkg, calib, frames, bx, bs, bb, n_threads=threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(out, args.dump_outputs)
     v = per_step * args.steps / dt
     sample = f"{per_step} frames/step of the same synthetic workload (first frames of video 0), {threads} threads"
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -144,6 +173,7 @@ def run_reference(args):
 
 # ---------------------------------------------------------------------------------------------------
 def main():
+    sys.dont_write_bytecode = True   # the benchmark may run from a read-only tree and leaves nothing in it
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=5)
@@ -157,7 +187,14 @@ def main():
     ap.add_argument("--nccl-gather", action="store_true", help="N > 1: move the result records to rank 0 with an NCCL gather instead of shared host memory")
     ap.add_argument("--even-shards", action="store_true", help="N > 1: keep the end-to-end job evenly split even when the ranks' measured host rates differ")
     ap.add_argument("--opt", action="append", default=[], metavar="NAME=VALUE", help="library option for the measured arm (lm_set_option), e.g. streams=3")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help=f"write the results of the last timed step (all ranks' frames; a seeded sample of {DUMP_FRAMES} of them) "
+                         "as DIR/<name>.npy in float32 / float64.  With --impl reference the dump holds the oracle's results "
+                         "for that arm's own frames (their number depends on the host's thread count), so it compares only "
+                         "with reference-arm dumps from hosts with as many threads")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -233,6 +270,11 @@ def main():
     dev_ms = max_over_ranks(dev_total)
     value = world * n * args.steps / wall
     overflow = int((res.flags != 0).sum())
+    if args.dump_outputs:   # before the passes below reuse `res`
+        parts = sharding.gather_to_rank0(res, device=dev) if world > 1 else [res]
+        if rank == 0:
+            dump_outputs(sharding.concat(parts) if world > 1 else res, args.dump_outputs)
+        barrier()
 
     # ---- instrumented pass: per-kernel device times --------------------------------------------------------------
     # In the timed loop above consecutive sub-batches overlap on two streams, so a kernel's event-to-event time there

@@ -4,6 +4,7 @@ shim in oracle/ref_shim.  TEST INFRASTRUCTURE ONLY (tests/ and the golden-vector
 from __future__ import annotations
 
 import ctypes as C
+import json
 import os
 import subprocess
 
@@ -11,15 +12,36 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "_ref", "libref_nms.so")
-REF_ROOT = "/root/reference"
+
+
+def _ref_root() -> str:
+    """The careylab/LocoMouse_cpp checkout: LOCOMOUSE_CPP_REFERENCE if set, else BASELINE.json's reference_path.  Where
+    there is none, the checks against the reference's own code skip and the committed golden vectors under tests/golden/
+    stand in for it."""
+    env = os.environ.get("LOCOMOUSE_CPP_REFERENCE")
+    if env:
+        return env
+    with open(os.path.join(_HERE, "..", "BASELINE.json")) as f:
+        return json.load(f)["reference_path"]
+
+
+REF_ROOT = _ref_root()
 CAND = np.dtype([("x", "<i4"), ("y", "<i4"), ("s", "<f8")])
 _lib = None
 
 
+def make_ref() -> None:
+    """Builds oracle/_ref/ from the checkout at REF_ROOT (`make -C oracle ref REF=...`); raises with make's output if
+    that fails."""
+    p = subprocess.run(["make", "-C", _HERE, "ref", f"REF={REF_ROOT}"], capture_output=True, text=True)
+    if p.returncode != 0:
+        raise RuntimeError(f"building oracle/_ref/ from {REF_ROOT} failed:\n{p.stdout[-2000:]}\n{p.stderr[-2000:]}")
+
+
 def available(build: bool = True) -> bool:
-    """True when the library exists (it is built here, where /root/reference is mounted, and travels to the GPU box)."""
-    if not os.path.exists(LIB_PATH) and build and os.path.isdir(REF_ROOT):
-        subprocess.run(["make", "-C", _HERE, "ref"], capture_output=True)
+    """True when the library exists (built from REF_ROOT on demand)."""
+    if not os.path.exists(LIB_PATH) and build and os.path.isdir(os.path.join(REF_ROOT, "LocoMouse_Core")):
+        make_ref()
     return os.path.exists(LIB_PATH)
 
 
@@ -27,7 +49,7 @@ def lib():
     global _lib
     if _lib is None:
         if not available():
-            raise RuntimeError("oracle/_ref/libref_nms.so is missing and /root/reference is not mounted")
+            raise RuntimeError(f"oracle/_ref/libref_nms.so is missing and there is no LocoMouse_cpp checkout at {REF_ROOT}")
         L = C.CDLL(LIB_PATH)
         f32p = C.POINTER(C.c_float)
         L.ref_nms_max.restype = C.c_int

@@ -84,7 +84,7 @@ def test_side_view_transitions_equal_reference_golden():
 def test_side_view_transitions_equal_reference_fresh():
     R = _ref_nms()
     if R is None:
-        pytest.skip("reference library not built (no /root/reference on this machine); golden vectors cover it")
+        pytest.skip("reference library not built (no LocoMouse_cpp checkout, see oracle/reference_nms.py); golden vectors cover it")
     H = _host()
     for c in side_cases(seed=123, n=150):
         assert _same(_side(H, "lmh_pairwise_potential_side", c), _side(R, "ref_pairwise_potential_side", c))

@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 
 from locomouse_cpp_b200.types import pairwise_params, location_priors
-from oracle import oracle
+from oracle import oracle, reference_nms
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
@@ -30,9 +30,8 @@ def _host():
 
 def _ref():
     if not os.path.exists(REF_LIB):
-        if os.path.isdir("/root/reference/match2nd"):
-            import subprocess
-            subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "ref"], check=True, capture_output=True)
+        if os.path.isdir(os.path.join(reference_nms.REF_ROOT, "match2nd")):
+            reference_nms.make_ref()
         else:
             return None
     return C.CDLL(REF_LIB)
@@ -160,7 +159,7 @@ def golden_cases():
 
 def make_golden():
     R = _ref()
-    assert R is not None, "needs /root/reference"
+    assert R is not None, "needs a LocoMouse_cpp checkout (see oracle/reference_nms.py)"
     out = {}
     for i, (T, perm, occ_cost, bam) in enumerate(golden_cases()):
         lab = run(R, "ref_match2nd", T, occ_cost, bam, perm)
@@ -191,7 +190,7 @@ def test_tracker_equals_reference_golden_vectors():
 def test_tracker_equals_reference_on_fresh_trellises():
     R = _ref()
     if R is None:
-        pytest.skip("reference library not built (no /root/reference on this machine); golden vectors cover it")
+        pytest.skip("reference library not built (no LocoMouse_cpp checkout, see oracle/reference_nms.py); golden vectors cover it")
     H = _host()
     rng = np.random.Generator(np.random.PCG64(99))
     for it in range(150):

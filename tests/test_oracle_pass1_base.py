@@ -68,7 +68,7 @@ def test_oracle_equals_reference_golden():
 
 def test_oracle_equals_reference_fresh():
     if not ref.available():
-        pytest.skip("reference library not built (no /root/reference on this machine); golden vectors cover it")
+        pytest.skip("reference library not built (no LocoMouse_cpp checkout, see oracle/reference_nms.py); golden vectors cover it")
     spec, cfg, bkg, calib, frames, imgs = _images(n=3, seed=1003, flip=True)
     side, bottom = _views(cfg, spec)
     for th, k, conn in ((1, 11, 8), (0, 5, 4), (3, 11, 4)):

@@ -55,7 +55,7 @@ def check(got, bbx_ref, st_ref):
     assert bbx == bbx_ref
 
 
-@pytest.mark.skipif(not reference_nms.available(), reason="/root/reference not mounted: committed vectors only")
+@pytest.mark.skipif(not reference_nms.available(), reason="no LocoMouse_cpp checkout (see oracle/reference_nms.py): committed vectors only")
 def test_oracle_equals_reference_compiled_code_stage_by_stage():
     rng = np.random.default_rng(77)
     for i, (kind, conn, min_count, min_vis, as_float) in enumerate(CASES * 2):
