@@ -529,11 +529,7 @@ int prepare(lm_ctx *ctx, int want_B = 0, int want_sets = 0) {
     if ((rc = dalloc(ctx, &b.cc_flag, B))) return rc;
     if ((rc = dalloc(ctx, &b.det, B * 4 * (size_t)k.det_cap))) return rc;
     if ((rc = dalloc(ctx, &b.det_count, B * 4))) return rc;
-    {
-        size_t P = 2;
-        while (P < (size_t)k.det_cap) P <<= 1;
-        if ((rc = dalloc(ctx, &b.nms_scratch, B * 2 * P * 16))) return rc;
-    }
+    if ((rc = dalloc(ctx, &b.nms_scratch, B * 2 * lm_nms_scratch_bytes(k.det_cap)))) return rc;
     for (int s = 0; s < lm_ctx::NRES; ++s)
         if ((rc = dalloc(ctx, &ctx->d_bb[s], 3 * B))) return rc;
     // results: one device block + two pinned host blocks, same sub-array order
@@ -589,11 +585,7 @@ int prepare(lm_ctx *ctx, int want_B = 0, int want_sets = 0) {
         if ((rc = dalloc(ctx, &c.cc_flag, B))) return rc;
         if ((rc = dalloc(ctx, &c.det, B * 4 * (size_t)k.det_cap))) return rc;
         if ((rc = dalloc(ctx, &c.det_count, B * 4))) return rc;
-        {
-            size_t P = 2;
-            while (P < (size_t)k.det_cap) P <<= 1;
-            if ((rc = dalloc(ctx, &c.nms_scratch, B * 2 * P * 16))) return rc;
-        }
+        if ((rc = dalloc(ctx, &c.nms_scratch, B * 2 * lm_nms_scratch_bytes(k.det_cap)))) return rc;
         if ((rc = bind_results(c, set))) return rc;
         if (b.scr.enabled) {
             if ((rc = dalloc(ctx, &c.scr.ntasks, 16))) return rc;

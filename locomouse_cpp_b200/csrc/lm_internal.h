@@ -106,7 +106,7 @@ struct LmBatch {
     int bb_w, bb_h[2], tail_w, tail_pitch;
     int flip, imadjust, conn, n_tail_points, fma_mode;
     int cand_cap, det_cap, match_cap;
-    unsigned char *nms_scratch;  // device, [2 B lists][16 * pow2(det_cap)] bytes: lists too long for the shared-memory NMS class
+    unsigned char *nms_scratch;  // device, [2 B lists][lm_nms_scratch_bytes(det_cap)]: lists too long for the NMS kernels' shared memory
     int ovlp[2];                // (int)(w_bottom * (1 - T)) per feature (class.cpp:1047), host computed
     LmView view[2];
     LmTemplateDev tmpl[2][3];
@@ -144,6 +144,8 @@ int lm_launch_fold_calib(const int32_t *calib, const uint8_t *bkg, int n_rows, i
 int lm_launch_corr(const LmBatch &b, cudaStream_t s);
 int lm_launch_tail(const LmBatch &b, cudaStream_t s);
 int lm_launch_nms(const LmBatch &b, cudaStream_t s);
+// bytes of nms_scratch per list: 8 + 8 + 4 bytes per entry (two key arrays, one link array), 16-byte aligned slices
+__host__ __device__ inline size_t lm_nms_scratch_bytes(int det_cap) { return ((size_t)det_cap * 20 + 15) & ~(size_t)15; }
 int lm_launch_pair(const LmBatch &b, cudaStream_t s);
 int lm_launch_bbox_tm_de(const LmBatch &b, const lm_bb_de_params &p, uint32_t *hist, uint8_t *pred, double *bb_x, int32_t *lims,
                          cudaStream_t s, uint8_t *diff = nullptr);
