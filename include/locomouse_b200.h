@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define LM_ABI_VERSION 5  /* 5: lm_bounding_box_tm; 4: lm_bounding_box_base, lm_mouse_box_size; 2: lm_set_option, lm_get_info, lm_debug_nms, lm_bounding_box_tm_de, lm_moving_average; 3: lm_host_alloc / lm_host_free, lm_unary_costs / lm_pairwise_costs, options streams 1..4, screen_layout, screen_priority */
+#define LM_ABI_VERSION 5  /* 5: lm_bounding_box_tm, and (backward compatible additions) lm_decode_png, lm_device_alloc / lm_device_free, lm_get_info("ms_decode"); 4: lm_bounding_box_base, lm_mouse_box_size; 2: lm_set_option, lm_get_info, lm_debug_nms, lm_bounding_box_tm_de, lm_moving_average; 3: lm_host_alloc / lm_host_free, lm_unary_costs / lm_pairwise_costs, options streams 1..4, screen_layout, screen_priority */
 
 /* feature / view indices used in every [2] / [3] array below */
 enum { LM_PAW = 0, LM_SNOUT = 1, LM_TAIL = 2 };
@@ -294,6 +294,18 @@ int lm_pairwise_costs(lm_ctx *ctx, const lm_results *res, int64_t n, int32_t fea
  * members of LocoMouse, LocoMouse_class.hpp:188-236; a binding backs those with this memory or accepts the copy.) */
 int lm_host_alloc(void **ptr, size_t bytes);
 int lm_host_free(void *ptr);
+
+/* compressed video ------------------------------------------------------------------------------------------------------ *
+ * PNG-coded AVI frames (fourcc 'MPNG' / 'png '): payload holds n complete PNG files, frame i = payload[offsets[i], offsets[i+1]),
+ * offsets on the host; payload in host (pageable or page-locked) or device memory.  frames: device memory,
+ * [n][vid_rows][vid_cols] of the configured geometry.  LM_ERR_INVALID names the first bad frame and why.
+ * Each frame must be 8-bit grey, RGB or RGBA, not interlaced, of the configured size; the output is channel 0 of the frame
+ * cv::VideoCapture delivers (grey, or blue), decoded on the device (inflate + the five row filters; checksums are not
+ * verified).  Host payloads are copied in pieces on the copy stream, overlapped with the decode of the previous piece.
+ * Needs lm_configure only.  lm_get_info("ms_decode"): device ms of the decode kernels in the last call. */
+int lm_decode_png(lm_ctx *ctx, const uint8_t *payload, int payload_on_device, const int64_t *offsets, int64_t n, uint8_t *frames);
+int lm_device_alloc(lm_ctx *ctx, void **ptr, size_t bytes);   /* on the context's device, for callers without a CUDA runtime */
+int lm_device_free(lm_ctx *ctx, void *ptr);
 
 /* measurement / debugging ---------------------------------------------------------------- */
 /* Device time (ms, CUDA events on the library's own stream) of the stages of the last

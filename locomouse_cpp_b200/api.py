@@ -26,7 +26,8 @@ _lib = None
 EXPORTS = ("lm_abi_version", "lm_create", "lm_destroy", "lm_last_error", "lm_configure", "lm_set_model",
            "lm_set_background", "lm_set_calibration", "lm_get_geometry", "lm_detect_batch", "lm_last_timing",
            "lm_debug_fetch", "lm_set_option", "lm_get_info", "lm_debug_nms", "lm_bounding_box_tm_de", "lm_moving_average",
-           "lm_host_alloc", "lm_host_free", "lm_unary_costs", "lm_pairwise_costs", "lm_bounding_box_base", "lm_mouse_box_size", "lm_bounding_box_tm")
+           "lm_host_alloc", "lm_host_free", "lm_unary_costs", "lm_pairwise_costs", "lm_bounding_box_base", "lm_mouse_box_size", "lm_bounding_box_tm",
+           "lm_decode_png", "lm_device_alloc", "lm_device_free")
 
 
 def _pinned_zeros(shape, dtype):
@@ -100,6 +101,12 @@ def load_library():
     L.lm_host_alloc.argtypes = [C.POINTER(vp), C.c_size_t]
     L.lm_host_free.restype = C.c_int
     L.lm_host_free.argtypes = [vp]
+    L.lm_decode_png.restype = C.c_int
+    L.lm_decode_png.argtypes = [vp, vp, i32, vp, i64, vp]
+    L.lm_device_alloc.restype = C.c_int
+    L.lm_device_alloc.argtypes = [vp, C.POINTER(vp), C.c_size_t]
+    L.lm_device_free.restype = C.c_int
+    L.lm_device_free.argtypes = [vp, vp]
     _lib = L
     return L
 
@@ -235,6 +242,44 @@ class Detector:
         lims = np.zeros((n, 2), np.int32)
         self._check(self._L.lm_bounding_box_tm(self._ctx, ptr, int(on_dev), n, C.addressof(params), raw.ctypes.data, lims.ctypes.data))
         return raw, lims
+
+    def decode_png(self, payload, offsets, out=None):
+        """PNG-coded video frames ('MPNG' / 'png ' AVI chunks) decoded on the device: frame i is payload[offsets[i]:offsets[i + 1]].
+        payload: uint8 numpy array, CPU tensor (pinned or not) or CUDA tensor on this detector's device.  Returns (or fills
+        `out`) a uint8 CUDA tensor [n, vid_rows, vid_cols], channel 0 of each decoded frame, ready for detect_batch and the
+        bounding_box_* methods.  A malformed frame raises ValueError naming it."""
+        import torch
+
+        offs = np.ascontiguousarray(offsets, dtype=np.int64)
+        if offs.ndim != 1 or offs.size < 1:
+            raise ValueError("offsets must be a 1-D array of n + 1 entries")
+        n = offs.size - 1
+        if isinstance(payload, torch.Tensor):
+            p = payload.reshape(-1)
+            if p.dtype != torch.uint8:
+                raise ValueError("payload must be uint8")
+            p = p.contiguous()
+            on_dev = p.is_cuda
+            if on_dev:
+                if p.device.index != self.device:
+                    raise ValueError(f"payload lives on cuda:{p.device.index}, detector is on cuda:{self.device}")
+                torch.cuda.current_stream(p.device).synchronize()
+        else:
+            p = np.ascontiguousarray(payload, dtype=np.uint8).reshape(-1)
+            on_dev = False
+        size = p.numel() if isinstance(p, torch.Tensor) else p.size
+        if n and (offs[0] < 0 or offs[-1] > size):
+            raise ValueError(f"offsets reach outside the payload ({size} bytes)")
+        ptr = p.data_ptr() if isinstance(p, torch.Tensor) else p.ctypes.data
+        shape = (n, self.cfg.vid_rows, self.cfg.vid_cols)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.uint8, device=f"cuda:{self.device}")
+        elif out.dtype != torch.uint8 or tuple(out.shape) != shape or not out.is_cuda or out.device.index != self.device or not out.is_contiguous():
+            raise ValueError(f"out must be a contiguous uint8 tensor {shape} on cuda:{self.device}")
+        else:
+            torch.cuda.current_stream(out.device).synchronize()
+        self._check(self._L.lm_decode_png(self._ctx, ptr, int(on_dev), offs.ctypes.data, n, out.data_ptr()))
+        return out
 
     def mouse_box_size(self, w, hb, hs):
         """computeMouseBoxSize (LocoMouse_class.cpp:1481-1506) -> (width, bottom height, side height)."""

@@ -109,6 +109,15 @@ struct lm_ctx {
         double *bbx = nullptr;
         int32_t *lims = nullptr;
     } bbs;
+    // lm_decode_png: grow-only device buffers (guarded like the scratch in guard mode), kept until lm_destroy
+    struct PngBuf {
+        uint8_t *base = nullptr, *p = nullptr;
+        size_t bytes = 0;
+    };
+    enum { PNG_SCRATCH, PNG_STAGE0, PNG_STAGE1, PNG_OFFS, PNG_STATUS, PNG_HDR, PNG_NBUF };
+    PngBuf png[PNG_NBUF];
+    cudaEvent_t ev_png_copy[2] = {}, ev_png_done[2] = {};
+    float ms_decode = 0.f;            // decode kernels of the last lm_decode_png call
     int last_B = 0;                   // size of the last sub-batch (for lm_debug_fetch)
     int last_slot = 0;
     int64_t last_s0 = 0;
@@ -703,6 +712,11 @@ int lm_destroy(lm_ctx *ctx) {
     cudaStreamDestroy(ctx->stream_hi);
     for (int s = 0; s < lm_ctx::NSLOT; ++s) cudaStreamDestroy(ctx->stream_back[s]);
     cudaStreamDestroy(ctx->copy_stream);
+    for (auto &b : ctx->png) cudaFree(b.base);
+    for (int s = 0; s < 2; ++s) {
+        if (ctx->ev_png_copy[s]) cudaEventDestroy(ctx->ev_png_copy[s]);
+        if (ctx->ev_png_done[s]) cudaEventDestroy(ctx->ev_png_done[s]);
+    }
     delete ctx;
     return LM_OK;
 }
@@ -1131,6 +1145,10 @@ int lm_get_info(const lm_ctx *ctx, const char *name, double *value) {
         *value = (double)ctx->timeline[(size_t)sub * 10 + q];
         return LM_OK;
     }
+    if (!strcmp(name, "ms_decode")) {  // device time of the decode kernels in the last lm_decode_png call
+        *value = (double)ctx->ms_decode;
+        return LM_OK;
+    }
     if (!strcmp(name, "ms_screen")) {  // device time of k_screen alone in the last lm_detect_batch call
         *value = (double)ctx->ms_screen;
         return LM_OK;
@@ -1152,7 +1170,9 @@ int lm_get_info(const lm_ctx *ctx, const char *name, double *value) {
         return LM_OK;
     }
     if (!strcmp(name, "guard_regions")) {
-        *value = (double)ctx->guard_regions.size();
+        size_t k = ctx->guard_regions.size();
+        for (const auto &b : ctx->png) k += b.base && ctx->guard ? 2 : 0;
+        *value = (double)k;
         return LM_OK;
     }
     const bool selftest = !strcmp(name, "guard_selftest");   // positive control: three guard bytes are overwritten, counted, restored
@@ -1167,6 +1187,11 @@ int lm_get_info(const lm_ctx *ctx, const char *name, double *value) {
         cudaMemset(bad, 0, sizeof *bad);
         if (selftest) cudaMemset(ctx->guard_regions.back().first + 7, 0, 3);
         for (const auto &r : ctx->guard_regions) k_guard_check<<<4, 256>>>(r.first, r.second, bad);
+        for (const auto &b : ctx->png)
+            if (b.base) {
+                k_guard_check<<<4, 256>>>(b.base, LM_GUARD_BYTES, bad);
+                k_guard_check<<<4, 256>>>(b.p + b.bytes, LM_GUARD_BYTES, bad);
+            }
         const cudaError_t e = cudaMemcpy(&h, bad, sizeof h, cudaMemcpyDeviceToHost);
         if (selftest) cudaMemset(ctx->guard_regions.back().first + 7, LM_GUARD_PATTERN, 3);
         cudaFree(bad);
@@ -1654,6 +1679,194 @@ int lm_host_alloc(void **ptr, size_t bytes) {
 int lm_host_free(void *ptr) {
     if (!ptr) return LM_OK;
     return cudaFreeHost(ptr) == cudaSuccess ? LM_OK : LM_ERR_RUNTIME;
+}
+
+int lm_device_alloc(lm_ctx *ctx, void **ptr, size_t bytes) {
+    if (!ctx || !ptr) return LM_ERR_INVALID;
+    *ptr = nullptr;
+    DeviceGuard guard(ctx->device);
+    const cudaError_t e = cudaMalloc(ptr, std::max<size_t>(bytes, 1));
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        *ptr = nullptr;
+        return fail(ctx, LM_ERR_RUNTIME, "cannot allocate %zu bytes of device memory: %s", bytes, cudaGetErrorString(e));
+    }
+    return LM_OK;
+}
+
+int lm_device_free(lm_ctx *ctx, void *ptr) {
+    if (!ctx) return LM_ERR_INVALID;
+    if (!ptr) return LM_OK;
+    DeviceGuard guard(ctx->device);
+    return cudaFree(ptr) == cudaSuccess ? LM_OK : fail(ctx, LM_ERR_RUNTIME, "cudaFree failed");
+}
+
+// ---- lm_decode_png -----------------------------------------------------------------------------------------------------
+namespace {
+// Grows one of the context's PNG buffers to at least `bytes` (contents are not kept).
+int png_reserve(lm_ctx *ctx, lm_ctx::PngBuf &b, size_t bytes) {
+    bytes = std::max<size_t>(bytes, 256);
+    if (b.bytes >= bytes) return LM_OK;
+    CK(cudaStreamSynchronize(ctx->stream));
+    CK(cudaStreamSynchronize(ctx->copy_stream));
+    cudaFree(b.base);
+    b = lm_ctx::PngBuf{};
+    const size_t g = ctx->guard ? LM_GUARD_BYTES : 0;
+    void *q = nullptr;
+    const cudaError_t e = cudaMalloc(&q, bytes + 2 * g);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(ctx, LM_ERR_RUNTIME, "cannot allocate %zu bytes of device memory for the PNG decode: %s", bytes, cudaGetErrorString(e));
+    }
+    b.base = static_cast<uint8_t *>(q);
+    b.p = b.base + g;
+    b.bytes = bytes;
+    if (g) {
+        CK(cudaMemset(b.base, LM_GUARD_PATTERN, g));
+        CK(cudaMemset(b.p + bytes, LM_GUARD_PATTERN, g));
+    } else {
+        b.base = b.p;
+    }
+    return LM_OK;
+}
+
+// Signature and IHDR of one frame (the first LM_PNG_HDR_BYTES bytes, len = the frame's size); bytes per pixel or 0 with `why`.
+int png_check_header(const uint8_t *h, int64_t len, int rows, int cols, char *why, size_t why_cap) {
+    static const uint8_t sig[8] = {0x89, 'P', 'N', 'G', 0x0d, 0x0a, 0x1a, 0x0a};
+    auto be32 = [](const uint8_t *p) { return ((uint32_t)p[0] << 24) | ((uint32_t)p[1] << 16) | ((uint32_t)p[2] << 8) | (uint32_t)p[3]; };
+    if (len < 45 || memcmp(h, sig, 8)) return snprintf(why, why_cap, "not a PNG file (%lld bytes)", (long long)len), 0;
+    if (be32(h + 8) != 13 || memcmp(h + 12, "IHDR", 4)) return snprintf(why, why_cap, "the first chunk is not IHDR"), 0;
+    const uint32_t w = be32(h + 16), ht = be32(h + 20);
+    if (w != (uint32_t)cols || ht != (uint32_t)rows)
+        return snprintf(why, why_cap, "%u x %u pixels, the configured video is %d x %d", w, ht, cols, rows), 0;
+    const int depth = h[24], ct = h[25];
+    if (depth != 8 || (ct != 0 && ct != 2 && ct != 6))
+        return snprintf(why, why_cap, "bit depth %d, colour type %d: only 8-bit grey (0), RGB (2) and RGBA (6) are decoded", depth, ct), 0;
+    if (h[26] || h[27]) return snprintf(why, why_cap, "unknown compression or filter method"), 0;
+    if (h[28]) return snprintf(why, why_cap, "interlaced frames are not decoded"), 0;
+    return ct == 0 ? 1 : ct == 2 ? 3 : 4;
+}
+
+int decode_png_impl(lm_ctx *ctx, const uint8_t *payload, int on_dev, const int64_t *offsets, int64_t n, uint8_t *frames) {
+    if (!ctx->configured) return fail(ctx, LM_ERR_STATE, "lm_decode_png needs lm_configure first");
+    if (n < 0) return fail(ctx, LM_ERR_INVALID, "negative frame count");
+    ctx->ms_decode = 0.f;
+    if (n == 0) return LM_OK;
+    if (!payload || !offsets || !frames) return fail(ctx, LM_ERR_INVALID, "null argument");
+    const int rows = ctx->cfg.vid_rows, cols = ctx->cfg.vid_cols;
+    for (int64_t i = 0; i < n; ++i)
+        if (offsets[i] < 0 || offsets[i + 1] < offsets[i]) return fail(ctx, LM_ERR_INVALID, "frame %lld: offsets must not decrease", (long long)i);
+    if ((int64_t)rows * (1 + (int64_t)cols * 4) >= INT32_MAX) return fail(ctx, LM_ERR_INVALID, "frame too large for the PNG decoder");
+    cudaStream_t st = ctx->stream, cp = ctx->copy_stream;
+    auto &B = ctx->png;
+    if (int rc = png_reserve(ctx, B[lm_ctx::PNG_OFFS], (size_t)(n + 1) * sizeof(int64_t))) return rc;
+    if (int rc = png_reserve(ctx, B[lm_ctx::PNG_STATUS], (size_t)n * sizeof(int32_t))) return rc;
+    int64_t *d_offs = reinterpret_cast<int64_t *>(B[lm_ctx::PNG_OFFS].p);
+    int32_t *d_status = reinterpret_cast<int32_t *>(B[lm_ctx::PNG_STATUS].p);
+    CK(cudaMemcpyAsync(d_offs, offsets, (size_t)(n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    CK(cudaMemsetAsync(d_status, 0xff, (size_t)n * sizeof(int32_t), st));  // -1: not decoded
+
+    // every frame's signature and IHDR, checked before anything is decoded
+    std::vector<uint8_t> hdr_dev;
+    if (on_dev) {
+        if (int rc = png_reserve(ctx, B[lm_ctx::PNG_HDR], (size_t)n * LM_PNG_HDR_BYTES)) return rc;
+        if (lm_launch_png_headers(payload, d_offs, 0, n, B[lm_ctx::PNG_HDR].p, st) < 0) return fail(ctx, LM_ERR_RUNTIME, "PNG header launch failed");
+        hdr_dev.resize((size_t)n * LM_PNG_HDR_BYTES);
+        CK(cudaMemcpyAsync(hdr_dev.data(), B[lm_ctx::PNG_HDR].p, hdr_dev.size(), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+    }
+    std::vector<uint8_t> bpp((size_t)n);
+    for (int64_t i = 0; i < n; ++i) {
+        char why[160];
+        const uint8_t *h = on_dev ? hdr_dev.data() + (size_t)i * LM_PNG_HDR_BYTES : payload + offsets[i];
+        if (!(bpp[i] = (uint8_t)png_check_header(h, offsets[i + 1] - offsets[i], rows, cols, why, sizeof why)))
+            return fail(ctx, LM_ERR_INVALID, "frame %lld: %s", (long long)i, why);
+    }
+
+    // Pieces of consecutive frames share one scratch allocation (one filtered stream per frame) and, from the host, one of
+    // two compressed staging buffers: the copy of piece k + 1 (copy stream) overlaps the decode of piece k.
+    const int64_t max_piece = on_dev ? 8192 : std::max<int64_t>(1024, (n + 3) / 4);
+    const size_t scratch_budget = (size_t)4 << 30, stage_budget = (size_t)2 << 30;
+    struct Piece {
+        int64_t s, e;
+        int64_t slot;
+    };
+    std::vector<Piece> pieces;
+    size_t scratch_need = 0, stage_need = 0;
+    for (int64_t s = 0; s < n;) {
+        int64_t e = s, slot = 0;
+        while (e < n && e - s < max_piece) {
+            const int64_t sl = std::max<int64_t>(slot, (int64_t)rows * (1 + (int64_t)cols * bpp[e]));
+            const size_t comp = (size_t)(offsets[e + 1] - offsets[s]);
+            if (e > s && ((size_t)sl * (e + 1 - s) > scratch_budget || (!on_dev && comp > stage_budget))) break;
+            slot = sl;
+            ++e;
+        }
+        pieces.push_back({s, e, slot});
+        scratch_need = std::max(scratch_need, (size_t)slot * (e - s));
+        stage_need = std::max(stage_need, (size_t)(offsets[e] - offsets[s]));
+        s = e;
+    }
+    if (int rc = png_reserve(ctx, B[lm_ctx::PNG_SCRATCH], scratch_need)) return rc;
+    if (!on_dev) {
+        for (int k = 0; k < 2 && k < (int)pieces.size(); ++k)
+            if (int rc = png_reserve(ctx, B[lm_ctx::PNG_STAGE0 + k], stage_need)) return rc;
+        for (int k = 0; k < 2; ++k) {
+            if (!ctx->ev_png_copy[k]) CK(cudaEventCreateWithFlags(&ctx->ev_png_copy[k], cudaEventDisableTiming));
+            if (!ctx->ev_png_done[k]) CK(cudaEventCreateWithFlags(&ctx->ev_png_done[k], cudaEventDisableTiming));
+        }
+    }
+    struct Events {  // start / end of each decode launch, for ms_decode
+        std::vector<cudaEvent_t> ev;
+        ~Events() {
+            for (cudaEvent_t e : ev) cudaEventDestroy(e);
+        }
+    } T;
+    T.ev.resize(2 * pieces.size());
+    for (auto &e : T.ev) CK(cudaEventCreate(&e));
+    for (size_t k = 0; k < pieces.size(); ++k) {
+        const Piece &P = pieces[k];
+        const uint8_t *src = payload;
+        int64_t base = 0;
+        if (!on_dev) {
+            uint8_t *stg = B[lm_ctx::PNG_STAGE0 + (k & 1)].p;
+            if (k >= 2) CK(cudaStreamWaitEvent(cp, ctx->ev_png_done[k & 1], 0));  // piece k - 2 no longer reads this buffer
+            CK(cudaMemcpyAsync(stg, payload + offsets[P.s], (size_t)(offsets[P.e] - offsets[P.s]), cudaMemcpyHostToDevice, cp));
+            CK(cudaEventRecord(ctx->ev_png_copy[k & 1], cp));
+            CK(cudaStreamWaitEvent(st, ctx->ev_png_copy[k & 1], 0));
+            src = stg;
+            base = offsets[P.s];
+        }
+        CK(cudaEventRecord(T.ev[2 * k], st));
+        if (lm_launch_png_decode(src, d_offs + P.s, base, (int)(P.e - P.s), rows, cols, B[lm_ctx::PNG_SCRATCH].p, P.slot,
+                                 frames + P.s * (int64_t)rows * cols, d_status + P.s, st) < 0)
+            return fail(ctx, LM_ERR_RUNTIME, "PNG decode launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        CK(cudaEventRecord(T.ev[2 * k + 1], st));
+        if (!on_dev) CK(cudaEventRecord(ctx->ev_png_done[k & 1], st));
+    }
+    std::vector<int32_t> status((size_t)n);
+    CK(cudaMemcpyAsync(status.data(), d_status, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    for (size_t k = 0; k < pieces.size(); ++k) {
+        float t = 0.f;
+        if (cudaEventElapsedTime(&t, T.ev[2 * k], T.ev[2 * k + 1]) == cudaSuccess) ctx->ms_decode += t;
+    }
+    for (int64_t i = 0; i < n; ++i)
+        if (status[i] != LM_PNG_OK) return fail(ctx, LM_ERR_INVALID, "frame %lld: %s", (long long)i, lm_png_status_text(status[i]));
+    return LM_OK;
+}
+}  // namespace
+
+int lm_decode_png(lm_ctx *ctx, const uint8_t *payload, int payload_on_device, const int64_t *offsets, int64_t n, uint8_t *frames) {
+    if (!ctx) return LM_ERR_INVALID;
+    DeviceGuard guard(ctx->device);
+    const int rc = decode_png_impl(ctx, payload, payload_on_device, offsets, n, frames);
+    if (rc != LM_OK) {  // nothing of this call may stay in flight: the caller's payload and frames would still be in use
+        cudaStreamSynchronize(ctx->copy_stream);
+        cudaStreamSynchronize(ctx->stream);
+        cudaGetLastError();
+    }
+    return rc;
 }
 
 int lm_last_timing(const lm_ctx *ctx, float ms[7], int64_t *launches) {

@@ -203,6 +203,20 @@ inline int lm_whatif_skip() {
 }
 long long lm_screen2_last_macs();  // int8 MACs issued by the last k_screen2 launch (whole sub-batch)
 
+// PNG frame decode (k_png.cu).  Per-frame status codes of k_png_decode:
+enum {
+    LM_PNG_OK = 0, LM_PNG_HEADER, LM_PNG_TRUNCATED, LM_PNG_ZLIB, LM_PNG_BLOCK_TYPE, LM_PNG_CODES, LM_PNG_SYMBOL, LM_PNG_DISTANCE,
+    LM_PNG_TOO_LONG, LM_PNG_TOO_SHORT, LM_PNG_STORED, LM_PNG_FILTER, LM_PNG_NO_IDAT, LM_PNG_NOT_RUN
+};
+constexpr int LM_PNG_HDR_BYTES = 33;  // signature + IHDR chunk
+// Frame j of the launch is payload[offs[j] - base, offs[j + 1] - base); its filtered stream goes to scratch + j * slot, its
+// pixels to out + j * rows * cols, its LM_PNG_* code to status[j].
+int lm_launch_png_decode(const uint8_t *payload, const int64_t *offs, int64_t base, int n, int rows, int cols, uint8_t *scratch, int64_t slot,
+                         uint8_t *out, int32_t *status, cudaStream_t s);
+// hdr[j][LM_PNG_HDR_BYTES] = the first bytes of frame j, zero-padded
+int lm_launch_png_headers(const uint8_t *payload, const int64_t *offs, int64_t base, int64_t n, uint8_t *hdr, cudaStream_t s);
+const char *lm_png_status_text(int st);
+
 // pick the padded kernel-row width the correlation kernel is instantiated for (>= kw), or -1
 int lm_corr_kwp(int kw);
 // dynamic shared memory the correlation kernel needs for a view/template (for capability checks)

@@ -292,10 +292,21 @@ void LocoMouse::initializePaths(const LocoMouse_ParseInputs &INPUT) {
 
 void LocoMouse::loadVideo() {
     if (lmmedia::is_avi(VIDEO_FILE)) {  // the reference's input: VideoCapture + extractChannel(0) (class.cpp:367-400, 1282-1293)
-        lmmedia::Video V = lmmedia::read_avi(VIDEO_FILE);
+        lmmedia::HostAlloc pinned;
+        pinned.alloc = [](size_t b) -> void * {
+            void *q = nullptr;
+            return lm_host_alloc(&q, b) == LM_OK ? q : nullptr;
+        };
+        pinned.release = [](void *q) { lm_host_free(q); };
+        lmmedia::Video V = lmmedia::read_avi(VIDEO_FILE, pinned);
         N_FRAMES = (unsigned int)V.n;
         VID_ROWS = V.rows;
         VID_COLS = V.cols;
+        if (V.png) {  // decoded on the device once lm_configure has run (configureDevice)
+            PNG_PAYLOAD = V.payload;
+            PNG_OFFSETS = std::move(V.offsets);
+            return;
+        }
         VIDEO.resize(V.frames.size());
         std::copy(V.frames.begin(), V.frames.end(), VIDEO.begin());
         return;
@@ -393,7 +404,15 @@ LocoMouse::LocoMouse(LocoMouse_ParseInputs INPUTS) {
     if (rc != LM_OK) throw std::runtime_error(std::string("lm_create: ") + lm_last_error(nullptr));
 }
 
-LocoMouse::~LocoMouse() { lm_destroy(CTX); }
+LocoMouse::~LocoMouse() {
+    lm_device_free(CTX, D_VIDEO);
+    lm_destroy(CTX);
+}
+
+const uint8_t *LocoMouse::frames(int &on_device) const {
+    on_device = D_VIDEO != nullptr;
+    return D_VIDEO ? D_VIDEO : VIDEO.data();
+}
 
 // ---- pass 1 (out of scope): positions come from the user box or from a pass-1 output file -------------
 namespace {
@@ -460,7 +479,9 @@ void LocoMouse::computeBoundingBox() {
     p.min_pixel_visible = LM_PARAMS.min_pixel_visible;
     p.sums_as_float = LM_PARAMS.pass1_integer_sums ? 0 : 1;
     std::vector<double> box((size_t)N_FRAMES * 6);
-    check(lm_bounding_box_base(CTX, VIDEO.data(), /*frames_on_device=*/0, N_FRAMES, &p, box.data(), nullptr));
+    int on_dev = 0;
+    const uint8_t *video = frames(on_dev);
+    check(lm_bounding_box_base(CTX, video, on_dev, N_FRAMES, &p, box.data(), nullptr));
     std::vector<double> bb_x(N_FRAMES), bb_yb(N_FRAMES), bb_ys(N_FRAMES), w(N_FRAMES), hb(N_FRAMES), hs(N_FRAMES);
     for (unsigned int f = 0; f < N_FRAMES; ++f) {
         const double *o = &box[(size_t)f * 6];
@@ -544,7 +565,9 @@ void LocoMouse_TM::computeBoundingBox() {
         p.disk_size = DISK_SIZE;
         p.disk = DISK_FILTER.data();
         std::vector<double> bb_x(N_FRAMES);
-        check(lm_bounding_box_tm(CTX, VIDEO.data(), /*frames_on_device=*/0, N_FRAMES, &p, bb_x.data(), nullptr));
+        int on_dev = 0;
+        const uint8_t *video = frames(on_dev);
+        check(lm_bounding_box_tm(CTX, video, on_dev, N_FRAMES, &p, bb_x.data(), nullptr));
         BB_X_POS.assign(N_FRAMES, 0);
         if (lm_moving_average(bb_x.data(), N_FRAMES, LM_PARAMS.moving_average_window, BB_X_POS.data()) != LM_OK)
             throw std::invalid_argument("moving_average_window is invalid.");
@@ -581,7 +604,9 @@ void LocoMouse_TM_DE::computeBoundingBox() {
         p.min_count = 10;
         p.width_margin = 1.1;
         std::vector<double> bb_x(N_FRAMES);
-        check(lm_bounding_box_tm_de(CTX, VIDEO.data(), /*frames_on_device=*/0, N_FRAMES, &p, bb_x.data(), nullptr));
+        int on_dev = 0;
+        const uint8_t *video = frames(on_dev);
+        check(lm_bounding_box_tm_de(CTX, video, on_dev, N_FRAMES, &p, bb_x.data(), nullptr));
         BB_X_POS.assign(N_FRAMES, 0);
         if (lm_moving_average(bb_x.data(), N_FRAMES, LM_PARAMS.moving_average_window, BB_X_POS.data()) != LM_OK)
             throw std::invalid_argument("moving_average_window is invalid.");
@@ -612,6 +637,15 @@ void LocoMouse::configureDevice() {
     check(lm_configure(CTX, &c));
     check(lm_set_background(CTX, BKG.data()));
     check(lm_set_calibration(CTX, CALIBRATION.data()));
+    if (PNG_PAYLOAD && !D_VIDEO) {  // the whole PNG-coded video, decoded once; pass 1 and the frame loop read it in place
+        const size_t bytes = (size_t)N_FRAMES * VID_ROWS * VID_COLS;
+        void *d = nullptr;
+        if (lm_device_alloc(CTX, &d, bytes) != LM_OK)
+            throw std::runtime_error("The decoded video (" + std::to_string(N_FRAMES) + " frames, " + std::to_string(bytes) +
+                                     " bytes) does not fit in device memory: " + lm_last_error(CTX));
+        D_VIDEO = static_cast<uint8_t *>(d);
+        check(lm_decode_png(CTX, PNG_PAYLOAD.get(), 0, PNG_OFFSETS.data(), N_FRAMES, D_VIDEO));
+    }
 }
 
 // ---- initializeFeatureLoop (LocoMouse_class.cpp:655-769): hand the per-video state to the device -------
@@ -689,8 +723,10 @@ void LocoMouse::runChunk(unsigned int first) {
     b->flags.resize(n);
     lm_results r = b->view();
     const size_t fsz = (size_t)VID_ROWS * VID_COLS;
-    const uint8_t *prev = first > 0 ? VIDEO.data() + (size_t)(first - 1) * fsz : nullptr;
-    check(lm_detect_batch(CTX, VIDEO.data() + (size_t)first * fsz, /*frames_on_device=*/0, prev, n, first, BB_X_POS.data() + first,
+    int on_dev = 0;
+    const uint8_t *video = frames(on_dev);
+    const uint8_t *prev = first > 0 ? video + (size_t)(first - 1) * fsz : nullptr;
+    check(lm_detect_batch(CTX, video + (size_t)first * fsz, on_dev, prev, n, first, BB_X_POS.data() + first,
                           BB_Y_SIDE_POS.data() + first, BB_Y_BOTTOM_POS.data() + first, &r));
     if (!LM_PARAMS.PRIOR_PAW.empty() && !LM_PARAMS.PRIOR_SNOUT.empty()) {
         // ---- cost builders for the whole chunk (class.cpp:873-919) --------------------------------------------------

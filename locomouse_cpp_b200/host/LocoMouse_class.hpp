@@ -151,6 +151,11 @@ protected:
     std::string output_file;
 
     PinnedArray<uint8_t> VIDEO;       // raw 8-bit frames (channel 0), N_FRAMES x vid_rows x vid_cols, page-locked
+    // PNG-coded AVI: the frame chunks (page-locked, frame i = [PNG_OFFSETS[i], PNG_OFFSETS[i + 1])), decoded once by
+    // configureDevice into D_VIDEO (device memory, same layout as VIDEO); VIDEO stays empty
+    std::shared_ptr<uint8_t> PNG_PAYLOAD;
+    std::vector<int64_t> PNG_OFFSETS;
+    uint8_t *D_VIDEO = nullptr;
     int VID_ROWS = 0, VID_COLS = 0;
     std::vector<uint8_t> BKG;
     std::vector<int32_t> CALIBRATION;  // ind_warp_mapping, N_ROWS x N_COLS
@@ -196,6 +201,7 @@ protected:
     void check(int rc) const;          // lm_status -> exception
     void runChunk(unsigned int first_frame);
     void configureDevice();            // lm_configure + background + calibration for the current box sizes
+    const uint8_t *frames(int &on_device) const;  // first frame of the video: VIDEO, or D_VIDEO for PNG-coded video
     const Batch &batchFor(int frame) const;
     virtual bool usesImadjust() const { return false; }  // LocoMouse_TM::readFrame applies imadjust(0, 0.6)
     // class.cpp:2221-2346, 2385-2482

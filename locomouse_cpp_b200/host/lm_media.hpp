@@ -3,8 +3,10 @@
 //   background  cv::imread(file, CV_LOAD_IMAGE_GRAYSCALE)    (LocoMouse_class.cpp:402-417)
 // Video: AVI (RIFF, also OpenDML 'AVIX' extensions) whose stream 0 holds UNCOMPRESSED frames -- 8-bit grey ('Y800' /
 // 'GREY' / 'Y8  ', what cv2.VideoWriter(fourcc = 0, isColor = False) writes), BI_RGB 8-bit with a palette, BI_RGB 24- / 32-bit
-// (channel 0 = blue, as extractChannel takes it).  Compressed or YUV-planar streams need a decoder, which is outside the hot
-// path: they are refused with a message that says so.  Background: PNG, 8 bits per channel, non-interlaced; colour images are
+// (channel 0 = blue, as extractChannel takes it).  PNG-coded streams ('MPNG' / 'png ', lossless, what cv2.VideoWriter writes
+// with those fourccs) are not decoded here: their frame chunks -- each a complete PNG file -- are returned as one payload with
+// offsets, for lm_decode_png to decode on the device.  Other compressed or YUV-planar streams need a decoder that is outside
+// this library: they are refused with a message that says so.  Background: PNG, 8 bits per channel, non-interlaced; colour images are
 // reduced to grey as libpng does for OpenCV (png_set_rgb_to_gray with 0.299 / 0.587).  Both are checked against what the
 // real OpenCV reads from the same files (tests/test_host_media.py).
 #pragma once
@@ -13,6 +15,7 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -44,13 +47,40 @@ inline bool is_png(const std::string &name) {
     return h.size() >= 8 && !std::memcmp(h.data(), sig, 8);
 }
 
-struct Video {
-    int n = 0, rows = 0, cols = 0;
-    std::vector<uint8_t> frames;  // channel 0 of every frame, [n][rows][cols]
+// Storage of a PNG stream's payload (the class mirror passes page-locked memory so that the upload runs at the PCIe rate)
+struct HostAlloc {
+    void *(*alloc)(size_t) = [](size_t b) { return std::malloc(b ? b : 1); };
+    void (*release)(void *) = [](void *p) { std::free(p); };
 };
 
+struct Video {
+    int n = 0, rows = 0, cols = 0;
+    std::vector<uint8_t> frames;  // channel 0 of every frame, [n][rows][cols] (uncompressed streams)
+    // PNG-coded streams: frame i = payload[offsets[i], offsets[i + 1]), a complete PNG file; `frames` stays empty
+    bool png = false;
+    std::shared_ptr<uint8_t> payload;
+    std::vector<int64_t> offsets;
+};
+
+// Signature and IHDR of one PNG frame: 8-bit grey / RGB / RGBA, not interlaced (what lm_decode_png decodes)
+inline void check_png_frame(const uint8_t *d, size_t len, int &rows, int &cols, const std::string &where) {
+    static const uint8_t sig[8] = {0x89, 'P', 'N', 'G', 0x0d, 0x0a, 0x1a, 0x0a};
+    auto fail = [&](const std::string &why) { throw std::runtime_error(where + ": " + why); };
+    if (len < 45 || std::memcmp(d, sig, 8) || be32(d + 8) != 13 || std::memcmp(d + 12, "IHDR", 4)) fail("not a PNG image");
+    const int w = (int)be32(d + 16), h = (int)be32(d + 20), depth = d[24], ct = d[25];
+    if (depth != 8 || (ct != 0 && ct != 2 && ct != 6))
+        fail("bit depth " + std::to_string(depth) + ", colour type " + std::to_string(ct) +
+             ": only 8-bit grey, RGB and RGBA PNG frames are decoded (no 16-bit or palette frames)");
+    if (d[26] || d[27]) fail("unknown PNG compression or filter method");
+    if (d[28]) fail("interlaced PNG frames are not decoded");
+    if (w <= 0 || h <= 0) fail("empty image");
+    if (rows == 0) rows = h, cols = w;
+    else if (h != rows || w != cols)
+        fail(std::to_string(w) + " x " + std::to_string(h) + " pixels, frame 0 has " + std::to_string(cols) + " x " + std::to_string(rows));
+}
+
 // Streams the frame chunks of stream 0 ('00db' / '00dc') in file order.
-inline Video read_avi(const std::string &name) {
+inline Video read_avi(const std::string &name, const HostAlloc &halloc = HostAlloc()) {
     FILE *f = std::fopen(name.c_str(), "rb");
     if (!f) throw std::runtime_error("Cannot open file: " + name);
     struct Closer {
@@ -70,6 +100,7 @@ inline Video read_avi(const std::string &name) {
     bool have_format = false, stream0_is_video = false;
     int stream_index = -1;
     std::vector<uint8_t> chunk;
+    std::vector<std::pair<int64_t, uint32_t>> png_chunks;  // file offset and size of every PNG frame chunk
     // A flat walk: LIST / RIFF headers are entered (only their 4-byte type is consumed), every other chunk is read or skipped.
     for (;;) {
         uint8_t ch[8];
@@ -115,6 +146,13 @@ inline Video read_avi(const std::string &name) {
         auto cc = [](const char *s) { return le32(reinterpret_cast<const uint8_t *>(s)); };
         const bool grey = fourcc == cc("Y800") || fourcc == cc("GREY") || fourcc == cc("Y8  ") || fourcc == cc("Y8\0\0");
         const bool rgb = fourcc == 0 || fourcc == cc("DIB ") || fourcc == cc("RGB ") || fourcc == cc("RAW ");
+        if (fourcc == cc("MPNG") || fourcc == cc("png ")) {  // read after the walk, straight into the payload
+            if (size == 0) continue;
+            const off_t at = ftello(f);
+            png_chunks.emplace_back((int64_t)at, size);
+            if (!skip((uint64_t)size + (size & 1))) fail("truncated frame");
+            continue;
+        }
         if (!(grey && bits == 8) && !(rgb && (bits == 8 || bits == 24 || bits == 32))) {
             char fc[5] = {(char)(fourcc & 255), (char)((fourcc >> 8) & 255), (char)((fourcc >> 16) & 255), (char)((fourcc >> 24) & 255), 0};
             fail(std::string("stream 0 is '") + fc + "' with " + std::to_string(bits) +
@@ -145,6 +183,23 @@ inline Video read_avi(const std::string &name) {
             }
         }
         ++V.n;
+    }
+    if (!png_chunks.empty()) {
+        uint64_t total = 0;
+        for (const auto &c : png_chunks) total += c.second;
+        uint8_t *buf = static_cast<uint8_t *>(halloc.alloc((size_t)total));
+        if (!buf) fail("cannot allocate " + std::to_string(total) + " bytes for the compressed frames");
+        V.payload = std::shared_ptr<uint8_t>(buf, halloc.release);
+        V.png = true;
+        V.offsets.push_back(0);
+        V.rows = V.cols = 0;  // taken from frame 0's IHDR
+        for (const auto &c : png_chunks) {
+            uint8_t *d = buf + V.offsets.back();
+            if (fseeko(f, (off_t)c.first, SEEK_SET) != 0 || !rd(d, c.second)) fail("truncated frame");
+            check_png_frame(d, c.second, V.rows, V.cols, "Video file " + name + ", frame " + std::to_string(V.n));
+            V.offsets.push_back(V.offsets.back() + c.second);
+            ++V.n;
+        }
     }
     if (V.n == 0) fail("no video frames found");
     return V;

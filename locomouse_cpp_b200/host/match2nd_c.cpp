@@ -88,10 +88,29 @@ int lmh_yaml_write(const char *path, const char *names, int n, const int32_t *ro
 int lmh_read_avi(const char *path, int32_t *dims, uint8_t *out, char *msg, int msg_cap) {
     try {
         const lmmedia::Video V = lmmedia::read_avi(path);
+        if (V.png) throw std::runtime_error(std::string("Video file ") + path + ": PNG-coded stream (lmh_read_avi_png)");
         dims[0] = V.n;
         dims[1] = V.rows;
         dims[2] = V.cols;
         if (out) std::memcpy(out, V.frames.data(), V.frames.size());
+        return 0;
+    } catch (const std::exception &e) {
+        if (msg && msg_cap > 0) std::snprintf(msg, (size_t)msg_cap, "%s", e.what());
+        return 1;
+    }
+}
+// PNG-coded AVI: dims = {n, rows, cols, payload bytes}; with payload / offsets NULL only the dimensions are returned,
+// otherwise payload receives the frame chunks and offsets[n + 1] their bounds.  0 ok, 1 error (msg filled)
+int lmh_read_avi_png(const char *path, int64_t *dims, uint8_t *payload, int64_t *offsets, char *msg, int msg_cap) {
+    try {
+        const lmmedia::Video V = lmmedia::read_avi(path);
+        if (!V.png) throw std::runtime_error(std::string("Video file ") + path + ": not a PNG-coded stream");
+        dims[0] = V.n;
+        dims[1] = V.rows;
+        dims[2] = V.cols;
+        dims[3] = V.offsets.back();
+        if (payload) std::memcpy(payload, V.payload.get(), (size_t)V.offsets.back());
+        if (offsets) std::memcpy(offsets, V.offsets.data(), V.offsets.size() * sizeof(int64_t));
         return 0;
     } catch (const std::exception &e) {
         if (msg && msg_cap > 0) std::snprintf(msg, (size_t)msg_cap, "%s", e.what());
