@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define LM_ABI_VERSION 5  /* 5: lm_bounding_box_tm, and (backward compatible additions) lm_decode_png, lm_device_alloc / lm_device_free, lm_get_info("ms_decode"); 4: lm_bounding_box_base, lm_mouse_box_size; 2: lm_set_option, lm_get_info, lm_debug_nms, lm_bounding_box_tm_de, lm_moving_average; 3: lm_host_alloc / lm_host_free, lm_unary_costs / lm_pairwise_costs, options streams 1..4, screen_layout, screen_priority */
+#define LM_ABI_VERSION 5  /* 5: lm_bounding_box_tm, and (backward compatible additions) lm_decode_png, lm_decode_ffv1, lm_device_alloc / lm_device_free, lm_get_info("ms_decode"); 4: lm_bounding_box_base, lm_mouse_box_size; 2: lm_set_option, lm_get_info, lm_debug_nms, lm_bounding_box_tm_de, lm_moving_average; 3: lm_host_alloc / lm_host_free, lm_unary_costs / lm_pairwise_costs, options streams 1..4, screen_layout, screen_priority */
 
 /* feature / view indices used in every [2] / [3] array below */
 enum { LM_PAW = 0, LM_SNOUT = 1, LM_TAIL = 2 };
@@ -304,6 +304,14 @@ int lm_host_free(void *ptr);
  * verified).  Host payloads are copied in pieces on the copy stream, overlapped with the decode of the previous piece.
  * Needs lm_configure only.  lm_get_info("ms_decode"): device ms of the decode kernels in the last call. */
 int lm_decode_png(lm_ctx *ctx, const uint8_t *payload, int payload_on_device, const int64_t *offsets, int64_t n, uint8_t *frames);
+/* FFV1-coded AVI frames (fourcc 'FFV1', version 3 as libavcodec writes it): extradata is the configuration record (the AVI
+ * 'strf' bytes after the BITMAPINFOHEADER), payload / offsets / frames as for lm_decode_png.  The record must be version 3,
+ * 8 bits, grey (colorspace 0 without chroma planes) or RGB (colorspace 1, with or without alpha), coder_type 0, 1 or 2;
+ * frame 0 must be a keyframe.  The output is channel 0 of the frame cv::VideoCapture delivers (grey, or blue), bit-exact.
+ * Each (GOP, slice) decodes serially on the device; slice CRCs are checked first.  LM_ERR_INVALID names the record problem
+ * or the first bad frame and slice.  Needs lm_configure only.  lm_get_info("ms_decode") covers it. */
+int lm_decode_ffv1(lm_ctx *ctx, const uint8_t *extradata, int64_t extradata_len, const uint8_t *payload, int payload_on_device,
+                   const int64_t *offsets, int64_t n, uint8_t *frames);
 int lm_device_alloc(lm_ctx *ctx, void **ptr, size_t bytes);   /* on the context's device, for callers without a CUDA runtime */
 int lm_device_free(lm_ctx *ctx, void *ptr);
 

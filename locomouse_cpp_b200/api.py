@@ -27,7 +27,7 @@ EXPORTS = ("lm_abi_version", "lm_create", "lm_destroy", "lm_last_error", "lm_con
            "lm_set_background", "lm_set_calibration", "lm_get_geometry", "lm_detect_batch", "lm_last_timing",
            "lm_debug_fetch", "lm_set_option", "lm_get_info", "lm_debug_nms", "lm_bounding_box_tm_de", "lm_moving_average",
            "lm_host_alloc", "lm_host_free", "lm_unary_costs", "lm_pairwise_costs", "lm_bounding_box_base", "lm_mouse_box_size", "lm_bounding_box_tm",
-           "lm_decode_png", "lm_device_alloc", "lm_device_free")
+           "lm_decode_png", "lm_device_alloc", "lm_device_free", "lm_decode_ffv1")
 
 
 def _pinned_zeros(shape, dtype):
@@ -103,6 +103,8 @@ def load_library():
     L.lm_host_free.argtypes = [vp]
     L.lm_decode_png.restype = C.c_int
     L.lm_decode_png.argtypes = [vp, vp, i32, vp, i64, vp]
+    L.lm_decode_ffv1.restype = C.c_int
+    L.lm_decode_ffv1.argtypes = [vp, vp, i64, vp, i32, vp, i64, vp]
     L.lm_device_alloc.restype = C.c_int
     L.lm_device_alloc.argtypes = [vp, C.POINTER(vp), C.c_size_t]
     L.lm_device_free.restype = C.c_int
@@ -248,6 +250,20 @@ class Detector:
         payload: uint8 numpy array, CPU tensor (pinned or not) or CUDA tensor on this detector's device.  Returns (or fills
         `out`) a uint8 CUDA tensor [n, vid_rows, vid_cols], channel 0 of each decoded frame, ready for detect_batch and the
         bounding_box_* methods.  A malformed frame raises ValueError naming it."""
+        return self._decode(lambda ptr, on_dev, offs, n, out_ptr: self._L.lm_decode_png(self._ctx, ptr, on_dev, offs, n, out_ptr),
+                            payload, offsets, out)
+
+    def decode_ffv1(self, extradata, payload, offsets, out=None):
+        """FFV1-coded video frames ('FFV1' AVI chunks, version 3) decoded on the device, bit-exact with cv2.VideoCapture's
+        channel 0.  extradata: the configuration record (the AVI 'strf' bytes after the BITMAPINFOHEADER); payload, offsets and
+        out as for decode_png.  A refused record or a malformed frame raises ValueError naming the reason, frame and slice."""
+        ex = np.ascontiguousarray(np.frombuffer(bytes(extradata), np.uint8) if isinstance(extradata, (bytes, bytearray)) else extradata,
+                                  dtype=np.uint8).reshape(-1)
+        return self._decode(lambda ptr, on_dev, offs, n, out_ptr: self._L.lm_decode_ffv1(self._ctx, ex.ctypes.data, ex.size, ptr, on_dev,
+                                                                                          offs, n, out_ptr),
+                            payload, offsets, out)
+
+    def _decode(self, call, payload, offsets, out):
         import torch
 
         offs = np.ascontiguousarray(offsets, dtype=np.int64)
@@ -278,7 +294,7 @@ class Detector:
             raise ValueError(f"out must be a contiguous uint8 tensor {shape} on cuda:{self.device}")
         else:
             torch.cuda.current_stream(out.device).synchronize()
-        self._check(self._L.lm_decode_png(self._ctx, ptr, int(on_dev), offs.ctypes.data, n, out.data_ptr()))
+        self._check(call(ptr, int(on_dev), offs.ctypes.data, n, out.data_ptr()))
         return out
 
     def mouse_box_size(self, w, hb, hs):

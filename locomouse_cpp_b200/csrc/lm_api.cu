@@ -8,10 +8,12 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <vector>
 
+#include "ffv1_format.h"
 #include "lm_internal.h"
 
 namespace {
@@ -114,10 +116,12 @@ struct lm_ctx {
         uint8_t *base = nullptr, *p = nullptr;
         size_t bytes = 0;
     };
-    enum { PNG_SCRATCH, PNG_STAGE0, PNG_STAGE1, PNG_OFFS, PNG_STATUS, PNG_HDR, PNG_NBUF };
+    // (lm_decode_ffv1 shares the staging, offset, status and header buffers and adds its own)
+    enum { PNG_SCRATCH, PNG_STAGE0, PNG_STAGE1, PNG_OFFS, PNG_STATUS, PNG_HDR, FFV1_REC, FFV1_INIT, FFV1_SOFF, FFV1_SLEN, FFV1_CHAINS,
+           FFV1_WORK0, FFV1_WORK1, PNG_NBUF };
     PngBuf png[PNG_NBUF];
     cudaEvent_t ev_png_copy[2] = {}, ev_png_done[2] = {};
-    float ms_decode = 0.f;            // decode kernels of the last lm_decode_png call
+    float ms_decode = 0.f;            // decode kernels of the last lm_decode_png / lm_decode_ffv1 call
     int last_B = 0;                   // size of the last sub-batch (for lm_debug_fetch)
     int last_slot = 0;
     int64_t last_s0 = 0;
@@ -1145,7 +1149,7 @@ int lm_get_info(const lm_ctx *ctx, const char *name, double *value) {
         *value = (double)ctx->timeline[(size_t)sub * 10 + q];
         return LM_OK;
     }
-    if (!strcmp(name, "ms_decode")) {  // device time of the decode kernels in the last lm_decode_png call
+    if (!strcmp(name, "ms_decode")) {  // device time of the decode kernels in the last lm_decode_png / lm_decode_ffv1 call
         *value = (double)ctx->ms_decode;
         return LM_OK;
     }
@@ -1856,6 +1860,180 @@ int decode_png_impl(lm_ctx *ctx, const uint8_t *payload, int on_dev, const int64
     return LM_OK;
 }
 }  // namespace
+
+// ---- lm_decode_ffv1 ----------------------------------------------------------------------------------------------------
+namespace {
+int decode_ffv1_impl(lm_ctx *ctx, const uint8_t *extradata, int64_t extradata_len, const uint8_t *payload, int on_dev, const int64_t *offsets,
+                     int64_t n, uint8_t *frames) {
+    if (!ctx->configured) return fail(ctx, LM_ERR_STATE, "lm_decode_ffv1 needs lm_configure first");
+    if (n < 0 || extradata_len < 0) return fail(ctx, LM_ERR_INVALID, "negative frame count or record length");
+    ctx->ms_decode = 0.f;
+    if (n == 0) return LM_OK;
+    if (!payload || !offsets || !frames || (extradata_len && !extradata)) return fail(ctx, LM_ERR_INVALID, "null argument");
+    const int rows = ctx->cfg.vid_rows, cols = ctx->cfg.vid_cols;
+    for (int64_t i = 0; i < n; ++i)
+        if (offsets[i] < 0 || offsets[i + 1] < offsets[i]) return fail(ctx, LM_ERR_INVALID, "frame %lld: offsets must not decrease", (long long)i);
+    std::unique_ptr<ffv1::Record> rec(new ffv1::Record);
+    char why[200];
+    int64_t init_bytes = 0;
+    if (ffv1::parse_record(extradata, extradata_len, rows, cols, *rec, nullptr, &init_bytes, why, sizeof why))
+        return fail(ctx, LM_ERR_INVALID, "FFV1 configuration record: %s", why);
+    std::vector<uint8_t> initial((size_t)std::max<int64_t>(init_bytes, 1));
+    ffv1::parse_record(extradata, extradata_len, rows, cols, *rec, initial.data(), &init_bytes, why, sizeof why);
+    const int S = rec->slices();
+    cudaStream_t st = ctx->stream, cp = ctx->copy_stream;
+    auto &B = ctx->png;
+    using L = lm_ctx;
+    if (int rc = png_reserve(ctx, B[L::PNG_OFFS], (size_t)(n + 1) * sizeof(int64_t))) return rc;
+    int64_t *d_offs = reinterpret_cast<int64_t *>(B[L::PNG_OFFS].p);
+    CK(cudaMemcpyAsync(d_offs, offsets, (size_t)(n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+
+    // keyframe flags (each frame's first decision): they cut the video into GOPs, and every (GOP, slice) is a chain
+    std::vector<uint8_t> hdr_dev;
+    if (on_dev) {
+        if (int rc = png_reserve(ctx, B[L::PNG_HDR], (size_t)n * LM_PNG_HDR_BYTES)) return rc;
+        if (lm_launch_png_headers(payload, d_offs, 0, n, B[L::PNG_HDR].p, st) < 0) return fail(ctx, LM_ERR_RUNTIME, "FFV1 header launch failed");
+        hdr_dev.resize((size_t)n * LM_PNG_HDR_BYTES);
+        CK(cudaMemcpyAsync(hdr_dev.data(), B[L::PNG_HDR].p, hdr_dev.size(), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+    }
+    std::vector<int64_t> gop;  // first frame of every GOP, then n
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t len = offsets[i + 1] - offsets[i];
+        const bool key = on_dev ? ffv1::keyframe_bit(hdr_dev.data() + (size_t)i * LM_PNG_HDR_BYTES, std::min<int64_t>(len, LM_PNG_HDR_BYTES))
+                                : ffv1::keyframe_bit(payload + offsets[i], len);
+        if (i == 0 && !key) return fail(ctx, LM_ERR_INVALID, "frame 0: the first FFV1 frame is not a keyframe");
+        if (key) gop.push_back(i);
+    }
+    gop.push_back(n);
+    const int64_t ngop = (int64_t)gop.size() - 1;
+    std::vector<LmFfv1Chain> chains((size_t)(ngop * S));
+    for (int64_t g = 0; g < ngop; ++g)
+        for (int s = 0; s < S; ++s) chains[(size_t)(g * S + s)] = LmFfv1Chain{gop[g], (int32_t)(gop[g + 1] - gop[g]), s};
+
+    const int64_t ns = n * S;
+    if (int rc = png_reserve(ctx, B[L::PNG_STATUS], (size_t)ns * sizeof(int32_t))) return rc;
+    if (int rc = png_reserve(ctx, B[L::FFV1_SOFF], (size_t)ns * sizeof(int64_t))) return rc;
+    if (int rc = png_reserve(ctx, B[L::FFV1_SLEN], (size_t)ns * sizeof(int32_t))) return rc;
+    if (int rc = png_reserve(ctx, B[L::FFV1_CHAINS], chains.size() * sizeof(LmFfv1Chain))) return rc;
+    if (int rc = png_reserve(ctx, B[L::FFV1_REC], sizeof(ffv1::Record))) return rc;
+    if (int rc = png_reserve(ctx, B[L::FFV1_INIT], initial.size())) return rc;
+    int32_t *d_status = reinterpret_cast<int32_t *>(B[L::PNG_STATUS].p);
+    int64_t *d_soff = reinterpret_cast<int64_t *>(B[L::FFV1_SOFF].p);
+    int32_t *d_slen = reinterpret_cast<int32_t *>(B[L::FFV1_SLEN].p);
+    LmFfv1Chain *d_chains = reinterpret_cast<LmFfv1Chain *>(B[L::FFV1_CHAINS].p);
+    const ffv1::Record *d_rec = reinterpret_cast<const ffv1::Record *>(B[L::FFV1_REC].p);
+    CK(cudaMemsetAsync(d_status, 0xff, (size_t)ns * sizeof(int32_t), st));  // -1: not decoded
+    CK(cudaMemcpyAsync(B[L::FFV1_CHAINS].p, chains.data(), chains.size() * sizeof(LmFfv1Chain), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(B[L::FFV1_REC].p, rec.get(), sizeof(ffv1::Record), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(B[L::FFV1_INIT].p, initial.data(), initial.size(), cudaMemcpyHostToDevice, st));
+
+    // A host payload goes up in (at most) two pieces of whole GOPs, one per staging buffer: piece 0 is decoded on the
+    // library stream while piece 1 is copied, and piece 1 is decoded on the copy stream after its copy, concurrently.
+    struct Piece {
+        int64_t g0, g1;  // GOPs [g0, g1)
+    };
+    std::vector<Piece> pieces;
+    if (!on_dev && ngop >= 2) {
+        int64_t g = 1;
+        while (g + 1 < ngop && gop[g] < n / 2) ++g;
+        pieces.push_back({0, g});
+        pieces.push_back({g, ngop});
+    } else {
+        pieces.push_back({0, ngop});
+    }
+    // Chain work memory: in shared memory when the launch still fits in one wave that way, else in global slots
+    // (at most 2 GB per piece; more chains run as consecutive launches over the same slots).
+    const int64_t wb = (ffv1::work_bytes(*rec, cols) + 15) & ~(int64_t)15;
+    int dev_smem = 0, sm_smem = 0, n_sm = 0;
+    CK(cudaDeviceGetAttribute(&dev_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
+    CK(cudaDeviceGetAttribute(&sm_smem, cudaDevAttrMaxSharedMemoryPerMultiprocessor, ctx->device));
+    CK(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, ctx->device));
+    const int64_t smem_cta = (int64_t)lm_ffv1_smem_tables() + LM_FFV1_CHAINS_PER_CTA * wb;
+    const int64_t smem_wave = smem_cta <= dev_smem ? (int64_t)(sm_smem / (smem_cta + 1024)) * n_sm * LM_FFV1_CHAINS_PER_CTA : 0;
+    const int64_t slot_budget = (int64_t)2 << 30;
+    const int64_t batch = std::max<int64_t>(LM_FFV1_CHAINS_PER_CTA, slot_budget / wb / LM_FFV1_CHAINS_PER_CTA * LM_FFV1_CHAINS_PER_CTA);
+    if (!on_dev) {
+        for (size_t k = 0; k < pieces.size(); ++k) {
+            const size_t bytes = (size_t)(offsets[gop[pieces[k].g1]] - offsets[gop[pieces[k].g0]]);
+            if (int rc = png_reserve(ctx, B[L::PNG_STAGE0 + k], bytes)) return rc;
+        }
+        for (int k = 0; k < 2; ++k)
+            if (!ctx->ev_png_copy[k]) CK(cudaEventCreateWithFlags(&ctx->ev_png_copy[k], cudaEventDisableTiming));
+    }
+    std::vector<int> in_smem(pieces.size());
+    for (size_t k = 0; k < pieces.size(); ++k) {
+        const int64_t nch = (pieces[k].g1 - pieces[k].g0) * S;
+        in_smem[k] = nch <= smem_wave;
+        if (!in_smem[k])
+            if (int rc = png_reserve(ctx, B[L::FFV1_WORK0 + k], (size_t)(std::min(nch, batch) * wb))) return rc;
+    }
+    struct Events {  // uploads done, decode start, decode end
+        cudaEvent_t e[3] = {};
+        ~Events() {
+            for (cudaEvent_t x : e)
+                if (x) cudaEventDestroy(x);
+        }
+    } T;
+    for (auto &e : T.e) CK(cudaEventCreate(&e));
+    CK(cudaEventRecord(T.e[0], st));
+    for (size_t k = 0; k < pieces.size(); ++k) {
+        const Piece &P = pieces[k];
+        const int64_t f0 = gop[P.g0], f1 = gop[P.g1];
+        cudaStream_t ks = k ? cp : st;
+        const uint8_t *src = payload;
+        int64_t base = 0;
+        if (!on_dev) {
+            src = B[L::PNG_STAGE0 + k].p;
+            base = offsets[f0];
+            CK(cudaMemcpyAsync(B[L::PNG_STAGE0 + k].p, payload + base, (size_t)(offsets[f1] - base), cudaMemcpyHostToDevice, cp));
+            if (k == 0) {
+                CK(cudaEventRecord(ctx->ev_png_copy[0], cp));
+                CK(cudaStreamWaitEvent(st, ctx->ev_png_copy[0], 0));
+            } else {
+                CK(cudaStreamWaitEvent(cp, T.e[0], 0));  // the offsets, record and chain list are on the device
+            }
+        }
+        if (k == 0) CK(cudaEventRecord(T.e[1], st));
+        if (lm_launch_ffv1_locate(src, d_offs + f0, base, f1 - f0, S, rec->ec, d_soff + f0 * S, d_slen + f0 * S, d_status + f0 * S, ks) < 0 ||
+            (rec->ec && lm_launch_ffv1_crc(src, d_soff + f0 * S, d_slen + f0 * S, (f1 - f0) * S, d_status + f0 * S, ks) < 0))
+            return fail(ctx, LM_ERR_RUNTIME, "FFV1 slice launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        for (int64_t c0 = P.g0 * S; c0 < P.g1 * S; c0 += batch) {  // (slice offsets are relative to src: frames keep their numbers)
+            const int nch = (int)std::min<int64_t>(batch, P.g1 * S - c0);
+            if (lm_launch_ffv1_decode(d_rec, rec->ac, B[L::FFV1_INIT].p, src, d_soff, d_slen, d_status, frames, rows, cols, d_chains + c0, nch,
+                                      B[L::FFV1_WORK0 + k].p, wb, in_smem[k], ks) < 0)
+                return fail(ctx, LM_ERR_RUNTIME, "FFV1 decode launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        }
+    }
+    if (pieces.size() > 1) {
+        CK(cudaEventRecord(ctx->ev_png_copy[1], cp));
+        CK(cudaStreamWaitEvent(st, ctx->ev_png_copy[1], 0));
+    }
+    CK(cudaEventRecord(T.e[2], st));
+    std::vector<int32_t> status((size_t)ns);
+    CK(cudaMemcpyAsync(status.data(), d_status, (size_t)ns * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    float t = 0.f;
+    if (cudaEventElapsedTime(&t, T.e[1], T.e[2]) == cudaSuccess) ctx->ms_decode = t;
+    for (int64_t i = 0; i < ns; ++i)
+        if (status[i] != ffv1::LM_FFV1_OK)
+            return fail(ctx, LM_ERR_INVALID, "frame %lld, slice %d: %s", (long long)(i / S), (int)(i % S), ffv1::status_text(status[i]));
+    return LM_OK;
+}
+}  // namespace
+
+int lm_decode_ffv1(lm_ctx *ctx, const uint8_t *extradata, int64_t extradata_len, const uint8_t *payload, int payload_on_device,
+                   const int64_t *offsets, int64_t n, uint8_t *frames) {
+    if (!ctx) return LM_ERR_INVALID;
+    DeviceGuard guard(ctx->device);
+    const int rc = decode_ffv1_impl(ctx, extradata, extradata_len, payload, payload_on_device, offsets, n, frames);
+    if (rc != LM_OK) {  // nothing of this call may stay in flight: the caller's payload and frames would still be in use
+        cudaStreamSynchronize(ctx->copy_stream);
+        cudaStreamSynchronize(ctx->stream);
+        cudaGetLastError();
+    }
+    return rc;
+}
 
 int lm_decode_png(lm_ctx *ctx, const uint8_t *payload, int payload_on_device, const int64_t *offsets, int64_t n, uint8_t *frames) {
     if (!ctx) return LM_ERR_INVALID;

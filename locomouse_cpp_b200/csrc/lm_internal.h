@@ -217,6 +217,26 @@ int lm_launch_png_decode(const uint8_t *payload, const int64_t *offs, int64_t ba
 int lm_launch_png_headers(const uint8_t *payload, const int64_t *offs, int64_t base, int64_t n, uint8_t *hdr, cudaStream_t s);
 const char *lm_png_status_text(int st);
 
+// FFV1 frame decode (k_ffv1.cu, format in ffv1_format.h).  One (GOP, slice) chain: slice s of frames f0 .. f0 + nf - 1.
+namespace ffv1 {
+struct Record;
+}
+struct LmFfv1Chain {
+    int64_t f0;
+    int32_t nf, s;
+};
+constexpr int LM_FFV1_CHAINS_PER_CTA = 32;
+size_t lm_ffv1_smem_tables();  // shared memory of the record's tables in k_ffv1_decode
+// Slice f * S + s of frame f (payload[offs[f] - base, offs[f + 1] - base)) is located at payload + soff[.], slen[.] bytes;
+// a broken footer chain sets status[.] = LM_FFV1_FOOTER for the whole frame.
+int lm_launch_ffv1_locate(const uint8_t *payload, const int64_t *offs, int64_t base, int64_t n, int S, int ec, int64_t *soff, int32_t *slen,
+                          int32_t *status, cudaStream_t s);
+int lm_launch_ffv1_crc(const uint8_t *payload, const int64_t *soff, const int32_t *slen, int64_t ns, int32_t *status, cudaStream_t s);
+// work: work_bytes per chain (global slots, or shared memory when work_in_smem)
+int lm_launch_ffv1_decode(const ffv1::Record *rec, int ac, const uint8_t *initial, const uint8_t *payload, const int64_t *soff,
+                          const int32_t *slen, int32_t *status, uint8_t *out, int rows, int cols, const LmFfv1Chain *chains, int nchains,
+                          uint8_t *work, int64_t work_bytes, int work_in_smem, cudaStream_t s);
+
 // pick the padded kernel-row width the correlation kernel is instantiated for (>= kw), or -1
 int lm_corr_kwp(int kw);
 // dynamic shared memory the correlation kernel needs for a view/template (for capability checks)

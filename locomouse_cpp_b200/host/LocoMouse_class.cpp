@@ -302,9 +302,11 @@ void LocoMouse::loadVideo() {
         N_FRAMES = (unsigned int)V.n;
         VID_ROWS = V.rows;
         VID_COLS = V.cols;
-        if (V.png) {  // decoded on the device once lm_configure has run (configureDevice)
-            PNG_PAYLOAD = V.payload;
-            PNG_OFFSETS = std::move(V.offsets);
+        if (V.codec != lmmedia::Codec::raw) {  // decoded on the device once lm_configure has run (configureDevice)
+            CODEC = V.codec;
+            CODED_PAYLOAD = V.payload;
+            CODED_OFFSETS = std::move(V.offsets);
+            CODED_EXTRADATA = std::move(V.extradata);
             return;
         }
         VIDEO.resize(V.frames.size());
@@ -637,14 +639,18 @@ void LocoMouse::configureDevice() {
     check(lm_configure(CTX, &c));
     check(lm_set_background(CTX, BKG.data()));
     check(lm_set_calibration(CTX, CALIBRATION.data()));
-    if (PNG_PAYLOAD && !D_VIDEO) {  // the whole PNG-coded video, decoded once; pass 1 and the frame loop read it in place
+    if (CODED_PAYLOAD && !D_VIDEO) {  // the whole compressed video, decoded once; pass 1 and the frame loop read it in place
         const size_t bytes = (size_t)N_FRAMES * VID_ROWS * VID_COLS;
         void *d = nullptr;
         if (lm_device_alloc(CTX, &d, bytes) != LM_OK)
             throw std::runtime_error("The decoded video (" + std::to_string(N_FRAMES) + " frames, " + std::to_string(bytes) +
                                      " bytes) does not fit in device memory: " + lm_last_error(CTX));
         D_VIDEO = static_cast<uint8_t *>(d);
-        check(lm_decode_png(CTX, PNG_PAYLOAD.get(), 0, PNG_OFFSETS.data(), N_FRAMES, D_VIDEO));
+        if (CODEC == lmmedia::Codec::png)
+            check(lm_decode_png(CTX, CODED_PAYLOAD.get(), 0, CODED_OFFSETS.data(), N_FRAMES, D_VIDEO));
+        else
+            check(lm_decode_ffv1(CTX, CODED_EXTRADATA.data(), (int64_t)CODED_EXTRADATA.size(), CODED_PAYLOAD.get(), 0, CODED_OFFSETS.data(),
+                                 N_FRAMES, D_VIDEO));
     }
 }
 

@@ -20,6 +20,7 @@
 #include "Candidates.hpp"
 #include "LocoMouse_ParseInputs.hpp"
 #include "MyMat.hpp"
+#include "lm_media.hpp"
 
 // LocoMouse_Parameters (class.hpp:48-100): the subset that reaches the detection path, plus the
 // inputs that replace the out-of-scope pass 1 (SURVEY §8f-1): per-frame box positions from a file.
@@ -151,10 +152,13 @@ protected:
     std::string output_file;
 
     PinnedArray<uint8_t> VIDEO;       // raw 8-bit frames (channel 0), N_FRAMES x vid_rows x vid_cols, page-locked
-    // PNG-coded AVI: the frame chunks (page-locked, frame i = [PNG_OFFSETS[i], PNG_OFFSETS[i + 1])), decoded once by
-    // configureDevice into D_VIDEO (device memory, same layout as VIDEO); VIDEO stays empty
-    std::shared_ptr<uint8_t> PNG_PAYLOAD;
-    std::vector<int64_t> PNG_OFFSETS;
+    // PNG- or FFV1-coded AVI: the frame chunks (page-locked, frame i = [CODED_OFFSETS[i], CODED_OFFSETS[i + 1])) and, for
+    // FFV1, the configuration record; decoded once by configureDevice into D_VIDEO (device memory, same layout as VIDEO);
+    // VIDEO stays empty
+    lmmedia::Codec CODEC = lmmedia::Codec::raw;
+    std::shared_ptr<uint8_t> CODED_PAYLOAD;
+    std::vector<int64_t> CODED_OFFSETS;
+    std::vector<uint8_t> CODED_EXTRADATA;
     uint8_t *D_VIDEO = nullptr;
     int VID_ROWS = 0, VID_COLS = 0;
     std::vector<uint8_t> BKG;
@@ -201,7 +205,7 @@ protected:
     void check(int rc) const;          // lm_status -> exception
     void runChunk(unsigned int first_frame);
     void configureDevice();            // lm_configure + background + calibration for the current box sizes
-    const uint8_t *frames(int &on_device) const;  // first frame of the video: VIDEO, or D_VIDEO for PNG-coded video
+    const uint8_t *frames(int &on_device) const;  // first frame of the video: VIDEO, or D_VIDEO for compressed video
     const Batch &batchFor(int frame) const;
     virtual bool usesImadjust() const { return false; }  // LocoMouse_TM::readFrame applies imadjust(0, 0.6)
     // class.cpp:2221-2346, 2385-2482

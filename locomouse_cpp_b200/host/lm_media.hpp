@@ -5,8 +5,10 @@
 // 'GREY' / 'Y8  ', what cv2.VideoWriter(fourcc = 0, isColor = False) writes), BI_RGB 8-bit with a palette, BI_RGB 24- / 32-bit
 // (channel 0 = blue, as extractChannel takes it).  PNG-coded streams ('MPNG' / 'png ', lossless, what cv2.VideoWriter writes
 // with those fourccs) are not decoded here: their frame chunks -- each a complete PNG file -- are returned as one payload with
-// offsets, for lm_decode_png to decode on the device.  Other compressed or YUV-planar streams need a decoder that is outside
-// this library: they are refused with a message that says so.  Background: PNG, 8 bits per channel, non-interlaced; colour images are
+// offsets, for lm_decode_png to decode on the device.  FFV1-coded streams ('FFV1', lossless, version 3 as libavcodec writes
+// it) are returned the same way, with the configuration record from 'strf' as extradata, for lm_decode_ffv1; the record is
+// checked here (ffv1_format.h) and so is every frame's keyframe bit.  Other compressed or YUV-planar streams need a decoder
+// that is outside this library: they are refused with a message that says so.  Background: PNG, 8 bits per channel, non-interlaced; colour images are
 // reduced to grey as libpng does for OpenCV (png_set_rgb_to_gray with 0.299 / 0.587).  Both are checked against what the
 // real OpenCV reads from the same files (tests/test_host_media.py).
 #pragma once
@@ -19,6 +21,8 @@
 #include <stdexcept>
 #include <string>
 #include <vector>
+
+#include "../csrc/ffv1_format.h"
 
 namespace lmmedia {
 
@@ -53,13 +57,17 @@ struct HostAlloc {
     void (*release)(void *) = [](void *p) { std::free(p); };
 };
 
+enum class Codec { raw, png, ffv1 };
+
 struct Video {
     int n = 0, rows = 0, cols = 0;
     std::vector<uint8_t> frames;  // channel 0 of every frame, [n][rows][cols] (uncompressed streams)
-    // PNG-coded streams: frame i = payload[offsets[i], offsets[i + 1]), a complete PNG file; `frames` stays empty
-    bool png = false;
+    // Compressed streams: frame i = payload[offsets[i], offsets[i + 1]), one frame chunk (a complete PNG file, or one FFV1
+    // frame whose configuration record is `extradata`); `frames` stays empty
+    Codec codec = Codec::raw;
     std::shared_ptr<uint8_t> payload;
     std::vector<int64_t> offsets;
+    std::vector<uint8_t> extradata;
 };
 
 // Signature and IHDR of one PNG frame: 8-bit grey / RGB / RGBA, not interlaced (what lm_decode_png decodes)
@@ -100,7 +108,8 @@ inline Video read_avi(const std::string &name, const HostAlloc &halloc = HostAll
     bool have_format = false, stream0_is_video = false;
     int stream_index = -1;
     std::vector<uint8_t> chunk;
-    std::vector<std::pair<int64_t, uint32_t>> png_chunks;  // file offset and size of every PNG frame chunk
+    std::vector<std::pair<int64_t, uint32_t>> coded_chunks;  // file offset and size of every PNG / FFV1 frame chunk
+    std::vector<uint8_t> extradata;
     // A flat walk: LIST / RIFF headers are entered (only their 4-byte type is consumed), every other chunk is read or skipped.
     for (;;) {
         uint8_t ch[8];
@@ -132,6 +141,7 @@ inline Video read_avi(const std::string &name, const HostAlloc &halloc = HostAll
             bits = chunk[14] | (chunk[15] << 8);
             fourcc = le32(chunk.data() + 16);
             const uint32_t used = le32(chunk.data() + 32);
+            extradata.assign(chunk.begin() + 40, chunk.end());
             const size_t ncol = used ? used : (bits <= 8 ? (size_t)1 << bits : 0);
             for (size_t i = 0; i < ncol && 40 + 4 * i + 3 < size && i < 256; ++i) palette_b[i] = chunk[40 + 4 * i];  // RGBQUAD: blue first
             have_format = true;
@@ -146,10 +156,12 @@ inline Video read_avi(const std::string &name, const HostAlloc &halloc = HostAll
         auto cc = [](const char *s) { return le32(reinterpret_cast<const uint8_t *>(s)); };
         const bool grey = fourcc == cc("Y800") || fourcc == cc("GREY") || fourcc == cc("Y8  ") || fourcc == cc("Y8\0\0");
         const bool rgb = fourcc == 0 || fourcc == cc("DIB ") || fourcc == cc("RGB ") || fourcc == cc("RAW ");
-        if (fourcc == cc("MPNG") || fourcc == cc("png ")) {  // read after the walk, straight into the payload
+        const bool png = fourcc == cc("MPNG") || fourcc == cc("png ");
+        if (png || fourcc == cc("FFV1")) {  // read after the walk, straight into the payload
             if (size == 0) continue;
+            V.codec = png ? Codec::png : Codec::ffv1;
             const off_t at = ftello(f);
-            png_chunks.emplace_back((int64_t)at, size);
+            coded_chunks.emplace_back((int64_t)at, size);
             if (!skip((uint64_t)size + (size & 1))) fail("truncated frame");
             continue;
         }
@@ -184,19 +196,27 @@ inline Video read_avi(const std::string &name, const HostAlloc &halloc = HostAll
         }
         ++V.n;
     }
-    if (!png_chunks.empty()) {
+    if (V.codec == Codec::ffv1) {
+        ffv1::Record rec;
+        char why[200];
+        if (ffv1::parse_record(extradata.data(), (int64_t)extradata.size(), V.rows, V.cols, rec, nullptr, nullptr, why, sizeof why))
+            fail(std::string("FFV1 configuration record: ") + why);
+        V.extradata = std::move(extradata);
+    }
+    if (!coded_chunks.empty()) {
         uint64_t total = 0;
-        for (const auto &c : png_chunks) total += c.second;
+        for (const auto &c : coded_chunks) total += c.second;
         uint8_t *buf = static_cast<uint8_t *>(halloc.alloc((size_t)total));
         if (!buf) fail("cannot allocate " + std::to_string(total) + " bytes for the compressed frames");
         V.payload = std::shared_ptr<uint8_t>(buf, halloc.release);
-        V.png = true;
         V.offsets.push_back(0);
-        V.rows = V.cols = 0;  // taken from frame 0's IHDR
-        for (const auto &c : png_chunks) {
+        if (V.codec == Codec::png) V.rows = V.cols = 0;  // taken from frame 0's IHDR
+        for (const auto &c : coded_chunks) {
             uint8_t *d = buf + V.offsets.back();
             if (fseeko(f, (off_t)c.first, SEEK_SET) != 0 || !rd(d, c.second)) fail("truncated frame");
-            check_png_frame(d, c.second, V.rows, V.cols, "Video file " + name + ", frame " + std::to_string(V.n));
+            const std::string where = "Video file " + name + ", frame " + std::to_string(V.n);
+            if (V.codec == Codec::png) check_png_frame(d, c.second, V.rows, V.cols, where);
+            else if (V.n == 0 && !ffv1::keyframe_bit(d, c.second)) throw std::runtime_error(where + ": the first FFV1 frame is not a keyframe");
             V.offsets.push_back(V.offsets.back() + c.second);
             ++V.n;
         }

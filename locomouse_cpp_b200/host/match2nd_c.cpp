@@ -2,6 +2,7 @@
 // packed arrays, exactly what lm_unary_costs / lm_pairwise_costs return and what the reference-compiled checker
 // (oracle/ref_glue.cpp: ref_match2nd) takes, so both are driven with identical inputs.
 #include <cstdint>
+#include <memory>
 #include <vector>
 
 #include "cv_yaml.hpp"
@@ -88,7 +89,8 @@ int lmh_yaml_write(const char *path, const char *names, int n, const int32_t *ro
 int lmh_read_avi(const char *path, int32_t *dims, uint8_t *out, char *msg, int msg_cap) {
     try {
         const lmmedia::Video V = lmmedia::read_avi(path);
-        if (V.png) throw std::runtime_error(std::string("Video file ") + path + ": PNG-coded stream (lmh_read_avi_png)");
+        if (V.codec == lmmedia::Codec::png) throw std::runtime_error(std::string("Video file ") + path + ": PNG-coded stream (lmh_read_avi_png)");
+        if (V.codec == lmmedia::Codec::ffv1) throw std::runtime_error(std::string("Video file ") + path + ": FFV1-coded stream (lmh_read_avi_ffv1)");
         dims[0] = V.n;
         dims[1] = V.rows;
         dims[2] = V.cols;
@@ -104,7 +106,7 @@ int lmh_read_avi(const char *path, int32_t *dims, uint8_t *out, char *msg, int m
 int lmh_read_avi_png(const char *path, int64_t *dims, uint8_t *payload, int64_t *offsets, char *msg, int msg_cap) {
     try {
         const lmmedia::Video V = lmmedia::read_avi(path);
-        if (!V.png) throw std::runtime_error(std::string("Video file ") + path + ": not a PNG-coded stream");
+        if (V.codec != lmmedia::Codec::png) throw std::runtime_error(std::string("Video file ") + path + ": not a PNG-coded stream");
         dims[0] = V.n;
         dims[1] = V.rows;
         dims[2] = V.cols;
@@ -116,6 +118,83 @@ int lmh_read_avi_png(const char *path, int64_t *dims, uint8_t *payload, int64_t 
         if (msg && msg_cap > 0) std::snprintf(msg, (size_t)msg_cap, "%s", e.what());
         return 1;
     }
+}
+// FFV1-coded AVI: dims = {n, rows, cols, payload bytes, extradata bytes}; with payload / offsets / extradata NULL only the
+// dimensions are returned.  0 ok, 1 error (msg filled)
+int lmh_read_avi_ffv1(const char *path, int64_t *dims, uint8_t *payload, int64_t *offsets, uint8_t *extradata, char *msg, int msg_cap) {
+    try {
+        const lmmedia::Video V = lmmedia::read_avi(path);
+        if (V.codec != lmmedia::Codec::ffv1) throw std::runtime_error(std::string("Video file ") + path + ": not an FFV1-coded stream");
+        dims[0] = V.n;
+        dims[1] = V.rows;
+        dims[2] = V.cols;
+        dims[3] = V.offsets.back();
+        dims[4] = (int64_t)V.extradata.size();
+        if (payload) std::memcpy(payload, V.payload.get(), (size_t)V.offsets.back());
+        if (offsets) std::memcpy(offsets, V.offsets.data(), V.offsets.size() * sizeof(int64_t));
+        if (extradata) std::memcpy(extradata, V.extradata.data(), V.extradata.size());
+        return 0;
+    } catch (const std::exception &e) {
+        if (msg && msg_cap > 0) std::snprintf(msg, (size_t)msg_cap, "%s", e.what());
+        return 1;
+    }
+}
+// ffv1_format.h run serially on the CPU: the record parse and the chain decode that k_ffv1.cu runs per thread, for the CPU
+// tests.  out: [n][rows][cols].  0 ok, 1 error (msg names the record problem, or the first bad frame and slice)
+int lmh_decode_ffv1(const uint8_t *extradata, int64_t extradata_len, const uint8_t *payload, const int64_t *offsets, int64_t n, int rows,
+                    int cols, uint8_t *out, char *msg, int msg_cap) {
+    auto *rec = new ffv1::Record;
+    std::unique_ptr<ffv1::Record> hold(rec);
+    char why[200];
+    int64_t ib = 0;
+    if (ffv1::parse_record(extradata, extradata_len, rows, cols, *rec, nullptr, &ib, why, sizeof why)) {
+        std::snprintf(msg, (size_t)msg_cap, "%s", why);
+        return 1;
+    }
+    std::vector<uint8_t> initial((size_t)ib);
+    ffv1::parse_record(extradata, extradata_len, rows, cols, *rec, initial.data(), &ib, why, sizeof why);
+    const int S = rec->slices();
+    std::vector<int64_t> soff((size_t)(n * S));
+    std::vector<int32_t> slen((size_t)(n * S)), status((size_t)(n * S), -1);
+    uint32_t ct[256];
+    ffv1::crc_table(ct);
+    for (int64_t f = 0; f < n; ++f) {
+        const uint8_t *fr = payload + offsets[f];
+        if (ffv1::locate_slices(fr, offsets[f + 1] - offsets[f], S, rec->ec, &soff[f * S], &slen[f * S])) {
+            for (int s = 0; s < S; ++s) status[f * S + s] = ffv1::LM_FFV1_FOOTER;
+            continue;
+        }
+        for (int s = 0; s < S; ++s) {
+            soff[f * S + s] += offsets[f];
+            uint32_t crc = 0;
+            for (int32_t i = 0; rec->ec && i < slen[f * S + s]; ++i) crc = ffv1::crc_update(ct, crc, payload[soff[f * S + s] + i]);
+            if (crc) status[f * S + s] = ffv1::LM_FFV1_CRC;
+        }
+    }
+    std::vector<uint64_t> work((size_t)(ffv1::work_bytes(*rec, cols) + 7) / 8);
+    for (int64_t f0 = 0; f0 < n;) {
+        int64_t f1 = f0 + 1;
+        while (f1 < n && !ffv1::keyframe_bit(payload + offsets[f1], offsets[f1 + 1] - offsets[f1])) ++f1;
+        if (f0 == 0 && !ffv1::keyframe_bit(payload, offsets[1] - offsets[0])) {
+            std::snprintf(msg, (size_t)msg_cap, "frame 0 is not a keyframe");
+            return 1;
+        }
+        for (int s = 0; s < S; ++s) {
+            if (rec->ac)
+                ffv1::decode_chain<true>(*rec, rec->t, initial.data(), payload, soff.data(), slen.data(), status.data(), out, rows, cols, f0,
+                                         (int)(f1 - f0), s, reinterpret_cast<uint8_t *>(work.data()));
+            else
+                ffv1::decode_chain<false>(*rec, rec->t, initial.data(), payload, soff.data(), slen.data(), status.data(), out, rows, cols, f0,
+                                          (int)(f1 - f0), s, reinterpret_cast<uint8_t *>(work.data()));
+        }
+        f0 = f1;
+    }
+    for (int64_t i = 0; i < n * S; ++i)
+        if (status[i]) {
+            std::snprintf(msg, (size_t)msg_cap, "frame %lld, slice %d: %s", (long long)(i / S), (int)(i % S), ffv1::status_text(status[i]));
+            return 1;
+        }
+    return 0;
 }
 int lmh_read_png(const char *path, int32_t *dims, uint8_t *out, char *msg, int msg_cap) {
     try {
