@@ -75,7 +75,8 @@ def test_screen_large_batch_property():
 def test_screen_dense_threshold_and_degenerate_templates(oracle):
     """Stress the decision thresholds: (a) biases lowered so that a large share of all outputs is positive (many
     survivors, overflow allowed), (b) an all-zero template with rho = 0 (every score is exactly -0.0 -> no
-    detection, quantisation scale degenerate), (c) rho exactly at a representable score level."""
+    detection, quantisation scale degenerate).  Outputs placed exactly on the screen's thresholds, and scores of exactly 0
+    and the smallest subnormal, are in tests/test_gpu_designed_frames.py."""
     def lower_rho(m):
         return Model(w=m.w, rho=[[r * 0.25 for r in row] for row in m.rho])
 
