@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define LM_ABI_VERSION 5  /* 5: lm_bounding_box_tm, and (backward compatible additions) lm_decode_png, lm_decode_ffv1, lm_device_alloc / lm_device_free, lm_get_info("ms_decode"); 4: lm_bounding_box_base, lm_mouse_box_size; 2: lm_set_option, lm_get_info, lm_debug_nms, lm_bounding_box_tm_de, lm_moving_average; 3: lm_host_alloc / lm_host_free, lm_unary_costs / lm_pairwise_costs, options streams 1..4, screen_layout, screen_priority */
+#define LM_ABI_VERSION 5  /* 5: lm_bounding_box_tm, and (backward compatible additions) lm_decode_png, lm_decode_ffv1, lm_device_alloc / lm_device_free, lm_get_info("ms_decode"), lm_get_info("device_allocs"); 4: lm_bounding_box_base, lm_mouse_box_size; 2: lm_set_option, lm_get_info, lm_debug_nms, lm_bounding_box_tm_de, lm_moving_average; 3: lm_host_alloc / lm_host_free, lm_unary_costs / lm_pairwise_costs, options streams 1..4, screen_layout, screen_priority */
 
 /* feature / view indices used in every [2] / [3] array below */
 enum { LM_PAW = 0, LM_SNOUT = 1, LM_TAIL = 2 };
@@ -108,7 +108,13 @@ typedef struct {
 
 typedef struct lm_ctx lm_ctx;
 
-/* lifetime ------------------------------------------------------------------------------- */
+/* lifetime ------------------------------------------------------------------------------- *
+ * Concurrency: different contexts may be used concurrently from different host threads, also on the same device; a context
+ * waits only for its own streams (no call synchronises the whole device), and the library's per-device one-time set-up is
+ * thread-safe.  One context is used by one thread at a time (it may move between threads between calls).
+ * Re-configuration keeps the context's device allocations: lm_configure / lm_set_model / lm_set_option only mark the
+ * scratch free, and the next call that needs scratch re-derives the layout from the new geometry and reuses every block
+ * that is large enough; it allocates (and returns the blocks it no longer fits to the driver) only when the geometry grew. */
 int lm_abi_version(void);
 int lm_create(lm_ctx **out, int device);            /* binds a CUDA device, creates streams   */
 int lm_destroy(lm_ctx *ctx);
@@ -165,7 +171,10 @@ int lm_detect_batch(lm_ctx *ctx, const uint8_t *frames, int frames_on_device,
  * lm_get_info: "screen_active" (2/1/0 after the first lm_detect_batch, -1 before), "subbatch", "ms_screen"
  *             (device ms of the tensor-core kernel alone in the last call; ms[2] of lm_last_timing = screen + exact pass),
  *             "screen_eps_<view><feat>" / "screen_scale_<view><feat>" (error bound / weight quantum), "screen_macs" (int8
- *             multiply-accumulates the last CTA-pair screen launch issued: executed work, beside the algorithmic count). */
+ *             multiply-accumulates the last CTA-pair screen launch issued: executed work, beside the algorithmic count),
+ *             "device_allocs" (cudaMalloc calls this context has made so far; each one waits for the whole device, so a context
+ *             re-configured for a video of the same geometry makes none; the stream-ordered allocations of lm_bounding_box_base /
+ *             _tm / _tm_de and of the cost builders are not counted). */
 int lm_set_option(lm_ctx *ctx, const char *name, int64_t value);
 int lm_get_info(const lm_ctx *ctx, const char *name, double *value);
 

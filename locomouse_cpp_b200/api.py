@@ -126,8 +126,13 @@ class Detector:
             msg = self._L.lm_last_error(None).decode()
             self._ctx = C.c_void_p()
             raise RuntimeError(f"lm_create failed ({rc}): {msg}")
-        self.cfg = cfg
         self.device = int(device)
+        self.configure(cfg, model, bkg, calib)
+
+    def configure(self, cfg: Config, model: Model, bkg, calib):
+        """Re-configures the context for another video (lm_configure + model, background and calibration); its device
+        allocations are kept and reused wherever they are large enough."""
+        self.cfg = cfg
         c = cfg.to_c()
         self._check(self._L.lm_configure(self._ctx, C.byref(c)))
         self.set_model(model)

@@ -315,7 +315,7 @@ int lm_launch_bbox_base(const LmBatch &b, const lm_bb_base_params &p, uint32_t *
     if (const char *e = getenv("LM_BBOX_RUNCAP")) runcap = std::max(0, std::min(runcap, atoi(e)));
     P.runcap = std::max(runcap, 0);
     static LmDevOnce once;
-    if (once.first()) {
+    if (auto setup = once.first()) {
         if (cudaFuncSetAttribute(k_bbb_cc, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_cc) != cudaSuccess) return -1;
         if (cudaFuncSetAttribute(k_bbb_cc_slow, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_slow) != cudaSuccess) return -1;
     }

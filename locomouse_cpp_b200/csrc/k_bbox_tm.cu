@@ -494,7 +494,7 @@ int lm_launch_bbox_tm(const LmBatch &b, const lm_bb_tm_params &p, const float *d
     if (const char *e = getenv("LM_BBOX_RUNCAP")) runcap = std::max(0, std::min(runcap, atoi(e)));
     P.runcap = std::max(runcap, 0);
     static LmDevOnce once;
-    if (once.first()) {
+    if (auto setup = once.first()) {
         if (cudaFuncSetAttribute(k_bbtm_open<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, budget) != cudaSuccess ||
             cudaFuncSetAttribute(k_bbtm_open<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, budget) != cudaSuccess ||
             cudaFuncSetAttribute(k_bbtm_fill<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, budget) != cudaSuccess ||

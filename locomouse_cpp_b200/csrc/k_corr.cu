@@ -274,16 +274,16 @@ template <int KW>
 cudaError_t launch_kw(const CorrParams &P, size_t smem, bool fma, cudaStream_t s) {
     auto kf = k_corr<KW, kTX, kTY, true>;
     auto km = k_corr<KW, kTX, kTY, false>;
-    cudaError_t e;
-    if (fma) {
-        e = cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    static LmDevOnce once;
+    if (auto setup = once.first()) {
+        cudaError_t e = lm_allow_max_dynamic_smem(kf);
+        if (e == cudaSuccess) e = lm_allow_max_dynamic_smem(km);
         if (e != cudaSuccess) return e;
-        kf<<<P.B * P.ctas_per_frame, CORR_THREADS, smem, s>>>(P);
-    } else {
-        e = cudaFuncSetAttribute(km, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        km<<<P.B * P.ctas_per_frame, CORR_THREADS, smem, s>>>(P);
     }
+    if (fma)
+        kf<<<P.B * P.ctas_per_frame, CORR_THREADS, smem, s>>>(P);
+    else
+        km<<<P.B * P.ctas_per_frame, CORR_THREADS, smem, s>>>(P);
     return cudaGetLastError();
 }
 

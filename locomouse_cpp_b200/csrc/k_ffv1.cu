@@ -102,7 +102,9 @@ int lm_launch_ffv1_decode(const ffv1::Record *rec, int ac, const uint8_t *initia
     if (nchains <= 0) return 0;
     const size_t smem = sizeof(ffv1::Tables) + (work_in_smem ? (size_t)LM_FFV1_CHAINS_PER_CTA * work_bytes : 0);
     auto kern = ac ? k_ffv1_decode<true> : k_ffv1_decode<false>;
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -1;
+    static LmDevOnce once;
+    if (auto setup = once.first())
+        if (lm_allow_max_dynamic_smem(k_ffv1_decode<true>) != cudaSuccess || lm_allow_max_dynamic_smem(k_ffv1_decode<false>) != cudaSuccess) return -1;
     const unsigned blocks = (unsigned)((nchains + LM_FFV1_CHAINS_PER_CTA - 1) / LM_FFV1_CHAINS_PER_CTA);
     kern<<<blocks, LM_FFV1_CHAINS_PER_CTA, smem, s>>>(rec, initial, payload, soff, slen, status, out, rows, cols, chains, nchains, work,
                                                       work_bytes, work_in_smem);

@@ -406,7 +406,7 @@ __global__ void __launch_bounds__(NMS_T) k_nms_side(const __grid_constant__ LmBa
 
 int lm_launch_nms(const LmBatch &b, cudaStream_t s) {
     static LmDevOnce once;
-    if (once.first()) {
+    if (auto setup = once.first()) {
         lm_prefer_max_shared(k_nms_bottom);
         lm_prefer_max_shared(k_nms_side);
     }

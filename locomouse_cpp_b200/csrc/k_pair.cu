@@ -187,7 +187,7 @@ int lm_launch_pair(const LmBatch &b, cudaStream_t s) {
     const size_t per_warp = (size_t)b.cand_cap * (sizeof(double) + 6 * sizeof(int));
     const int units = b.B * 2;
     static LmDevOnce once;  // cand_cap > 384 needs more than the default 48 kB of dynamic shared memory
-    if (once.first()) {
+    if (auto setup = once.first()) {
         if (cudaFuncSetAttribute(k_pair, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024) != cudaSuccess) return -1;
         lm_prefer_max_shared(k_pair);
     }

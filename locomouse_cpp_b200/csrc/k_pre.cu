@@ -339,7 +339,7 @@ int lm_launch_minmax(const LmBatch &b, cudaStream_t s) {
     const bool aligned = (b.frame_bytes & 15) == 0 && (reinterpret_cast<uintptr_t>(b.frames) & 15) == 0 && (reinterpret_cast<uintptr_t>(b.bkg) & 15) == 0 &&
                          (b.prev == nullptr || (reinterpret_cast<uintptr_t>(b.prev) & 15) == 0);
     static LmDevOnce once;
-    if (once.first()) {
+    if (auto setup = once.first()) {
         lm_prefer_max_shared(k_minmax<true>);
         lm_prefer_max_shared(k_minmax<false>);
         lm_prefer_max_shared(k_lut);
@@ -357,7 +357,7 @@ int lm_launch_prep(const LmBatch &b, cudaStream_t s) {
     for (int v = 0; v < 2; ++v) maxh = b.view[v].win_h > maxh ? b.view[v].win_h : maxh;
     const int bx = (maxh + PREP_ROWS - 1) / PREP_ROWS;
     static LmDevOnce once;
-    if (once.first()) lm_prefer_max_shared(k_prep);
+    if (auto setup = once.first()) lm_prefer_max_shared(k_prep);
     k_prep<<<dim3(bx < 1 ? 1 : bx, b.B, 2), PREP_THREADS, 0, s>>>(b);
     return 1;
 }

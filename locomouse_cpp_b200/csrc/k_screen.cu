@@ -467,7 +467,7 @@ __global__ void __launch_bounds__(SP_THREADS) k_corr_sparse(const __grid_constan
 template <int KW>
 cudaError_t launch_sparse_kw(const SparseParams &P, dim3 grid, size_t smem, bool fma, cudaStream_t s) {
     static LmDevOnce once;
-    if (once.first()) {
+    if (auto setup = once.first()) {
         lm_prefer_max_shared(k_corr_sparse<KW, true>);
         lm_prefer_max_shared(k_corr_sparse<KW, false>);
     }
@@ -663,7 +663,7 @@ int lm_launch_screen(const LmBatch &b, cudaStream_t s) {
 
     if (cudaMemsetAsync(b.scr.ntasks, 0, 16 * sizeof(int), s) != cudaSuccess) return -1;
     static LmDevOnce once;
-    if (once.first()) {
+    if (auto setup = once.first()) {
         if (cudaFuncSetAttribute(k_screen, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024) != cudaSuccess) return -1;
     }
     if (b.scr.enabled == 2) {

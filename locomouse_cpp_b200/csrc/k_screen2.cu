@@ -451,13 +451,13 @@ size_t lm_screen2_smem_bytes(int KH, int ks, int rows, int nhalf, int stages) {
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
                                   const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 static EncodeTiledFn encode_tiled_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
+    static const EncodeTiledFn fn = [] {  // initialised once, also when several host threads launch at once
         void *p = nullptr;
         cudaDriverEntryPointQueryResult q;
         if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<EncodeTiledFn>(p);
-    }
+            return reinterpret_cast<EncodeTiledFn>(p);
+        return (EncodeTiledFn) nullptr;
+    }();
     return fn;
 }
 // One K panel of a window tile = a box of 16 bytes x `rows` rows; out-of-range rows / columns / frames read as zero.
@@ -478,11 +478,6 @@ static bool encode_window_map(CUtensorMap *tm, const uint8_t *win, int pitch, in
     return enc(tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<uint8_t *>(win), dim, str, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
-
-// int8 multiply-accumulates the last launch issued to the tensor cores (all instructions: M = 256 x N x K = 32 each), for
-// bench.py's executed-work figure beside the algorithmic one
-static std::atomic<long long> g_last_macs{0};
-long long lm_screen2_last_macs() { return g_last_macs.load(); }
 
 // Launches k_screen2 for the pair-level jobs; the caller has zeroed the task counters.
 int lm_launch_screen2_kernel(const LmBatch &b, cudaStream_t s) {
@@ -559,7 +554,7 @@ int lm_launch_screen2_kernel(const LmBatch &b, cudaStream_t s) {
     }
     static_assert(sizeof(Screen2Params) <= 4000, "kernel parameter space");
     static LmDevOnce once;
-    if (once.first()) {
+    if (auto setup = once.first()) {
         if (cudaFuncSetAttribute(k_screen2, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024) != cudaSuccess) return -1;
     }
     if (P.whatif & 64) {
@@ -569,7 +564,9 @@ int lm_launch_screen2_kernel(const LmBatch &b, cudaStream_t s) {
                     J.j.view, J.j.ntmpl, J.j.KH, J.j.ks, J.j.rows, J.j.nhalf, J.j.nhalf_narrow, J.j.narrow_x0, J.nxt, J.ntp, J.VH, J.npair, J.j.stages, J.j.stacked, smem);
         }
     }
-    g_last_macs.store(macs);
+    // int8 multiply-accumulates this launch issues to the tensor cores (all instructions: M = 256 x N x K = 32 each), for
+    // bench.py's executed-work figure beside the algorithmic one
+    if (b.screen_macs) *b.screen_macs = macs;
     const int pairs = P.job[P.njobs - 1].pair_begin + P.job[P.njobs - 1].npair;
     k_screen2<<<2 * pairs, S2_THREADS, smem, s>>>(P);
     if (P.whatif & 128) {

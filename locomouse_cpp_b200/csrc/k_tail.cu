@@ -207,7 +207,7 @@ size_t tail_smem(const LmBatch &b, int runcap) {
 int lm_launch_tail(const LmBatch &b, cudaStream_t s) {
     if (b.tail_w <= 0) return 0;
     static LmDevOnce once;
-    if (once.first()) {
+    if (auto setup = once.first()) {
         cudaFuncSetAttribute(k_tail, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         lm_prefer_max_shared(k_tail);
         lm_prefer_max_shared(k_tail_slow);

@@ -48,8 +48,9 @@ struct lm_ctx {
     LmGeom geom{};
     std::string err;
 
-    uint8_t *d_bkg = nullptr;
+    uint8_t *d_bkg = nullptr;         // d_bkg / d_calib / d_tmpl: grow-only, kept across re-configuration
     int32_t *d_calib = nullptr;
+    size_t bkg_bytes = 0, calib_bytes = 0, tmpl_bytes[2][3] = {};
     int32_t *d_calib_flip = nullptr;  // calibration with the mirror folded in + the background seen through it (k_fold_calib):
     uint8_t *d_run_mode = nullptr;
     uint8_t *d_bkg_warp = nullptr;    // scratch of prepare(), rebuilt when the background / calibration change (fold_dirty)
@@ -70,12 +71,23 @@ struct lm_ctx {
     LmBatch bt_more[NSLOT - 1] = {};  // the same with scratch sets 1..: consecutive sub-batches overlap on their own streams
     int nsets = 0;                    // scratch sets allocated by prepare()
     int last_Bsub = 0;                // sub-batch size of the last lm_detect_batch call
-    std::vector<void *> dev_allocs;   // everything cudaMalloc'ed for the scratch
+    int hint_B = 0, hint_sets = 0;    // scratch capacity of the last prepare(): a re-configured context asks for at least as much
+    // Scratch blocks.  They outlive re-configuration: release_scratch() only marks them free and the next prepare() takes, for
+    // each request, the smallest free block that is large enough (a video of the same geometry reuses every block; cudaMalloc
+    // and cudaFree wait for the whole device, i.e. for every other context's work too).  Blocks that stay free after a prepare()
+    // that had to allocate are returned to the driver.
+    struct Block {
+        uint8_t *base;                // cudaMalloc result (the leading guard region in guard mode)
+        size_t bytes;                 // usable bytes
+        size_t req;                   // bytes of the buffer placed in it; in guard mode [req, bytes) holds the guard pattern too
+        bool used;
+    };
+    std::vector<Block> blocks;
+    int64_t device_allocs = 0;        // cudaMalloc calls so far (lm_get_info("device_allocs"))
     // Guard mode (environment variable LM_GUARD=1 when the context is created; compute-sanitizer is not available on the pool):
-    // every scratch allocation sits between two 4 kB regions filled with a pattern, lm_get_info("guard_violations") counts the
+    // every scratch block sits between two 4 kB regions filled with a pattern, lm_get_info("guard_violations") counts the
     // bytes of those regions that no longer hold it, i.e. out-of-bounds WRITES of any kernel since the allocation.
     bool guard = false;
-    std::vector<std::pair<uint8_t *, size_t>> guard_regions;
     uint8_t *d_stage[2] = {};         // staged raw frames (Bcap + 1 each) when frames come from the host
     uint32_t *d_bb[10] = {};           // [3][Bcap] per ring set
     // result staging
@@ -87,7 +99,8 @@ struct lm_ctx {
     // (index mod the number of slots in use): the host queues as many sub-batches ahead of the one it is copying out as
     // there are slots, so the device always has several sub-batches to overlap while the host copies results out.
     static constexpr int NRES = 10;    // > the deepest lookahead (= number of slots in use)
-    uint8_t *h_res[NRES] = {};        // pinned
+    uint8_t *h_res[NRES] = {};        // pinned, h_res_bytes each (grow-only)
+    size_t h_res_bytes = 0;
     cudaEvent_t ev_h2d[NRES] = {}, ev_done[NRES] = {};
     cudaEvent_t ev_stage[NRES][8] = {};
     cudaEvent_t ev_call[2] = {};      // first kernel / last D2H of a whole lm_detect_batch call
@@ -95,6 +108,7 @@ struct lm_ctx {
     cudaEvent_t ev_go[NRES] = {};     // before k_screen (hand-over to the high-priority stream)
     cudaEvent_t ev_sstart[NRES] = {}; // on the screen's stream right before k_screen2 (device timeline only)
     float ms_screen = 0.f;            // k_screen alone, summed over the sub-batches of the last call
+    long long screen_macs = 0;        // int8 MACs of the last k_screen2 launch
     float ms[7] = {};
     std::vector<float> timeline;     // [sub-batch][9]: ms from the start of the last call to its stage events 0..7 and to the end of the screen kernel
     int64_t launches = 0;
@@ -103,7 +117,7 @@ struct lm_ctx {
         int cap = 0;
         int32_t *minmax = nullptr;
         uint8_t *lut = nullptr, *pred = nullptr, *stage = nullptr, *diff = nullptr;
-        size_t diff_bytes = 0;
+        size_t stage_bytes = 0, diff_bytes = 0;
         int32_t *calib_flip = nullptr;   // k_fold_calib's arrays for pass 1 (folded at every call: the background may have changed)
         uint8_t *bkg_warp = nullptr, *run_mode = nullptr;
         size_t fold_px = 0;
@@ -195,7 +209,68 @@ bool roi_ok(const lm_ctx *c, uint32_t bbx, uint32_t bbys, uint32_t bbyb) {
     return true;
 }
 
-void free_scratch(lm_ctx *c) {
+// Waits for this context's own work only (cudaDeviceSynchronize would wait for every other context on the device too).
+cudaError_t sync_streams(lm_ctx *c) {
+    cudaError_t e = cudaSuccess, x;
+    auto one = [&](cudaStream_t s) {
+        if (s && (x = cudaStreamSynchronize(s)) != cudaSuccess && e == cudaSuccess) e = x;
+    };
+    one(c->copy_stream);
+    one(c->stream);
+    for (cudaStream_t s : c->stream_more) one(s);
+    one(c->stream_hi);
+    for (cudaStream_t s : c->stream_back) one(s);
+    return e;
+}
+
+cudaError_t count_alloc(lm_ctx *c, cudaError_t e) {
+    if (e == cudaSuccess) ++c->device_allocs;
+    return e;
+}
+
+// Grow-only device buffer of per-context state (contents are not kept when it grows).
+template <typename T>
+cudaError_t reserve(lm_ctx *c, T **p, size_t *cap, size_t bytes) {
+    if (*p && *cap >= bytes) return cudaSuccess;
+    cudaFree(*p);
+    *p = nullptr;
+    *cap = 0;
+    const cudaError_t e = cudaMalloc((void **)p, std::max<size_t>(bytes, 1));
+    if (e != cudaSuccess) return e;
+    ++c->device_allocs;
+    *cap = bytes;
+    return e;
+}
+
+// Marks every scratch block free (the streams have been drained) and forgets the derived layout; prepare() re-derives it.
+void release_scratch(lm_ctx *c) {
+    for (auto &b : c->blocks) b.used = false;
+    for (int s = 0; s < 2; ++s) c->d_stage[s] = nullptr;
+    c->d_calib_flip = nullptr;
+    c->d_bkg_warp = nullptr;
+    c->d_run_mode = nullptr;
+    c->fold_dirty = true;
+    for (int s = 0; s < lm_ctx::NRES; ++s) c->d_bb[s] = nullptr;
+    for (int s = 0; s < lm_ctx::NSLOT; ++s) c->d_res[s] = nullptr;
+    c->bt = LmBatch{};
+    for (auto &b : c->bt_more) b = LmBatch{};
+    c->nsets = 0;
+    c->Bcap = 0;
+}
+
+// Returns the free scratch blocks to the driver (all of them after release_scratch).
+void trim_scratch(lm_ctx *c) {
+    std::vector<lm_ctx::Block> keep;
+    for (auto &b : c->blocks)
+        if (b.used) keep.push_back(b);
+        else cudaFree(b.base);
+    c->blocks.swap(keep);
+}
+
+// Everything the context owns on the device and in page-locked memory (lm_destroy).
+void free_all(lm_ctx *c) {
+    release_scratch(c);
+    trim_scratch(c);
     cudaFree(c->bbs.minmax);
     cudaFree(c->bbs.lut);
     cudaFree(c->bbs.pred);
@@ -208,46 +283,49 @@ void free_scratch(lm_ctx *c) {
     cudaFree(c->bbs.bbx);
     cudaFree(c->bbs.lims);
     c->bbs = lm_ctx::BBScratch{};
-    for (void *p : c->dev_allocs) cudaFree(p);
-    c->dev_allocs.clear();
-    c->guard_regions.clear();
     for (int s = 0; s < lm_ctx::NRES; ++s) {
         if (c->h_res[s]) cudaFreeHost(c->h_res[s]);
         c->h_res[s] = nullptr;
     }
-    for (int s = 0; s < 2; ++s) c->d_stage[s] = nullptr;
-    c->d_calib_flip = nullptr;
-    c->d_bkg_warp = nullptr;
-    c->d_run_mode = nullptr;
-    c->fold_dirty = true;
-    for (int s = 0; s < lm_ctx::NRES; ++s) c->d_bb[s] = nullptr;
-    for (int s = 0; s < lm_ctx::NSLOT; ++s) c->d_res[s] = nullptr;
-    c->nsets = 0;
-    c->Bcap = 0;
+    c->h_res_bytes = 0;
 }
 
 constexpr size_t LM_GUARD_BYTES = 4096;
 constexpr int LM_GUARD_PATTERN = 0xA5;
 
+// One scratch buffer of `count` T, zero-filled: a free block that is large enough (the smallest such), else a new one.
 template <typename T>
 int dalloc(lm_ctx *ctx, T **p, size_t count) {
-    void *q = nullptr;
     const size_t bytes = std::max<size_t>(count * sizeof(T), 256);
-    if (ctx->guard) {
-        CK(cudaMalloc(&q, bytes + 2 * LM_GUARD_BYTES));
-        ctx->dev_allocs.push_back(q);
-        uint8_t *base = static_cast<uint8_t *>(q);
-        CK(cudaMemset(base, LM_GUARD_PATTERN, LM_GUARD_BYTES));
-        CK(cudaMemset(base + LM_GUARD_BYTES, 0, bytes));
-        CK(cudaMemset(base + LM_GUARD_BYTES + bytes, LM_GUARD_PATTERN, LM_GUARD_BYTES));
-        ctx->guard_regions.emplace_back(base, LM_GUARD_BYTES);
-        ctx->guard_regions.emplace_back(base + LM_GUARD_BYTES + bytes, LM_GUARD_BYTES);
-        *p = reinterpret_cast<T *>(base + LM_GUARD_BYTES);
-        return LM_OK;
+    const size_t g = ctx->guard ? LM_GUARD_BYTES : 0;
+    lm_ctx::Block *best = nullptr;
+    for (auto &b : ctx->blocks)
+        if (!b.used && b.bytes >= bytes && (!best || b.bytes < best->bytes)) best = &b;
+    if (!best) {
+        void *q = nullptr;
+        cudaError_t e = cudaMalloc(&q, bytes + 2 * g);
+        if (e == cudaErrorMemoryAllocation) {  // the free blocks (too small for this geometry) go back to the driver first
+            cudaGetLastError();
+            trim_scratch(ctx);
+            e = cudaMalloc(&q, bytes + 2 * g);
+        }
+        CK(count_alloc(ctx, e));
+        ctx->blocks.push_back(lm_ctx::Block{static_cast<uint8_t *>(q), bytes, bytes, false});
+        best = &ctx->blocks.back();
+        if (g) {
+            CK(cudaMemsetAsync(best->base, LM_GUARD_PATTERN, g, ctx->stream));
+            CK(cudaMemsetAsync(best->base + g + bytes, LM_GUARD_PATTERN, g, ctx->stream));
+        }
     }
-    CK(cudaMalloc(&q, bytes));
-    ctx->dev_allocs.push_back(q);
-    *p = reinterpret_cast<T *>(q);
+    best->used = true;
+    best->req = bytes;
+    // guard mode: the slack of a larger reused block is guarded like the region behind it (an overrun into it is counted)
+    if (g && best->bytes > bytes) CK(cudaMemsetAsync(best->base + g + bytes, LM_GUARD_PATTERN, best->bytes - bytes, ctx->stream));
+    // fresh or reused (a reused block holds the previous video's data), every buffer starts zero-filled: results never depend
+    // on whether a context was re-configured
+    CK(cudaMemsetAsync(best->base + g, 0, bytes, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    *p = reinterpret_cast<T *>(best->base + g);
     return LM_OK;
 }
 
@@ -389,7 +467,8 @@ int prepare_screen(lm_ctx *ctx, LmBatch &b, int want, size_t B) {
             if (have1) {
                 int8_t *dimg = nullptr;
                 if ((rc = dalloc(ctx, &dimg, img1[v][f].size()))) return rc;
-                CK(cudaMemcpy(dimg, img1[v][f].data(), img1[v][f].size(), cudaMemcpyHostToDevice));
+                CK(cudaMemcpyAsync(dimg, img1[v][f].data(), img1[v][f].size(), cudaMemcpyHostToDevice, ctx->stream));
+                CK(cudaStreamSynchronize(ctx->stream));
                 J.Bimg = dimg;
             }
         }
@@ -402,7 +481,8 @@ int prepare_screen(lm_ctx *ctx, LmBatch &b, int want, size_t B) {
                 for (int r = 0; r < 2; ++r) {
                     int8_t *dimg = nullptr;
                     if ((rc = dalloc(ctx, &dimg, img2[v][q][r].size()))) return rc;
-                    CK(cudaMemcpy(dimg, img2[v][q][r].data(), img2[v][q][r].size(), cudaMemcpyHostToDevice));
+                    CK(cudaMemcpyAsync(dimg, img2[v][q][r].data(), img2[v][q][r].size(), cudaMemcpyHostToDevice, ctx->stream));
+                    CK(cudaStreamSynchronize(ctx->stream));
                     J2.Bimg[r] = dimg;
                 }
                 J2.view = v;
@@ -444,7 +524,8 @@ int prepare_screen(lm_ctx *ctx, LmBatch &b, int want, size_t B) {
 // derive window geometry + allocate scratch for sub-batches of Bcap frames
 // Scratch for sub-batches of up to `want_B` frames in `want_sets` rotating sets (0: the configured sub-batch size / stream
 // count).  Grows on demand and never shrinks: a short first video does not pay for (or wait for the allocation of) the
-// ~2.5 GB per set that a long one uses.
+// ~2.5 GB per set that a long one uses, and a re-configured context keeps the capacity of its last videos.
+int prepare_impl(lm_ctx *ctx, int want_B, int want_sets);
 int prepare(lm_ctx *ctx, int want_B = 0, int want_sets = 0) {
     int cap_B = ctx->opt_subbatch;
     if (const char *e = getenv("LM_SUBBATCH")) cap_B = std::max(1, atoi(e));
@@ -452,11 +533,20 @@ int prepare(lm_ctx *ctx, int want_B = 0, int want_sets = 0) {
     want_B = want_B <= 0 ? cap_B : std::min(want_B, cap_B);
     want_sets = want_sets <= 0 ? cap_sets : std::max(2, std::min(want_sets, cap_sets));
     if (ctx->Bcap >= want_B && ctx->nsets >= want_sets) return LM_OK;
-    if (ctx->Bcap) {   // too small for this call: every stream was drained when the previous call returned
-        want_B = std::max(want_B, ctx->Bcap);
-        want_sets = std::max(want_sets, ctx->nsets);
-        free_scratch(ctx);
-    }
+    // too small for this call (every stream was drained when the previous call returned), or re-derived after re-configuration
+    want_B = std::min(cap_B, std::max({want_B, ctx->Bcap, ctx->hint_B}));
+    want_sets = std::min(cap_sets, std::max({want_sets, ctx->nsets, ctx->hint_sets}));
+    release_scratch(ctx);
+    const int64_t allocs = ctx->device_allocs;
+    const int rc = prepare_impl(ctx, want_B, want_sets);
+    if (rc != LM_OK) return rc;
+    ctx->hint_B = ctx->Bcap;
+    ctx->hint_sets = ctx->nsets;
+    if (ctx->device_allocs != allocs) trim_scratch(ctx);  // the geometry grew: blocks too small for it go back to the driver
+    return LM_OK;
+}
+
+int prepare_impl(lm_ctx *ctx, int want_B, int want_sets) {
     const lm_config &k = ctx->cfg;
     LmBatch &b = ctx->bt;
     b = LmBatch{};
@@ -558,7 +648,15 @@ int prepare(lm_ctx *ctx, int want_B = 0, int want_sets = 0) {
     o.tail = off;     off = align256(off + B * 3 * k.n_tail_points * 4);
     o.flags = off;    off = align256(off + B * 4);
     o.total = off;
-    for (int s = 0; s < lm_ctx::NRES; ++s) CK(cudaMallocHost((void **)&ctx->h_res[s], o.total));
+    if (ctx->h_res_bytes < o.total) {
+        for (int s = 0; s < lm_ctx::NRES; ++s) {
+            if (ctx->h_res[s]) cudaFreeHost(ctx->h_res[s]);
+            ctx->h_res[s] = nullptr;
+        }
+        ctx->h_res_bytes = 0;
+        for (int s = 0; s < lm_ctx::NRES; ++s) CK(cudaMallocHost((void **)&ctx->h_res[s], o.total));
+        ctx->h_res_bytes = o.total;
+    }
     auto bind_results = [&](LmBatch &x, int set) -> int {
         int rc2;
         if ((rc2 = dalloc(ctx, &ctx->d_res[set], o.total))) return rc2;
@@ -696,8 +794,8 @@ int lm_create(lm_ctx **out, int device) {
 int lm_destroy(lm_ctx *ctx) {
     if (!ctx) return LM_OK;
     DeviceGuard guard(ctx->device);
-    cudaDeviceSynchronize();
-    free_scratch(ctx);
+    sync_streams(ctx);
+    free_all(ctx);
     cudaFree(ctx->d_bkg);
     cudaFree(ctx->d_calib);
     for (int v = 0; v < 2; ++v)
@@ -740,12 +838,8 @@ int lm_configure(lm_ctx *ctx, const lm_config *cfg) {
     if ((int64_t)k.bb_w * std::max(k.bb_h_bottom, k.bb_h_side) >= (1 << 21))
         return fail(ctx, LM_ERR_INVALID, "box too large for the connected-component key packing");
     DeviceGuard guard(ctx->device);
-    cudaDeviceSynchronize();
-    free_scratch(ctx);
-    cudaFree(ctx->d_bkg);
-    cudaFree(ctx->d_calib);
-    ctx->d_bkg = nullptr;
-    ctx->d_calib = nullptr;
+    CK(sync_streams(ctx));
+    release_scratch(ctx);  // the allocations stay for the next video; the layout follows the new geometry
     ctx->bkg_set = ctx->calib_set = false;
     ctx->cfg = k;
     ctx->configured = true;
@@ -758,18 +852,18 @@ int lm_set_model(lm_ctx *ctx, const lm_template t[2][3]) {
     if (!ctx->configured) return fail(ctx, LM_ERR_STATE, "lm_set_model before lm_configure");
     if (!t) return fail(ctx, LM_ERR_INVALID, "null model");
     DeviceGuard guard(ctx->device);
-    cudaDeviceSynchronize();
-    free_scratch(ctx);
+    CK(sync_streams(ctx));
+    release_scratch(ctx);
     ctx->model_set = false;  // a failure below must not leave a half-updated model in use
     for (int v = 0; v < 2; ++v)
         for (int f = 0; f < 3; ++f) {
             const lm_template &T = t[v][f];
             if (!T.w || T.rows <= 0 || T.cols <= 0) return fail(ctx, LM_ERR_INVALID, "template [%d][%d] is empty", v, f);
             if (T.cols > LM_MAX_KW) return fail(ctx, LM_ERR_INVALID, "template [%d][%d] has %d columns (max %d)", v, f, T.cols, LM_MAX_KW);
-            cudaFree(ctx->d_tmpl[v][f]);
-            ctx->d_tmpl[v][f] = nullptr;
-            CK(cudaMalloc((void **)&ctx->d_tmpl[v][f], (size_t)T.rows * T.cols * sizeof(float)));
-            CK(cudaMemcpy(ctx->d_tmpl[v][f], T.w, (size_t)T.rows * T.cols * sizeof(float), cudaMemcpyHostToDevice));
+            const size_t bytes = (size_t)T.rows * T.cols * sizeof(float);
+            CK(reserve(ctx, &ctx->d_tmpl[v][f], &ctx->tmpl_bytes[v][f], bytes));
+            CK(cudaMemcpyAsync(ctx->d_tmpl[v][f], T.w, bytes, cudaMemcpyHostToDevice, ctx->stream));
+            CK(cudaStreamSynchronize(ctx->stream));
             ctx->h_tmpl[v][f].assign(T.w, T.w + (size_t)T.rows * T.cols);
             ctx->t_rows[v][f] = T.rows;
             ctx->t_cols[v][f] = T.cols;
@@ -786,9 +880,10 @@ int lm_set_background(lm_ctx *ctx, const uint8_t *bkg) {
     if (!bkg) return fail(ctx, LM_ERR_INVALID, "null background");
     DeviceGuard guard(ctx->device);
     const size_t n = (size_t)ctx->cfg.vid_rows * ctx->cfg.vid_cols;
-    if (!ctx->d_bkg) CK(cudaMalloc((void **)&ctx->d_bkg, n));
-    cudaDeviceSynchronize();
-    CK(cudaMemcpy(ctx->d_bkg, bkg, n, cudaMemcpyHostToDevice));
+    CK(sync_streams(ctx));
+    CK(reserve(ctx, &ctx->d_bkg, &ctx->bkg_bytes, n));
+    CK(cudaMemcpyAsync(ctx->d_bkg, bkg, n, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
     ctx->bt.bkg = ctx->d_bkg;
     ctx->bkg_set = true;
     ctx->fold_dirty = true;
@@ -807,9 +902,10 @@ int lm_set_calibration(lm_ctx *ctx, const int32_t *map) {
             return fail(ctx, LM_ERR_RUNTIME, "Calibration mapping indices out of range (index %zu = %d, frame has %lld pixels)",
                         i, map[i], (long long)lim);
     DeviceGuard guard(ctx->device);
-    if (!ctx->d_calib) CK(cudaMalloc((void **)&ctx->d_calib, n * sizeof(int32_t)));
-    cudaDeviceSynchronize();
-    CK(cudaMemcpy(ctx->d_calib, map, n * sizeof(int32_t), cudaMemcpyHostToDevice));
+    CK(sync_streams(ctx));
+    CK(reserve(ctx, &ctx->d_calib, &ctx->calib_bytes, n * sizeof(int32_t)));
+    CK(cudaMemcpyAsync(ctx->d_calib, map, n * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
     ctx->bt.calib = ctx->d_calib;
     ctx->calib_set = true;
     ctx->fold_dirty = true;
@@ -892,7 +988,8 @@ static int detect_batch_impl(lm_ctx *ctx, const uint8_t *frames, int frames_on_d
     int rc = prepare(ctx, Bsub, (int)std::min<int64_t>(lm_ctx::NSLOT, (n + Bsub - 1) / Bsub));
     if (rc == LM_OK && !frames_on_device) rc = ensure_stage(ctx);
     if (rc) {  // a half-built scratch set (device or pinned memory ran out) is released, not leaked
-        free_scratch(ctx);
+        release_scratch(ctx);
+        trim_scratch(ctx);
         return rc;
     }
     if (ctx->fold_dirty) {  // per-video constants of k_prep / k_pair; every stream of the previous call has been drained
@@ -1008,6 +1105,7 @@ static int detect_batch_impl(lm_ctx *ctx, const uint8_t *frames, int frames_on_d
         b.screen_stream = (ctx->opt_streams > 1 && ctx->opt_screen_priority) ? ctx->stream_hi : nullptr;
         b.ev_screen_go = ctx->ev_go[ring];
         b.ev_screen_start = ctx->ev_sstart[ring];
+        b.screen_macs = &ctx->screen_macs;
         cudaEvent_t *ev = ctx->ev_stage[ring];
         CK(cudaStreamWaitEvent(stf, ctx->ev_h2d[ring], 0));
         // with the back phase on its own stream the slot's scratch is no longer protected by stream order alone
@@ -1108,8 +1206,8 @@ int lm_set_option(lm_ctx *ctx, const char *name, int64_t value) {
     } else {
         return fail(ctx, LM_ERR_INVALID, "unknown option '%s'", name);
     }
-    cudaDeviceSynchronize();
-    free_scratch(ctx);  // re-derived by the next lm_detect_batch
+    CK(sync_streams(ctx));
+    release_scratch(ctx);  // re-derived by the next lm_detect_batch
     return LM_OK;
 }
 
@@ -1162,7 +1260,7 @@ int lm_get_info(const lm_ctx *ctx, const char *name, double *value) {
         return LM_OK;
     }
     if (!strcmp(name, "screen_macs")) {  // int8 MACs the last k_screen2 launch (one sub-batch) issued to the tensor cores
-        *value = (double)lm_screen2_last_macs();
+        *value = (double)ctx->screen_macs;
         return LM_OK;
     }
     if (!strcmp(name, "subbatch")) {   // frames per sub-batch of the last lm_detect_batch call (before the first: the configured size)
@@ -1173,32 +1271,44 @@ int lm_get_info(const lm_ctx *ctx, const char *name, double *value) {
         *value = (double)ctx->Bcap;
         return LM_OK;
     }
+    if (!strcmp(name, "device_allocs")) {   // cudaMalloc calls of this context so far (each waits for the whole device)
+        *value = (double)ctx->device_allocs;
+        return LM_OK;
+    }
     if (!strcmp(name, "guard_regions")) {
-        size_t k = ctx->guard_regions.size();
+        size_t k = ctx->guard ? 2 * ctx->blocks.size() : 0;
         for (const auto &b : ctx->png) k += b.base && ctx->guard ? 2 : 0;
         *value = (double)k;
         return LM_OK;
     }
     const bool selftest = !strcmp(name, "guard_selftest");   // positive control: three guard bytes are overwritten, counted, restored
     if (!strcmp(name, "guard_violations") || selftest) {   // bytes of the guard regions overwritten so far (-1: guard mode is off)
-        if (!ctx->guard || (selftest && ctx->guard_regions.empty())) {
+        if (!ctx->guard || (selftest && ctx->blocks.empty())) {
             *value = -1.0;
             return LM_OK;
         }
         DeviceGuard dg(ctx->device);
+        lm_ctx *c = const_cast<lm_ctx *>(ctx);  // only its streams are used
+        cudaStream_t st = c->stream;
         unsigned long long *bad = nullptr, h = 0;
-        if (cudaDeviceSynchronize() != cudaSuccess || cudaMalloc(&bad, sizeof *bad) != cudaSuccess) return LM_ERR_RUNTIME;
-        cudaMemset(bad, 0, sizeof *bad);
-        if (selftest) cudaMemset(ctx->guard_regions.back().first + 7, 0, 3);
-        for (const auto &r : ctx->guard_regions) k_guard_check<<<4, 256>>>(r.first, r.second, bad);
+        if (sync_streams(c) != cudaSuccess || cudaMallocAsync((void **)&bad, sizeof *bad, st) != cudaSuccess) return LM_ERR_RUNTIME;
+        uint8_t *probe = selftest ? ctx->blocks.back().base + LM_GUARD_BYTES + ctx->blocks.back().req + 7 : nullptr;  // trailing guard
+        cudaMemsetAsync(bad, 0, sizeof *bad, st);
+        if (selftest) cudaMemsetAsync(probe, 0, 3, st);
+        for (const auto &b : ctx->blocks)  // retained blocks (free until the next prepare) keep their guards too
+        {
+            k_guard_check<<<4, 256, 0, st>>>(b.base, LM_GUARD_BYTES, bad);
+            k_guard_check<<<4, 256, 0, st>>>(b.base + LM_GUARD_BYTES + b.req, b.bytes - b.req + LM_GUARD_BYTES, bad);
+        }
         for (const auto &b : ctx->png)
             if (b.base) {
-                k_guard_check<<<4, 256>>>(b.base, LM_GUARD_BYTES, bad);
-                k_guard_check<<<4, 256>>>(b.p + b.bytes, LM_GUARD_BYTES, bad);
+                k_guard_check<<<4, 256, 0, st>>>(b.base, LM_GUARD_BYTES, bad);
+                k_guard_check<<<4, 256, 0, st>>>(b.p + b.bytes, LM_GUARD_BYTES, bad);
             }
-        const cudaError_t e = cudaMemcpy(&h, bad, sizeof h, cudaMemcpyDeviceToHost);
-        if (selftest) cudaMemset(ctx->guard_regions.back().first + 7, LM_GUARD_PATTERN, 3);
-        cudaFree(bad);
+        cudaError_t e = cudaMemcpyAsync(&h, bad, sizeof h, cudaMemcpyDeviceToHost, st);
+        if (selftest) cudaMemsetAsync(probe, LM_GUARD_PATTERN, 3, st);
+        cudaFreeAsync(bad, st);
+        if (cudaStreamSynchronize(st) != cudaSuccess) e = cudaErrorUnknown;
         if (e != cudaSuccess) return LM_ERR_RUNTIME;
         *value = (double)h;
         return LM_OK;
@@ -1208,14 +1318,19 @@ int lm_get_info(const lm_ctx *ctx, const char *name, double *value) {
     if (!strcmp(name, "sparse_tasks") || !strcmp(name, "positives")) {
         if (!ctx->Bcap) return LM_ERR_INVALID;
         const LmBatch &b = ctx->bt;
+        DeviceGuard dg(ctx->device);
+        cudaStream_t st = ctx->stream;
+        auto fetch = [st](void *dst, const void *src, size_t n) {
+            return cudaMemcpyAsync(dst, src, n, cudaMemcpyDeviceToHost, st) == cudaSuccess && cudaStreamSynchronize(st) == cudaSuccess;
+        };
         double tot = 0.0;
         if (name[0] == 's') {
             int32_t nt[8] = {};
-            if (!b.scr.ntasks || cudaMemcpy(nt, b.scr.ntasks, sizeof nt, cudaMemcpyDeviceToHost) != cudaSuccess) return LM_ERR_RUNTIME;
+            if (!b.scr.ntasks || !fetch(nt, b.scr.ntasks, sizeof nt)) return LM_ERR_RUNTIME;
             for (int i = 0; i < 6; ++i) tot += nt[i];
         } else {
             std::vector<int32_t> c((size_t)ctx->Bcap * 4);
-            if (cudaMemcpy(c.data(), b.det_count, c.size() * sizeof(int32_t), cudaMemcpyDeviceToHost) != cudaSuccess) return LM_ERR_RUNTIME;
+            if (!fetch(c.data(), b.det_count, c.size() * sizeof(int32_t))) return LM_ERR_RUNTIME;
             for (int32_t x : c) tot += x;
         }
         *value = tot;
@@ -1258,26 +1373,19 @@ int lm_bounding_box_tm_de(lm_ctx *ctx, const uint8_t *frames, int frames_on_devi
     const int64_t fsz = (int64_t)k.vid_rows * k.vid_cols;
     lm_ctx::BBScratch &S = ctx->bbs;
     const int cap = 1024;  // frames per chunk: large enough that launch gaps do not matter, small scratch (1.3 MB)
+    // (kept across re-configuration; the buffers that depend on the geometry grow when it does)
     if (!S.cap) {
-        CK(cudaMalloc((void **)&S.minmax, (size_t)(cap + 1) * 2 * sizeof(int32_t)));
-        CK(cudaMalloc((void **)&S.lut, (size_t)(cap + 1) * 256));
-        CK(cudaMalloc((void **)&S.pred, (size_t)cap * 256));
-        CK(cudaMalloc((void **)&S.hist, (size_t)cap * 256 * sizeof(uint32_t)));
-        CK(cudaMalloc((void **)&S.bbx, (size_t)cap * sizeof(double)));
-        CK(cudaMalloc((void **)&S.lims, (size_t)cap * 2 * sizeof(int32_t)));
+        CK(count_alloc(ctx, cudaMalloc((void **)&S.minmax, (size_t)(cap + 1) * 2 * sizeof(int32_t))));
+        CK(count_alloc(ctx, cudaMalloc((void **)&S.lut, (size_t)(cap + 1) * 256)));
+        CK(count_alloc(ctx, cudaMalloc((void **)&S.pred, (size_t)cap * 256)));
+        CK(count_alloc(ctx, cudaMalloc((void **)&S.hist, (size_t)cap * 256 * sizeof(uint32_t))));
+        CK(count_alloc(ctx, cudaMalloc((void **)&S.bbx, (size_t)cap * sizeof(double))));
+        CK(count_alloc(ctx, cudaMalloc((void **)&S.lims, (size_t)cap * 2 * sizeof(int32_t))));
         S.cap = cap;
     }
-    if (!frames_on_device && !S.stage) CK(cudaMalloc((void **)&S.stage, (size_t)cap * fsz));
-    {   // the side view's raw differences of one chunk (one gather instead of two; see k_bb_hist)
-        const size_t need = (size_t)cap * p->side_w * p->side_h;
-        if (S.diff_bytes < need) {
-            cudaFree(S.diff);
-            S.diff = nullptr;
-            S.diff_bytes = 0;
-            CK(cudaMalloc((void **)&S.diff, need));
-            S.diff_bytes = need;
-        }
-    }
+    if (!frames_on_device) CK(reserve(ctx, &S.stage, &S.stage_bytes, (size_t)cap * fsz));
+    // the side view's raw differences of one chunk (one gather instead of two; see k_bb_hist)
+    CK(reserve(ctx, &S.diff, &S.diff_bytes, (size_t)cap * p->side_w * p->side_h));
     cudaStream_t st = ctx->stream;
     {   // calibration map with the mirror folded in, background seen through it, run flags (k_prep's vector tier, used by k_bb_hist16)
         const size_t px = (size_t)k.n_rows * k.n_cols;
@@ -1288,9 +1396,9 @@ int lm_bounding_box_tm_de(lm_ctx *ctx, const uint8_t *frames, int frames_on_devi
             S.calib_flip = nullptr;
             S.bkg_warp = S.run_mode = nullptr;
             S.fold_px = 0;
-            CK(cudaMalloc((void **)&S.calib_flip, px * sizeof(int32_t)));
-            CK(cudaMalloc((void **)&S.bkg_warp, px + 32));
-            CK(cudaMalloc((void **)&S.run_mode, px));
+            CK(count_alloc(ctx, cudaMalloc((void **)&S.calib_flip, px * sizeof(int32_t))));
+            CK(count_alloc(ctx, cudaMalloc((void **)&S.bkg_warp, px + 32)));
+            CK(count_alloc(ctx, cudaMalloc((void **)&S.run_mode, px)));
             CK(cudaMemsetAsync(S.bkg_warp, 0, px + 32, st));
             S.fold_px = px;
         }
@@ -1298,13 +1406,11 @@ int lm_bounding_box_tm_de(lm_ctx *ctx, const uint8_t *frames, int frames_on_devi
             return fail(ctx, LM_ERR_RUNTIME, "calibration fold launch failed");
     }
     // results for the whole call stay on the device until the end: chunks run back to back without a host sync
-    double *d_bbx = nullptr;
-    int32_t *d_lims = nullptr;
-    CK(cudaMalloc((void **)&d_bbx, (size_t)n * sizeof(double)));
-    if (cudaMalloc((void **)&d_lims, (size_t)n * 2 * sizeof(int32_t)) != cudaSuccess) {
-        cudaFree(d_bbx);
-        return fail(ctx, LM_ERR_RUNTIME, "out of device memory");
-    }
+    DevBuf bbx_buf(st), lims_buf(st);
+    CK(bbx_buf.alloc((size_t)n * sizeof(double)));
+    CK(lims_buf.alloc((size_t)n * 2 * sizeof(int32_t)));
+    double *d_bbx = (double *)bbx_buf.p;
+    int32_t *d_lims = (int32_t *)lims_buf.p;
     int rc = LM_OK;
     for (int64_t s0 = 0; s0 < n && rc == LM_OK; s0 += cap) {
         const int B = (int)std::min<int64_t>(cap, n - s0);
@@ -1342,8 +1448,6 @@ int lm_bounding_box_tm_de(lm_ctx *ctx, const uint8_t *frames, int frames_on_devi
         rc = fail(ctx, LM_ERR_RUNTIME, "D2H copy failed");
     if (cudaStreamSynchronize(st) != cudaSuccess && rc == LM_OK)
         rc = fail(ctx, LM_ERR_RUNTIME, "pass 1 failed on the device: %s", cudaGetErrorString(cudaGetLastError()));
-    cudaFree(d_bbx);
-    cudaFree(d_lims);
     return rc;
 }
 
@@ -1631,7 +1735,8 @@ int lm_debug_nms(lm_ctx *ctx, int view, int feat, const float *scores, lm_cand *
     DeviceGuard guard(ctx->device);
     int rc = prepare(ctx, 64, 2);   // one frame's lists: the smallest scratch set will do (grows later if a detection call needs more)
     if (rc) {
-        free_scratch(ctx);
+        release_scratch(ctx);
+        trim_scratch(ctx);
         return rc;
     }
     LmBatch b = ctx->bt;
@@ -1689,7 +1794,7 @@ int lm_device_alloc(lm_ctx *ctx, void **ptr, size_t bytes) {
     if (!ctx || !ptr) return LM_ERR_INVALID;
     *ptr = nullptr;
     DeviceGuard guard(ctx->device);
-    const cudaError_t e = cudaMalloc(ptr, std::max<size_t>(bytes, 1));
+    const cudaError_t e = count_alloc(ctx, cudaMalloc(ptr, std::max<size_t>(bytes, 1)));
     if (e != cudaSuccess) {
         cudaGetLastError();
         *ptr = nullptr;
@@ -1717,7 +1822,7 @@ int png_reserve(lm_ctx *ctx, lm_ctx::PngBuf &b, size_t bytes) {
     b = lm_ctx::PngBuf{};
     const size_t g = ctx->guard ? LM_GUARD_BYTES : 0;
     void *q = nullptr;
-    const cudaError_t e = cudaMalloc(&q, bytes + 2 * g);
+    const cudaError_t e = count_alloc(ctx, cudaMalloc(&q, bytes + 2 * g));
     if (e != cudaSuccess) {
         cudaGetLastError();
         return fail(ctx, LM_ERR_RUNTIME, "cannot allocate %zu bytes of device memory for the PNG decode: %s", bytes, cudaGetErrorString(e));
@@ -1726,8 +1831,8 @@ int png_reserve(lm_ctx *ctx, lm_ctx::PngBuf &b, size_t bytes) {
     b.p = b.base + g;
     b.bytes = bytes;
     if (g) {
-        CK(cudaMemset(b.base, LM_GUARD_PATTERN, g));
-        CK(cudaMemset(b.p + bytes, LM_GUARD_PATTERN, g));
+        CK(cudaMemsetAsync(b.base, LM_GUARD_PATTERN, g, ctx->stream));
+        CK(cudaMemsetAsync(b.p + bytes, LM_GUARD_PATTERN, g, ctx->stream));
     } else {
         b.base = b.p;
     }
@@ -2087,7 +2192,8 @@ int64_t lm_debug_fetch(lm_ctx *ctx, int what, int64_t frame, void *dst, int64_t 
     }
     if (dims) memcpy(dims, d, sizeof d);
     if (!dst || dst_bytes < bytes) return fail(ctx, LM_ERR_INVALID, "debug buffer too small (%lld needed)", (long long)bytes);
-    cudaError_t e = cudaMemcpy(dst, src, (size_t)bytes, cudaMemcpyDeviceToHost);
+    cudaError_t e = cudaMemcpyAsync(dst, src, (size_t)bytes, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) return fail(ctx, LM_ERR_RUNTIME, "cudaMemcpy: %s", cudaGetErrorString(e));
     return bytes;
 }

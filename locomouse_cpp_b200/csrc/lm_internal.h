@@ -15,6 +15,7 @@
 #include <stdint.h>
 
 #include <atomic>
+#include <mutex>
 #include <vector>
 
 #include "../../include/locomouse_b200.h"
@@ -125,6 +126,7 @@ struct LmBatch {
     cudaStream_t screen_stream; // when set (with ev_screen_go and ev_screen_done): the screen kernel runs on this (high-priority) stream
     cudaEvent_t ev_screen_start;  // recorded on the screen's stream right before the kernel (device timeline)
     cudaEvent_t ev_screen_go;
+    long long *screen_macs;     // host, may be null: receives the int8 MACs of the k_screen2 launch (the context's lm_get_info("screen_macs"))
     LmDet *det;                 // [B][2][2][det_cap]   index: ((f*2+feat)*2+view)
     int32_t *det_count;         // [B][2][2]
     // results (device mirrors of lm_results)
@@ -201,7 +203,6 @@ inline int lm_whatif_skip() {
     const char *e = getenv("LM_WHATIF_SKIP");
     return e ? atoi(e) : 0;
 }
-long long lm_screen2_last_macs();  // int8 MACs issued by the last k_screen2 launch (whole sub-batch)
 
 // PNG frame decode (k_png.cu).  Per-frame status codes of k_png_decode:
 enum {
@@ -242,16 +243,48 @@ int lm_corr_kwp(int kw);
 // dynamic shared memory the correlation kernel needs for a view/template (for capability checks)
 size_t lm_corr_smem_bytes(const LmBatch &b, int view, int feat);
 
-// Per-device one-time state of the launchers (function attributes are per device; a process may own several contexts).
+// Per-device one-time set-up of the launchers (function attributes are per device; a process may own several contexts, driven
+// from several host threads).  `if (auto setup = once.first()) { ... }`: exactly one caller per current device gets an open gate
+// and runs the block; a concurrent caller on the same device waits until that block has finished (it must not launch a kernel
+// whose shared-memory attribute is not set yet), later callers pass at the cost of one atomic load.
 struct LmDevOnce {
     std::atomic<bool> done[64] = {};
-    bool first(void) {  // true exactly once per current device, also when several host threads launch at once
+    std::mutex m;
+    struct Gate {
+        std::unique_lock<std::mutex> lock;
+        std::atomic<bool> *flag = nullptr;
+        Gate() = default;
+        Gate(Gate &&o) noexcept : lock(std::move(o.lock)), flag(o.flag) { o.flag = nullptr; }
+        explicit operator bool() const { return flag != nullptr; }
+        ~Gate() {
+            if (flag) flag->store(true, std::memory_order_release);
+        }
+    };
+    Gate first(void) {
         int dev = 0;
         cudaGetDevice(&dev);
         dev &= 63;
-        return !done[dev].exchange(true);
+        Gate g;
+        if (done[dev].load(std::memory_order_acquire)) return g;
+        g.lock = std::unique_lock<std::mutex>(m);
+        if (!done[dev].load(std::memory_order_acquire)) g.flag = &done[dev];
+        else g.lock.unlock();
+        return g;
     }
 };
+// Raises a kernel's dynamic shared-memory limit to all the device allows one block.  The attribute belongs to the function on the
+// device, shared by every context and host thread there: it is set once (under an LmDevOnce), never per call to a call-dependent
+// value that another thread's launch could overwrite between its own set and launch.
+template <class F>
+inline cudaError_t lm_allow_max_dynamic_smem(F *kernel) {
+    int dev = 0, optin = 0;
+    cudaGetDevice(&dev);
+    cudaError_t e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    cudaFuncAttributes a{};
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, kernel);
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)a.sharedSizeBytes);
+}
 // The SM's L1 / shared-memory split is a per-SM setting.  Hypothesis tested in round 2: a kernel that prefers another split than
 // k_screen2's (the largest shared-memory carve-out) cannot join an SM the screen runs on.  Measured: it can (tools/
 // coresidency_probe.cu; what decides is registers per SM sub-partition and the shared memory left), and asking every kernel of the

@@ -71,6 +71,29 @@ public:
     const T *end() const { return p_ + n_; }
 };
 
+// One video's frames (or coded frame chunks) and its background, as read from the files.  The page-locked buffer only grows,
+// so a LocoMouse_Media reused across videos is a pool: locomouse_b200_batch reads each worker's next video into one of two.
+struct LocoMouse_Media {
+    unsigned int n_frames = 0;
+    int rows = 0, cols = 0;
+    lmmedia::Codec codec = lmmedia::Codec::raw;
+    PinnedArray<uint8_t> data;          // raw: channel 0 of every frame, [n_frames][rows][cols]; coded: the frame chunks
+    std::vector<int64_t> offsets;       // coded: frame i = data[offsets[i], offsets[i + 1])
+    std::vector<uint8_t> extradata;     // FFV1: the configuration record
+    std::vector<uint8_t> bkg;           // rows x cols
+    // loadVideo + loadBackground (LocoMouse_class.cpp:367-417): throws std::runtime_error as the reference's constructor does
+    void load(const std::string &video_file, const std::string &bkg_file);
+};
+
+// Device memory that a compressed video is decoded into (grow-only, lm_device_alloc on the context that uses it).  Whoever
+// owns it reuses it across videos: locomouse_b200_batch keeps one per worker.
+struct LocoMouse_DeviceFrames {
+    uint8_t *p = nullptr;
+    size_t bytes = 0;
+    bool reserve(lm_ctx *ctx, size_t need);  // false (lm_last_error(ctx) says why) when the device memory is not there
+    void release(lm_ctx *ctx);
+};
+
 class LocoMouse_Parameters {
 public:
     // host-tracker cost builders (class.hpp:59-68, 88; class.cpp:132-145): used by computeUnaryCostsBottom / computePairwiseCostsBottom
@@ -83,7 +106,9 @@ public:
     int max_displacement_side = 15;
     int occlusion_grid_spacing_pixels_side = 20;
     double alpha_vel_side = 100;
-    int tracker_threads = 0;          // host threads for the independent match2nd problems (0: one per hardware thread)
+    int tracker_threads = 0;          // host threads for the independent match2nd problems (0: one per hardware thread;
+                                      // locomouse_b200_batch: hardware threads / workers)
+    int batch_workers_per_gpu = 2;    // locomouse_b200_batch: host threads (one lm_ctx each) per visible device
     std::vector<LocoMouse_LocationPrior> PRIOR_PAW, PRIOR_SNOUT;  // config key location_prior (5 x 7); empty: cost builders are skipped
     int conn_comp_connectivity = 8;
     int median_filter_size = 11;      // class.hpp:54-55: pass 1 of the base class
@@ -151,17 +176,14 @@ protected:
     std::string LM_CALL, CONFIG_FILE, VIDEO_FILE, BKG_FILE, MODEL_FILE, CALIBRATION_FILE, FLIP_CHAR, OUTPUT_PATH;
     std::string output_file;
 
-    PinnedArray<uint8_t> VIDEO;       // raw 8-bit frames (channel 0), N_FRAMES x vid_rows x vid_cols, page-locked
-    // PNG- or FFV1-coded AVI: the frame chunks (page-locked, frame i = [CODED_OFFSETS[i], CODED_OFFSETS[i + 1])) and, for
-    // FFV1, the configuration record; decoded once by configureDevice into D_VIDEO (device memory, same layout as VIDEO);
-    // VIDEO stays empty
-    lmmedia::Codec CODEC = lmmedia::Codec::raw;
-    std::shared_ptr<uint8_t> CODED_PAYLOAD;
-    std::vector<int64_t> CODED_OFFSETS;
-    std::vector<uint8_t> CODED_EXTRADATA;
-    uint8_t *D_VIDEO = nullptr;
+    // The video and background (raw frames, or PNG- / FFV1-coded frame chunks decoded once by configureDevice into DECODED,
+    // device memory in the layout of raw frames), read by the constructor into OWN_MEDIA or handed in by the caller
+    std::unique_ptr<LocoMouse_Media> OWN_MEDIA;
+    const LocoMouse_Media *MEDIA = nullptr;
+    std::unique_ptr<LocoMouse_DeviceFrames> OWN_DECODED;
+    LocoMouse_DeviceFrames *DECODED = nullptr;
+    bool DECODED_READY = false;
     int VID_ROWS = 0, VID_COLS = 0;
-    std::vector<uint8_t> BKG;
     std::vector<int32_t> CALIBRATION;  // ind_warp_mapping, N_ROWS x N_COLS
     bool IMAGE_FLIP = false;
 
@@ -192,20 +214,20 @@ protected:
 
     // ---- device side ------------------------------------------------------------------------------
     lm_ctx *CTX = nullptr;
+    bool OWN_CTX = true;               // false: the caller's context, left alone by the destructor
     struct Batch;                      // result buffers of the chunk that contains CURRENT_FRAME
     std::unique_ptr<Batch> BATCH, SPARE;   // SPARE: the chunk before BATCH, whose page-locked arrays the next chunk reuses
     bool LOOP_READY = false;
 
     void initializePaths(const LocoMouse_ParseInputs &INPUT);
-    void loadVideo();
-    void loadBackground();
+    void initializeInputs(const LocoMouse_Media &media, LocoMouse_DeviceFrames *decoded);  // calibration, model, side, sizes
     void loadCalibration();
     void loadFlip();
     void validateImageVideoSize();
     void check(int rc) const;          // lm_status -> exception
     void runChunk(unsigned int first_frame);
     void configureDevice();            // lm_configure + background + calibration for the current box sizes
-    const uint8_t *frames(int &on_device) const;  // first frame of the video: VIDEO, or D_VIDEO for compressed video
+    const uint8_t *frames(int &on_device) const;  // first frame of the video: MEDIA's raw frames, or DECODED for compressed video
     const Batch &batchFor(int frame) const;
     virtual bool usesImadjust() const { return false; }  // LocoMouse_TM::readFrame applies imadjust(0, 0.6)
     // class.cpp:2221-2346, 2385-2482
@@ -218,6 +240,12 @@ protected:
 
 public:
     explicit LocoMouse(LocoMouse_ParseInputs INPUTS);
+    // For a driver of many videos (locomouse_b200_batch): the configuration already parsed (params), the video and background
+    // already read (media, which must outlive the object), a context the object does not own (ctx, not destroyed with it) and
+    // the device memory a compressed video is decoded into (decoded, kept by the caller for the next video).  The paths in
+    // INPUTS name the calibration, model and output files as for the constructor above; the results are the same.
+    LocoMouse(LocoMouse_ParseInputs INPUTS, const LocoMouse_Parameters &params, const LocoMouse_Media &media, lm_ctx *ctx,
+              LocoMouse_DeviceFrames *decoded);
     virtual ~LocoMouse();
     LocoMouse(const LocoMouse &) = delete;
     LocoMouse &operator=(const LocoMouse &) = delete;
@@ -270,6 +298,8 @@ protected:
 
 public:
     explicit LocoMouse_TM(LocoMouse_ParseInputs INPUTS);
+    LocoMouse_TM(LocoMouse_ParseInputs INPUTS, const LocoMouse_Parameters &params, const LocoMouse_Media &media, lm_ctx *ctx,
+                 LocoMouse_DeviceFrames *decoded);
     void computeBoundingBox() override;
 
 protected:
@@ -283,8 +313,13 @@ protected:
 class LocoMouse_TM_DE : public LocoMouse_TM {
 public:
     explicit LocoMouse_TM_DE(LocoMouse_ParseInputs INPUTS);
+    LocoMouse_TM_DE(LocoMouse_ParseInputs INPUTS, const LocoMouse_Parameters &params, const LocoMouse_Media &media, lm_ctx *ctx,
+                    LocoMouse_DeviceFrames *decoded);
     void computeBoundingBox() override;
 };
 
 // LocoMouse_Methods.cpp:3-26
 std::unique_ptr<LocoMouse> LocoMouse_Initialize(LocoMouse_ParseInputs INPUT);
+// the same choice of class for the constructor on loaded inputs and a caller's context (see LocoMouse above)
+std::unique_ptr<LocoMouse> LocoMouse_Initialize(LocoMouse_ParseInputs INPUT, const LocoMouse_Parameters &params, const LocoMouse_Media &media,
+                                                lm_ctx *ctx, LocoMouse_DeviceFrames *decoded);

@@ -17,6 +17,7 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 #include <memory>
 #include <stdexcept>
 #include <string>
@@ -51,17 +52,16 @@ inline bool is_png(const std::string &name) {
     return h.size() >= 8 && !std::memcmp(h.data(), sig, 8);
 }
 
-// Storage of a PNG stream's payload (the class mirror passes page-locked memory so that the upload runs at the PCIe rate)
-struct HostAlloc {
-    void *(*alloc)(size_t) = [](size_t b) { return std::malloc(b ? b : 1); };
-    void (*release)(void *) = [](void *p) { std::free(p); };
-};
+// Where read_avi puts the pixels of an uncompressed stream or the frame chunks of a coded one: a buffer of the requested size
+// that the caller owns (the class mirror passes pooled page-locked memory, so that the frames are read from the file straight
+// into memory the upload runs from at the PCIe rate).  Without one they go to Video::frames / a malloc'ed Video::payload.
+using Dest = std::function<uint8_t *(size_t bytes)>;
 
 enum class Codec { raw, png, ffv1 };
 
 struct Video {
     int n = 0, rows = 0, cols = 0;
-    std::vector<uint8_t> frames;  // channel 0 of every frame, [n][rows][cols] (uncompressed streams)
+    std::vector<uint8_t> frames;  // channel 0 of every frame, [n][rows][cols] (uncompressed streams read without a Dest)
     // Compressed streams: frame i = payload[offsets[i], offsets[i + 1]), one frame chunk (a complete PNG file, or one FFV1
     // frame whose configuration record is `extradata`); `frames` stays empty
     Codec codec = Codec::raw;
@@ -87,8 +87,9 @@ inline void check_png_frame(const uint8_t *d, size_t len, int &rows, int &cols, 
         fail(std::to_string(w) + " x " + std::to_string(h) + " pixels, frame 0 has " + std::to_string(cols) + " x " + std::to_string(rows));
 }
 
-// Streams the frame chunks of stream 0 ('00db' / '00dc') in file order.
-inline Video read_avi(const std::string &name, const HostAlloc &halloc = HostAlloc()) {
+// Streams the frame chunks of stream 0 ('00db' / '00dc') in file order: a walk over the chunk headers, then one read per frame
+// chunk into the destination.
+inline Video read_avi(const std::string &name, const Dest &dest = nullptr) {
     FILE *f = std::fopen(name.c_str(), "rb");
     if (!f) throw std::runtime_error("Cannot open file: " + name);
     struct Closer {
@@ -109,6 +110,13 @@ inline Video read_avi(const std::string &name, const HostAlloc &halloc = HostAll
     int stream_index = -1;
     std::vector<uint8_t> chunk;
     std::vector<std::pair<int64_t, uint32_t>> coded_chunks;  // file offset and size of every PNG / FFV1 frame chunk
+    struct RawChunk {
+        int64_t at;
+        uint32_t size;
+        size_t stride;
+    };
+    std::vector<RawChunk> raw_chunks;                        // every uncompressed frame chunk
+    bool raw_grey = false, raw_rgb = false;
     std::vector<uint8_t> extradata;
     // A flat walk: LIST / RIFF headers are entered (only their 4-byte type is consumed), every other chunk is read or skipped.
     for (;;) {
@@ -172,29 +180,51 @@ inline Video read_avi(const std::string &name, const HostAlloc &halloc = HostAll
                  "YUV-planar video is outside this library (convert the video first).");
         }
         if (size == 0) continue;  // dropped frame: VideoCapture repeats nothing, it simply has one frame less
-        chunk.resize(size);
-        if (!rd(chunk.data(), size)) fail("truncated frame");
-        if (size & 1) skip(1);
-        const int bpp = bits / 8;
-        const size_t tight = (size_t)V.cols * bpp, padded = (tight + 3) & ~(size_t)3;
+        const size_t tight = (size_t)V.cols * (bits / 8), padded = (tight + 3) & ~(size_t)3;
         size_t stride;
         if (size >= padded * V.rows) stride = padded;
         else if (size >= tight * V.rows) stride = tight;
         else { fail("frame chunk smaller than one image"); return V; }
-        const bool bottom_up = rgb && height_signed > 0;  // BI_RGB DIBs are stored bottom-up unless the height is negative
-        const size_t base = V.frames.size();
-        V.frames.resize(base + (size_t)V.rows * V.cols);
-        for (int r = 0; r < V.rows; ++r) {
-            const uint8_t *src = chunk.data() + (size_t)(bottom_up ? V.rows - 1 - r : r) * stride;
-            uint8_t *dst = V.frames.data() + base + (size_t)r * V.cols;
-            if (bpp == 1) {
-                if (grey) std::memcpy(dst, src, (size_t)V.cols);
-                else for (int c = 0; c < V.cols; ++c) dst[c] = palette_b[src[c]];
-            } else {
-                for (int c = 0; c < V.cols; ++c) dst[c] = src[(size_t)c * bpp];  // B of BGR(A): channel 0
-            }
+        raw_grey = grey;
+        raw_rgb = rgb;
+        raw_chunks.push_back(RawChunk{(int64_t)ftello(f), size, stride});
+        if (!skip((uint64_t)size + (size & 1))) fail("truncated frame");
+    }
+    if (!raw_chunks.empty()) {
+        const size_t fsz = (size_t)V.rows * V.cols;
+        // a chunk must be in the file whole, also the bytes behind the image area that are not read
+        if (fseeko(f, 0, SEEK_END) != 0) fail("truncated frame");
+        const int64_t file_bytes = (int64_t)ftello(f);
+        uint8_t *out = nullptr;
+        if (dest) {
+            out = dest(raw_chunks.size() * fsz);
+            if (!out) fail("cannot allocate " + std::to_string(raw_chunks.size() * fsz) + " bytes for the frames");
+        } else {
+            V.frames.resize(raw_chunks.size() * fsz);
+            out = V.frames.data();
         }
-        ++V.n;
+        const int bpp = bits / 8;
+        const bool bottom_up = raw_rgb && height_signed > 0;  // BI_RGB DIBs are stored bottom-up unless the height is negative
+        for (const RawChunk &c : raw_chunks) {
+            const size_t stride = c.stride;
+            if (c.at + (int64_t)c.size > file_bytes) fail("truncated frame");
+            const bool direct = raw_grey && bpp == 1 && stride == (size_t)V.cols;  // the chunk is the frame: read it in place
+            uint8_t *frame = out + (size_t)V.n * fsz;
+            chunk.resize(stride * V.rows);
+            if (fseeko(f, (off_t)c.at, SEEK_SET) != 0 || !rd(direct ? frame : chunk.data(), direct ? fsz : chunk.size())) fail("truncated frame");
+            if (!direct)
+                for (int r = 0; r < V.rows; ++r) {
+                    const uint8_t *src = chunk.data() + (size_t)(bottom_up ? V.rows - 1 - r : r) * stride;
+                    uint8_t *dst = frame + (size_t)r * V.cols;
+                    if (bpp == 1) {
+                        if (raw_grey) std::memcpy(dst, src, (size_t)V.cols);
+                        else for (int c = 0; c < V.cols; ++c) dst[c] = palette_b[src[c]];
+                    } else {
+                        for (int c = 0; c < V.cols; ++c) dst[c] = src[(size_t)c * bpp];  // B of BGR(A): channel 0
+                    }
+                }
+            ++V.n;
+        }
     }
     if (V.codec == Codec::ffv1) {
         ffv1::Record rec;
@@ -206,9 +236,10 @@ inline Video read_avi(const std::string &name, const HostAlloc &halloc = HostAll
     if (!coded_chunks.empty()) {
         uint64_t total = 0;
         for (const auto &c : coded_chunks) total += c.second;
-        uint8_t *buf = static_cast<uint8_t *>(halloc.alloc((size_t)total));
+        uint8_t *buf = dest ? dest((size_t)total) : static_cast<uint8_t *>(std::malloc(total ? (size_t)total : 1));
         if (!buf) fail("cannot allocate " + std::to_string(total) + " bytes for the compressed frames");
-        V.payload = std::shared_ptr<uint8_t>(buf, halloc.release);
+        if (dest) V.payload = std::shared_ptr<uint8_t>(buf, [](uint8_t *) {});  // owned by the caller
+        else V.payload = std::shared_ptr<uint8_t>(buf, [](uint8_t *q) { std::free(q); });
         V.offsets.push_back(0);
         if (V.codec == Codec::png) V.rows = V.cols = 0;  // taken from frame 0's IHDR
         for (const auto &c : coded_chunks) {
