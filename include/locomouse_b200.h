@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define LM_ABI_VERSION 5  /* 5: lm_bounding_box_tm, and (backward compatible additions) lm_decode_png, lm_decode_ffv1, lm_device_alloc / lm_device_free, lm_get_info("ms_decode"), lm_get_info("device_allocs"); 4: lm_bounding_box_base, lm_mouse_box_size; 2: lm_set_option, lm_get_info, lm_debug_nms, lm_bounding_box_tm_de, lm_moving_average; 3: lm_host_alloc / lm_host_free, lm_unary_costs / lm_pairwise_costs, options streams 1..4, screen_layout, screen_priority */
+#define LM_ABI_VERSION 5  /* 5: lm_bounding_box_tm, and (backward compatible additions) lm_decode_png, lm_decode_ffv1, lm_device_alloc / lm_device_free / lm_device_copy, lm_get_info("ms_decode"), lm_get_info("device_allocs"); 4: lm_bounding_box_base, lm_mouse_box_size; 2: lm_set_option, lm_get_info, lm_debug_nms, lm_bounding_box_tm_de, lm_moving_average; 3: lm_host_alloc / lm_host_free, lm_unary_costs / lm_pairwise_costs, options streams 1..4, screen_layout, screen_priority */
 
 /* feature / view indices used in every [2] / [3] array below */
 enum { LM_PAW = 0, LM_SNOUT = 1, LM_TAIL = 2 };
@@ -323,6 +323,9 @@ int lm_decode_ffv1(lm_ctx *ctx, const uint8_t *extradata, int64_t extradata_len,
                    const int64_t *offsets, int64_t n, uint8_t *frames);
 int lm_device_alloc(lm_ctx *ctx, void **ptr, size_t bytes);   /* on the context's device, for callers without a CUDA runtime */
 int lm_device_free(lm_ctx *ctx, void *ptr);
+/* Copies `bytes` between two device buffers of the context's device on its stream and returns when the copy is done (a
+ * driver that streams decoded video keeps the last frame of one window as the previous frame of the next). */
+int lm_device_copy(lm_ctx *ctx, void *dst, const void *src, size_t bytes);
 
 /* measurement / debugging ---------------------------------------------------------------- */
 /* Device time (ms, CUDA events on the library's own stream) of the stages of the last

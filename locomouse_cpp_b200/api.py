@@ -27,7 +27,8 @@ EXPORTS = ("lm_abi_version", "lm_create", "lm_destroy", "lm_last_error", "lm_con
            "lm_set_background", "lm_set_calibration", "lm_get_geometry", "lm_detect_batch", "lm_last_timing",
            "lm_debug_fetch", "lm_set_option", "lm_get_info", "lm_debug_nms", "lm_bounding_box_tm_de", "lm_moving_average",
            "lm_host_alloc", "lm_host_free", "lm_unary_costs", "lm_pairwise_costs", "lm_bounding_box_base", "lm_mouse_box_size", "lm_bounding_box_tm",
-           "lm_decode_png", "lm_device_alloc", "lm_device_free", "lm_decode_ffv1")
+           "lm_decode_png", "lm_device_alloc", "lm_device_free", "lm_decode_ffv1",
+           "lm_device_copy")
 
 
 def _pinned_zeros(shape, dtype):
@@ -109,6 +110,8 @@ def load_library():
     L.lm_device_alloc.argtypes = [vp, C.POINTER(vp), C.c_size_t]
     L.lm_device_free.restype = C.c_int
     L.lm_device_free.argtypes = [vp, vp]
+    L.lm_device_copy.restype = C.c_int
+    L.lm_device_copy.argtypes = [vp, vp, vp, C.c_size_t]
     _lib = L
     return L
 

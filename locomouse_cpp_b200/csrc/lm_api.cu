@@ -1810,6 +1810,15 @@ int lm_device_free(lm_ctx *ctx, void *ptr) {
     return cudaFree(ptr) == cudaSuccess ? LM_OK : fail(ctx, LM_ERR_RUNTIME, "cudaFree failed");
 }
 
+int lm_device_copy(lm_ctx *ctx, void *dst, const void *src, size_t bytes) {
+    if (!ctx || (bytes && (!dst || !src))) return LM_ERR_INVALID;
+    if (!bytes) return LM_OK;
+    DeviceGuard guard(ctx->device);
+    cudaError_t e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    return e == cudaSuccess ? LM_OK : fail(ctx, LM_ERR_RUNTIME, "device copy of %zu bytes failed: %s", bytes, cudaGetErrorString(e));
+}
+
 // ---- lm_decode_png -----------------------------------------------------------------------------------------------------
 namespace {
 // Grows one of the context's PNG buffers to at least `bytes` (contents are not kept).

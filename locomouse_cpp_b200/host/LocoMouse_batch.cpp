@@ -12,9 +12,10 @@
 //
 // Every visible device (restrict with CUDA_VISIBLE_DEVICES) runs batch_workers_per_gpu workers (config key); a worker is one
 // host thread owning one lm_ctx.  Videos go through one shared queue, largest file first.  While a worker runs a video, a
-// reader thread reads its next one into the second of its two pooled page-locked buffers, so a worker holds at most two
-// videos in host memory (frames or coded chunks, plus background): the host footprint is about 2 x workers x the largest
-// video.  tracker_threads defaults to hardware threads / workers.  Each video runs exactly main()'s sequence on its worker's
+// reader thread reads the index and first window of its next one into the second of its two pooled page-locked buffers; a
+// video longer than one window (max_resident_bytes) reads its later windows into the worker's third buffer (LocoMouse_WindowPool)
+// while the device works on the one before.  So a worker holds at most three windows of frames or coded chunks in host
+// memory: the host footprint is at most 3 x workers x max_resident_bytes (less for videos shorter than a window).  tracker_threads defaults to hardware threads / workers.  Each video runs exactly main()'s sequence on its worker's
 // context and writes the files locomouse_b200 writes for it alone.  OUTPUT_FOLDER/batch_summary.tsv gets one row per video
 // of the list: status (ok, invalid, runtime, not run), device, frames, seconds of load (file read + construction) / pass 1 /
 // loop / tracks / export, and the message main() would have printed.  A failing video is recorded and the others go on; a
@@ -176,7 +177,7 @@ struct Shared {
 // One worker: one host thread, one context.
 void worker(Shared &S, int dev, lm_ctx *ctx) {
     LocoMouse_Media media[2];
-    LocoMouse_DeviceFrames decoded;
+    LocoMouse_WindowPool pool;
     struct Load {
         std::string status, message;  // empty: loaded
         double secs = 0;
@@ -185,7 +186,7 @@ void worker(Shared &S, int dev, lm_ctx *ctx) {
         Load r;
         const auto t0 = clk::now();
         try {
-            m->load(S.E[i].video, S.E[i].bkg);
+            m->load(S.E[i].video, S.E[i].bkg, (size_t)S.params.max_resident_bytes, S.params.batch_frames);
         } catch (const std::invalid_argument &e) {
             r.status = "invalid", r.message = std::string("Invalid inputs: ") + e.what();
         } catch (const std::exception &e) {
@@ -217,7 +218,7 @@ void worker(Shared &S, int dev, lm_ctx *ctx) {
             try {
                 // main()'s sequence (LocoMouse_main.cpp)
                 const auto t0 = clk::now();
-                std::unique_ptr<LocoMouse> L = LocoMouse_Initialize(in, S.params, media[slot], ctx, &decoded);
+                std::unique_ptr<LocoMouse> L = LocoMouse_Initialize(in, S.params, media[slot], ctx, &pool);
                 e.frames = L->N_frames();
                 const auto t1 = clk::now();
                 L->getBoundingBox();
@@ -273,7 +274,7 @@ void worker(Shared &S, int dev, lm_ctx *ctx) {
         }
         cur = next;
     }
-    decoded.release(ctx);
+    pool.release(ctx);
 }
 
 }  // namespace

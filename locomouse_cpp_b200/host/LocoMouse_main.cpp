@@ -60,8 +60,13 @@ int main(int argc, char *argv[]) {
         L->exportResults();
         const auto t5 = clk::now();
         // phases of the reference's main(): construction (file loading), pass 1, the per-frame loop, the tracker, export
+        // windows: how many pieces the video was read, decoded and tracked in (max_resident_bytes); resident_bytes: the page-locked
+        // bytes of frames held at the peak plus the device bytes of decoded frames; guard_violations: -1 unless LM_GUARD=1
+        double guard = -1;
+        lm_get_info(L->context(), "guard_violations", &guard);
         std::cout << "LM_TIMING frames=" << L->N_frames() << " load_s=" << secs(t0, t1) << " pass1_s=" << secs(t1, t2) << " loop_s=" << secs(t2, t3)
-                  << " tracks_s=" << secs(t3, t4) << " export_s=" << secs(t4, t5) << " warm_loop_s=" << warm_loop_s << std::endl;
+                  << " tracks_s=" << secs(t3, t4) << " export_s=" << secs(t4, t5) << " warm_loop_s=" << warm_loop_s << " windows=" << L->windows()
+                  << " resident_bytes=" << L->residentBytes() << " guard_violations=" << guard << std::endl;
     } catch (const std::invalid_argument &e) {
         std::cout << "Invalid inputs: " << e.what() << std::endl;
         return_val = EXIT_FAILURE;

@@ -3,6 +3,7 @@
 // and OpenCV-YAML parsing are outside the hot path (SURVEY §8f-3); these little-endian containers carry
 // exactly the arrays those loaders would produce, so the class mirror can be driven end to end.
 //   video        "LMV1" i32 n_frames, rows, cols        then n*rows*cols u8      (channel 0 of each frame)
+//                       (read in frame ranges by lmmedia::index_lmv + read_frames, lm_media.hpp)
 //   background   "LMI1" i32 rows, cols                  then rows*cols u8
 //   model        "LMM1" 6 x { i32 rows, cols; f64 rho; rows*cols f32 }  in the order
 //                       paw_bottom, snout_bottom, tail_bottom, paw_side, snout_side, tail_side

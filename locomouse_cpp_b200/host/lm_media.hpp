@@ -10,13 +10,15 @@
 // checked here (ffv1_format.h) and so is every frame's keyframe bit.  Other compressed or YUV-planar streams need a decoder
 // that is outside this library: they are refused with a message that says so.  Background: PNG, 8 bits per channel, non-interlaced; colour images are
 // reduced to grey as libpng does for OpenCV (png_set_rgb_to_gray with 0.299 / 0.587).  Both are checked against what the
-// real OpenCV reads from the same files (tests/test_host_media.py).
+// real OpenCV reads from the same files (tests/test_host_media.py).  A video is read in two steps, so that a long one can be
+// streamed: index_avi walks the chunk headers once, read_frames reads any range of frames (tests/test_avi_ranges.py).
 #pragma once
 #include <zlib.h>
 
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
+#include <algorithm>
 #include <functional>
 #include <memory>
 #include <stdexcept>
@@ -87,37 +89,58 @@ inline void check_png_frame(const uint8_t *d, size_t len, int &rows, int &cols, 
         fail(std::to_string(w) + " x " + std::to_string(h) + " pixels, frame 0 has " + std::to_string(cols) + " x " + std::to_string(rows));
 }
 
-// Streams the frame chunks of stream 0 ('00db' / '00dc') in file order: a walk over the chunk headers, then one read per frame
-// chunk into the destination.
-inline Video read_avi(const std::string &name, const Dest &dest = nullptr) {
-    FILE *f = std::fopen(name.c_str(), "rb");
-    if (!f) throw std::runtime_error("Cannot open file: " + name);
-    struct Closer {
-        FILE *f;
-        ~Closer() { std::fclose(f); }
-    } closer{f};
-    auto fail = [&](const std::string &why) -> void { throw std::runtime_error("Video file " + name + ": " + why); };
-    auto rd = [&](void *dst, size_t n) { return std::fread(dst, 1, n, f) == n; };
-    auto skip = [&](uint64_t n) { return fseeko(f, (off_t)n, SEEK_CUR) == 0; };
-    uint8_t h[12];
-    if (!rd(h, 12) || std::memcmp(h, "RIFF", 4) || std::memcmp(h + 8, "AVI ", 4)) fail("not an AVI file");
-    Video V;
-    int bits = 0, height_signed = 0;
-    uint32_t fourcc = 0;
-    uint8_t palette_b[256];
-    for (int i = 0; i < 256; ++i) palette_b[i] = (uint8_t)i;
-    bool have_format = false, stream0_is_video = false;
-    int stream_index = -1;
-    std::vector<uint8_t> chunk;
-    std::vector<std::pair<int64_t, uint32_t>> coded_chunks;  // file offset and size of every PNG / FFV1 frame chunk
+// Where every frame of a video lies in its file: the result of one walk over the chunk headers (index_avi, or index_lmv for
+// the LMV1 container of lm_files.hpp), from which read_frames reads any range of frames.  Every chunk is checked against the
+// file size here, so a truncated chunk is refused before any frame is used, wherever it lies.
+struct Index {
+    std::string name;
+    int n = 0, rows = 0, cols = 0;
+    Codec codec = Codec::raw;
+    // uncompressed frames: chunk position, size and row stride; channel-0 extraction as extractChannel(F, F, 0) takes it
     struct RawChunk {
         int64_t at;
         uint32_t size;
         size_t stride;
     };
-    std::vector<RawChunk> raw_chunks;                        // every uncompressed frame chunk
-    bool raw_grey = false, raw_rgb = false;
-    std::vector<uint8_t> extradata;
+    std::vector<RawChunk> raw;
+    int bpp = 1;
+    bool grey = true, bottom_up = false;
+    uint8_t palette_b[256] = {};
+    // coded frames: file offset and size of every frame chunk; FFV1: every frame's keyframe bit and the configuration record
+    std::vector<std::pair<int64_t, uint32_t>> coded;
+    std::vector<uint8_t> keyframe, extradata;
+};
+
+namespace detail {
+struct File {
+    FILE *f;
+    explicit File(const std::string &name) : f(std::fopen(name.c_str(), "rb")) {
+        if (!f) throw std::runtime_error("Cannot open file: " + name);
+    }
+    ~File() { std::fclose(f); }
+    bool read(void *dst, size_t n) { return std::fread(dst, 1, n, f) == n; }
+    bool seek(int64_t at) { return fseeko(f, (off_t)at, SEEK_SET) == 0; }
+    int64_t size() { return fseeko(f, 0, SEEK_END) == 0 ? (int64_t)ftello(f) : -1; }
+};
+}  // namespace detail
+
+// The walk over stream 0's frame chunks ('00db' / '00dc') in file order, with the format and record checks.
+inline Index index_avi(const std::string &name) {
+    detail::File file(name);
+    FILE *f = file.f;
+    auto fail = [&](const std::string &why) -> void { throw std::runtime_error("Video file " + name + ": " + why); };
+    auto rd = [&](void *dst, size_t n) { return file.read(dst, n); };
+    auto skip = [&](uint64_t n) { return fseeko(f, (off_t)n, SEEK_CUR) == 0; };
+    uint8_t h[12];
+    if (!rd(h, 12) || std::memcmp(h, "RIFF", 4) || std::memcmp(h + 8, "AVI ", 4)) fail("not an AVI file");
+    Index V;
+    V.name = name;
+    int bits = 0, height_signed = 0;
+    uint32_t fourcc = 0;
+    for (int i = 0; i < 256; ++i) V.palette_b[i] = (uint8_t)i;
+    bool have_format = false, stream0_is_video = false, raw_rgb = false;
+    int stream_index = -1;
+    std::vector<uint8_t> chunk;
     // A flat walk: LIST / RIFF headers are entered (only their 4-byte type is consumed), every other chunk is read or skipped.
     for (;;) {
         uint8_t ch[8];
@@ -149,9 +172,9 @@ inline Video read_avi(const std::string &name, const Dest &dest = nullptr) {
             bits = chunk[14] | (chunk[15] << 8);
             fourcc = le32(chunk.data() + 16);
             const uint32_t used = le32(chunk.data() + 32);
-            extradata.assign(chunk.begin() + 40, chunk.end());
+            V.extradata.assign(chunk.begin() + 40, chunk.end());
             const size_t ncol = used ? used : (bits <= 8 ? (size_t)1 << bits : 0);
-            for (size_t i = 0; i < ncol && 40 + 4 * i + 3 < size && i < 256; ++i) palette_b[i] = chunk[40 + 4 * i];  // RGBQUAD: blue first
+            for (size_t i = 0; i < ncol && 40 + 4 * i + 3 < size && i < 256; ++i) V.palette_b[i] = chunk[40 + 4 * i];  // RGBQUAD: blue first
             have_format = true;
             continue;
         }
@@ -165,11 +188,11 @@ inline Video read_avi(const std::string &name, const Dest &dest = nullptr) {
         const bool grey = fourcc == cc("Y800") || fourcc == cc("GREY") || fourcc == cc("Y8  ") || fourcc == cc("Y8\0\0");
         const bool rgb = fourcc == 0 || fourcc == cc("DIB ") || fourcc == cc("RGB ") || fourcc == cc("RAW ");
         const bool png = fourcc == cc("MPNG") || fourcc == cc("png ");
-        if (png || fourcc == cc("FFV1")) {  // read after the walk, straight into the payload
+        if (png || fourcc == cc("FFV1")) {
             if (size == 0) continue;
             V.codec = png ? Codec::png : Codec::ffv1;
             const off_t at = ftello(f);
-            coded_chunks.emplace_back((int64_t)at, size);
+            V.coded.emplace_back((int64_t)at, size);
             if (!skip((uint64_t)size + (size & 1))) fail("truncated frame");
             continue;
         }
@@ -185,75 +208,167 @@ inline Video read_avi(const std::string &name, const Dest &dest = nullptr) {
         if (size >= padded * V.rows) stride = padded;
         else if (size >= tight * V.rows) stride = tight;
         else { fail("frame chunk smaller than one image"); return V; }
-        raw_grey = grey;
+        V.grey = grey;
         raw_rgb = rgb;
-        raw_chunks.push_back(RawChunk{(int64_t)ftello(f), size, stride});
+        V.raw.push_back(Index::RawChunk{(int64_t)ftello(f), size, stride});
         if (!skip((uint64_t)size + (size & 1))) fail("truncated frame");
     }
-    if (!raw_chunks.empty()) {
-        const size_t fsz = (size_t)V.rows * V.cols;
-        // a chunk must be in the file whole, also the bytes behind the image area that are not read
-        if (fseeko(f, 0, SEEK_END) != 0) fail("truncated frame");
-        const int64_t file_bytes = (int64_t)ftello(f);
-        uint8_t *out = nullptr;
-        if (dest) {
-            out = dest(raw_chunks.size() * fsz);
-            if (!out) fail("cannot allocate " + std::to_string(raw_chunks.size() * fsz) + " bytes for the frames");
-        } else {
-            V.frames.resize(raw_chunks.size() * fsz);
-            out = V.frames.data();
-        }
-        const int bpp = bits / 8;
-        const bool bottom_up = raw_rgb && height_signed > 0;  // BI_RGB DIBs are stored bottom-up unless the height is negative
-        for (const RawChunk &c : raw_chunks) {
-            const size_t stride = c.stride;
-            if (c.at + (int64_t)c.size > file_bytes) fail("truncated frame");
-            const bool direct = raw_grey && bpp == 1 && stride == (size_t)V.cols;  // the chunk is the frame: read it in place
-            uint8_t *frame = out + (size_t)V.n * fsz;
-            chunk.resize(stride * V.rows);
-            if (fseeko(f, (off_t)c.at, SEEK_SET) != 0 || !rd(direct ? frame : chunk.data(), direct ? fsz : chunk.size())) fail("truncated frame");
-            if (!direct)
-                for (int r = 0; r < V.rows; ++r) {
-                    const uint8_t *src = chunk.data() + (size_t)(bottom_up ? V.rows - 1 - r : r) * stride;
-                    uint8_t *dst = frame + (size_t)r * V.cols;
-                    if (bpp == 1) {
-                        if (raw_grey) std::memcpy(dst, src, (size_t)V.cols);
-                        else for (int c = 0; c < V.cols; ++c) dst[c] = palette_b[src[c]];
-                    } else {
-                        for (int c = 0; c < V.cols; ++c) dst[c] = src[(size_t)c * bpp];  // B of BGR(A): channel 0
-                    }
-                }
-            ++V.n;
-        }
+    // a chunk must be in the file whole, also the bytes behind the image area that are not read
+    const int64_t file_bytes = file.size();
+    if (file_bytes < 0) fail("truncated frame");
+    for (const Index::RawChunk &c : V.raw)
+        if (c.at + (int64_t)c.size > file_bytes) fail("truncated frame");
+    for (const auto &c : V.coded)
+        if (c.first + (int64_t)c.second > file_bytes) fail("truncated frame");
+    V.bpp = bits / 8;
+    V.bottom_up = raw_rgb && height_signed > 0;  // BI_RGB DIBs are stored bottom-up unless the height is negative
+    if (!V.raw.empty()) {
+        V.codec = Codec::raw;
+        V.coded.clear();
+        V.n = (int)V.raw.size();
+    } else {
+        V.n = (int)V.coded.size();
     }
     if (V.codec == Codec::ffv1) {
         ffv1::Record rec;
         char why[200];
-        if (ffv1::parse_record(extradata.data(), (int64_t)extradata.size(), V.rows, V.cols, rec, nullptr, nullptr, why, sizeof why))
+        if (ffv1::parse_record(V.extradata.data(), (int64_t)V.extradata.size(), V.rows, V.cols, rec, nullptr, nullptr, why, sizeof why))
             fail(std::string("FFV1 configuration record: ") + why);
-        V.extradata = std::move(extradata);
-    }
-    if (!coded_chunks.empty()) {
-        uint64_t total = 0;
-        for (const auto &c : coded_chunks) total += c.second;
-        uint8_t *buf = dest ? dest((size_t)total) : static_cast<uint8_t *>(std::malloc(total ? (size_t)total : 1));
-        if (!buf) fail("cannot allocate " + std::to_string(total) + " bytes for the compressed frames");
-        if (dest) V.payload = std::shared_ptr<uint8_t>(buf, [](uint8_t *) {});  // owned by the caller
-        else V.payload = std::shared_ptr<uint8_t>(buf, [](uint8_t *q) { std::free(q); });
-        V.offsets.push_back(0);
-        if (V.codec == Codec::png) V.rows = V.cols = 0;  // taken from frame 0's IHDR
-        for (const auto &c : coded_chunks) {
-            uint8_t *d = buf + V.offsets.back();
-            if (fseeko(f, (off_t)c.first, SEEK_SET) != 0 || !rd(d, c.second)) fail("truncated frame");
-            const std::string where = "Video file " + name + ", frame " + std::to_string(V.n);
-            if (V.codec == Codec::png) check_png_frame(d, c.second, V.rows, V.cols, where);
-            else if (V.n == 0 && !ffv1::keyframe_bit(d, c.second)) throw std::runtime_error(where + ": the first FFV1 frame is not a keyframe");
-            V.offsets.push_back(V.offsets.back() + c.second);
-            ++V.n;
+        V.keyframe.resize(V.coded.size());
+        for (size_t i = 0; i < V.coded.size(); ++i) {  // the first two bytes of each chunk hold its keyframe bit
+            uint8_t d[2] = {0, 0};
+            const uint32_t len = std::min<uint32_t>(V.coded[i].second, 2);
+            if (!file.seek(V.coded[i].first) || !rd(d, len)) fail("truncated frame");
+            V.keyframe[i] = (uint8_t)ffv1::keyframe_bit(d, len);
         }
+        if (!V.keyframe.empty() && !V.keyframe[0])
+            throw std::runtime_error("Video file " + name + ", frame 0: the first FFV1 frame is not a keyframe");
+    } else {
+        V.extradata.clear();
+    }
+    if (V.codec == Codec::png && !V.coded.empty()) {  // the size is frame 0's (IHDR); read_frames checks every other frame against it
+        uint8_t d[45];
+        const uint32_t len = std::min<uint32_t>(V.coded[0].second, sizeof d);
+        V.rows = V.cols = 0;
+        if (!file.seek(V.coded[0].first) || !rd(d, len)) fail("truncated frame");
+        check_png_frame(d, V.coded[0].second < sizeof d ? V.coded[0].second : sizeof d, V.rows, V.cols, "Video file " + name + ", frame 0");
     }
     if (V.n == 0) fail("no video frames found");
     return V;
+}
+
+// The LMV1 container (lm_files.hpp): a header, then every frame's rows x cols bytes back to back.
+inline Index index_lmv(const std::string &name) {
+    detail::File file(name);
+    uint8_t h[16];
+    if (!file.read(h, 4) || std::memcmp(h, "LMV1", 4)) throw std::runtime_error("Unexpected file format (LMV1 expected): " + name);
+    if (!file.read(h + 4, 12)) throw std::runtime_error("File is truncated: " + name);
+    Index V;
+    V.name = name;
+    V.n = (int)le32(h + 4);
+    V.rows = (int)le32(h + 8);
+    V.cols = (int)le32(h + 12);
+    if (V.n <= 0 || V.rows <= 0 || V.cols <= 0) throw std::runtime_error("Video file is empty: " + name);
+    const size_t fsz = (size_t)V.rows * V.cols;
+    if (file.size() < 16 + (int64_t)(fsz * V.n)) throw std::runtime_error("File is truncated: " + name);
+    V.raw.reserve((size_t)V.n);
+    for (int i = 0; i < V.n; ++i) V.raw.push_back(Index::RawChunk{16 + (int64_t)(fsz * i), (uint32_t)fsz, (size_t)V.cols});
+    return V;
+}
+
+// An AVI file, or else the LMV1 container.
+inline Index index_video(const std::string &name) { return is_avi(name) ? index_avi(name) : index_lmv(name); }
+
+// Frames [first, first + n) of an indexed video.  Uncompressed: channel 0 of each frame, [n][rows][cols]; coded: the frame
+// chunks back to back, with offsets relative to the first of them (PNG frames are checked here against frame 0's size).
+inline Video read_frames(const Index &ix, int first, int n, const Dest &dest = nullptr) {
+    if (first < 0 || n <= 0 || first + n > ix.n) throw std::runtime_error("Video file " + ix.name + ": frame range outside the video");
+    detail::File file(ix.name);
+    auto fail = [&](const std::string &why) -> void { throw std::runtime_error("Video file " + ix.name + ": " + why); };
+    Video V;
+    V.rows = ix.rows;
+    V.cols = ix.cols;
+    V.codec = ix.codec;
+    if (ix.codec == Codec::raw) {
+        const size_t fsz = (size_t)V.rows * V.cols;
+        uint8_t *out = nullptr;
+        if (dest) {
+            out = dest((size_t)n * fsz);
+            if (!out) fail("cannot allocate " + std::to_string((size_t)n * fsz) + " bytes for the frames");
+        } else {
+            V.frames.resize((size_t)n * fsz);
+            out = V.frames.data();
+        }
+        std::vector<uint8_t> chunk;
+        for (int i = 0; i < n; ++i) {
+            const Index::RawChunk &c = ix.raw[(size_t)(first + i)];
+            const size_t stride = c.stride;
+            const bool direct = ix.grey && ix.bpp == 1 && stride == (size_t)V.cols;  // the chunk is the frame: read it in place
+            uint8_t *frame = out + (size_t)i * fsz;
+            chunk.resize(stride * V.rows);
+            if (!file.seek(c.at) || !file.read(direct ? frame : chunk.data(), direct ? fsz : chunk.size())) fail("truncated frame");
+            if (!direct)
+                for (int r = 0; r < V.rows; ++r) {
+                    const uint8_t *src = chunk.data() + (size_t)(ix.bottom_up ? V.rows - 1 - r : r) * stride;
+                    uint8_t *dst = frame + (size_t)r * V.cols;
+                    if (ix.bpp == 1) {
+                        if (ix.grey) std::memcpy(dst, src, (size_t)V.cols);
+                        else for (int x = 0; x < V.cols; ++x) dst[x] = ix.palette_b[src[x]];
+                    } else {
+                        for (int x = 0; x < V.cols; ++x) dst[x] = src[(size_t)x * ix.bpp];  // B of BGR(A): channel 0
+                    }
+                }
+        }
+        V.n = n;
+        return V;
+    }
+    uint64_t total = 0;
+    for (int i = 0; i < n; ++i) total += ix.coded[(size_t)(first + i)].second;
+    uint8_t *buf = dest ? dest((size_t)total) : static_cast<uint8_t *>(std::malloc(total ? (size_t)total : 1));
+    if (!buf) fail("cannot allocate " + std::to_string(total) + " bytes for the compressed frames");
+    if (dest) V.payload = std::shared_ptr<uint8_t>(buf, [](uint8_t *) {});  // owned by the caller
+    else V.payload = std::shared_ptr<uint8_t>(buf, [](uint8_t *q) { std::free(q); });
+    V.offsets.push_back(0);
+    for (int i = 0; i < n; ++i) {
+        const auto &c = ix.coded[(size_t)(first + i)];
+        uint8_t *d = buf + V.offsets.back();
+        if (!file.seek(c.first) || !file.read(d, c.second)) fail("truncated frame");
+        if (ix.codec == Codec::png) check_png_frame(d, c.second, V.rows, V.cols, "Video file " + ix.name + ", frame " + std::to_string(first + i));
+        V.offsets.push_back(V.offsets.back() + c.second);
+    }
+    V.n = n;
+    V.extradata = ix.extradata;
+    return V;
+}
+
+// The whole video: its index, then every frame in one read.
+inline Video read_avi(const std::string &name, const Dest &dest = nullptr) {
+    const Index ix = index_avi(name);
+    return read_frames(ix, 0, ix.n, dest);
+}
+
+// Window length for a budget of `max_bytes` of frames: whole multiples of batch_frames, at least one.
+inline int window_frames(size_t max_bytes, size_t frame_bytes, int batch_frames) {
+    const size_t w = max_bytes / frame_bytes / (size_t)batch_frames * (size_t)batch_frames;
+    return (int)std::min<size_t>(std::max<size_t>(w, (size_t)batch_frames), (size_t)1 << 30);
+}
+
+// The first frame of every window of at most W frames, then n.  A video of n <= W frames is one window.  FFV1 (keyframe
+// given): a window ends just before a keyframe, so that each window decodes on its own; a GOP longer than W is one window.
+inline std::vector<int> plan_windows(int n, int W, const std::vector<uint8_t> &keyframe) {
+    std::vector<int> s{0};
+    while (n - s.back() > W) {
+        const int a = s.back();
+        int b = a + W;
+        if (!keyframe.empty()) {
+            while (b > a && !keyframe[(size_t)b]) --b;                       // the last keyframe in (a, a + W]
+            if (b == a)
+                for (b = a + W + 1; b < n && !keyframe[(size_t)b]; ++b) {}  // none: the window runs to the next keyframe
+        }
+        s.push_back(b);
+    }
+    if (s.back() != n) s.push_back(n);
+    return s;
 }
 
 struct Image {

@@ -139,6 +139,42 @@ int lmh_read_avi_ffv1(const char *path, int64_t *dims, uint8_t *payload, int64_t
         return 1;
     }
 }
+// Frames [first, first + count) of an AVI or LMV1 video through lmmedia::index_video + read_frames: dims = {n (whole video),
+// rows, cols, codec (0 raw, 1 PNG, 2 FFV1), bytes of the range}.  out receives the pixels (raw) or the frame chunks (coded, with
+// offsets[count + 1] relative to the first); with out NULL only dims are returned.  0 ok, 1 error (msg filled)
+int lmh_read_avi_range(const char *path, int64_t first, int64_t count, int64_t *dims, uint8_t *out, int64_t *offsets, char *msg, int msg_cap) {
+    try {
+        const lmmedia::Index ix = lmmedia::index_video(path);
+        dims[0] = ix.n;
+        dims[1] = ix.rows;
+        dims[2] = ix.cols;
+        dims[3] = (int64_t)ix.codec;
+        dims[4] = 0;
+        if (count <= 0) return 0;
+        const lmmedia::Video V = lmmedia::read_frames(ix, (int)first, (int)count);
+        dims[4] = V.codec == lmmedia::Codec::raw ? (int64_t)V.frames.size() : V.offsets.back();
+        if (out) std::memcpy(out, V.codec == lmmedia::Codec::raw ? V.frames.data() : V.payload.get(), (size_t)dims[4]);
+        if (offsets && V.codec != lmmedia::Codec::raw) std::memcpy(offsets, V.offsets.data(), V.offsets.size() * sizeof(int64_t));
+        return 0;
+    } catch (const std::exception &e) {
+        if (msg && msg_cap > 0) std::snprintf(msg, (size_t)msg_cap, "%s", e.what());
+        return 1;
+    }
+}
+// The windows LocoMouse streams a video through for a budget of max_bytes frame bytes and batch_frames: starts[] receives
+// the first frame of each window, then the number of frames.  Returns the number of windows, or -1 (msg filled).
+int lmh_plan_windows(const char *path, int64_t max_bytes, int batch_frames, int32_t *starts, int cap, char *msg, int msg_cap) {
+    try {
+        const lmmedia::Index ix = lmmedia::index_video(path);
+        const int W = lmmedia::window_frames((size_t)max_bytes, (size_t)ix.rows * ix.cols, batch_frames);
+        const std::vector<int> s = lmmedia::plan_windows(ix.n, W, ix.keyframe);
+        for (size_t i = 0; i < s.size() && (int)i < cap; ++i) starts[i] = s[i];
+        return (int)s.size() - 1;
+    } catch (const std::exception &e) {
+        if (msg && msg_cap > 0) std::snprintf(msg, (size_t)msg_cap, "%s", e.what());
+        return -1;
+    }
+}
 // ffv1_format.h run serially on the CPU: the record parse and the chain decode that k_ffv1.cu runs per thread, for the CPU
 // tests.  out: [n][rows][cols].  0 ok, 1 error (msg names the record problem, or the first bad frame and slice)
 int lmh_decode_ffv1(const uint8_t *extradata, int64_t extradata_len, const uint8_t *payload, const int64_t *offsets, int64_t n, int rows,
