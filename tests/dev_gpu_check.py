@@ -9,11 +9,14 @@ import time
 import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 from locomouse_cpp_b200 import synth  # noqa: E402
 from locomouse_cpp_b200.api import Detector  # noqa: E402
 from locomouse_cpp_b200.types import diff_results  # noqa: E402
 from oracle import oracle  # noqa: E402
+
+import _preprocess_designs as designs  # noqa: E402
 
 
 def main():
@@ -48,29 +51,19 @@ def main():
     got = det.detect_batch(fr, bx, bs, bb, allow_overflow=True)
     print(f"gpu: {time.time() - t:.3f}s rc={got.rc} timing={det.last_timing()}")
 
-    # stage diagnostics on the last sub-batch
+    # stage diagnostics on the last sub-batch (windows placed and sized by tests/_preprocess_designs.py)
     for f in range(args.frames):
         I, mm = oracle.preprocess(cfg, bkg, calib, frames_np[f])
         try:
             gmm, _ = det.debug_fetch(3, f)
-        except Exception as e:  # frame not in last sub-batch
+        except Exception:  # frame not in last sub-batch
             continue
         if not np.array_equal(gmm, mm):
             print(f"frame {f}: minmax gpu {gmm} oracle {mm}")
-        for v, (ypos, h) in enumerate(((bb[f], cfg.bb_h_bottom), (bs[f], cfg.bb_h_side))):
+        for v, ypos in ((0, bb[f]), (1, bs[f])):
             win, dims = det.debug_fetch(v, f)
-            hy, hx = int(dims[2]), int(dims[3])
-            x0 = int(bx[f]) - cfg.bb_w + 1 - hx
-            y0 = int(ypos) - h + 1 - hy
-            exp = np.zeros_like(win)
-            H, P = win.shape
-            ys = np.arange(y0, y0 + H)
-            xs = np.arange(x0, x0 + P)
-            yv = (ys >= 0) & (ys < cfg.n_rows)
-            xv = (xs >= 0) & (xs < cfg.n_cols)
-            exp[np.ix_(yv, xv)] = I[np.ix_(ys[yv], xs[xv])]
-            win_w = cfg.bb_w + hx + (spec.scaled().tsize - 1 - hx)
-            exp[:, win_w:] = 0  # pitch padding must be zero
+            x0, y0, win_w, _ = designs.window_origin(cfg, model, v, bx[f], ypos)
+            exp = designs.expected_window(I, x0, y0, win.shape[0], win.shape[1], win_w)
             ncmp = (win != exp)
             if ncmp.any():
                 idx = np.argwhere(ncmp)
