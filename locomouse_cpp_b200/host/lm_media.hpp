@@ -8,10 +8,13 @@
 // offsets, for lm_decode_png to decode on the device.  FFV1-coded streams ('FFV1', lossless, version 3 as libavcodec writes
 // it) are returned the same way, with the configuration record from 'strf' as extradata, for lm_decode_ffv1; the record is
 // checked here (ffv1_format.h) and so is every frame's keyframe bit.  Other compressed or YUV-planar streams need a decoder
-// that is outside this library: they are refused with a message that says so.  Background: PNG, 8 bits per channel, non-interlaced; colour images are
+// that is outside this library: they are refused with a message that says so.  The same frames in Matroska and QuickTime / MP4
+// files are indexed by lm_containers.hpp into the same Index; index_video picks the container by signature (AVI, Matroska,
+// ISO BMFF, LMV1).  Background: PNG, 8 bits per channel, non-interlaced; colour images are
 // reduced to grey as libpng does for OpenCV (png_set_rgb_to_gray with 0.299 / 0.587).  Both are checked against what the
 // real OpenCV reads from the same files (tests/test_host_media.py).  A video is read in two steps, so that a long one can be
-// streamed: index_avi walks the chunk headers once, read_frames reads any range of frames (tests/test_avi_ranges.py).
+// streamed: index_avi (index_mkv, index_mov) walks the file's structure once, read_frames reads any range of frames
+// (tests/test_avi_ranges.py, tests/test_containers.py).
 #pragma once
 #include <zlib.h>
 
@@ -103,7 +106,7 @@ struct Index {
         size_t stride;
     };
     std::vector<RawChunk> raw;
-    int bpp = 1;
+    int bpp = 1, channel0 = 0;  // bytes per pixel; byte of channel 0 in a pixel (2 where a container stores RGB, not BGR)
     bool grey = true, bottom_up = false;
     uint8_t palette_b[256] = {};
     // coded frames: file offset and size of every frame chunk; FFV1: every frame's keyframe bit and the configuration record
@@ -123,6 +126,49 @@ struct File {
     int64_t size() { return fseeko(f, 0, SEEK_END) == 0 ? (int64_t)ftello(f) : -1; }
 };
 }  // namespace detail
+
+// The checks every container's index ends with (index_avi, index_mkv, index_mov), once V.n, the codec, the chunks and the
+// record are set: every chunk lies inside the file, also the bytes behind the image area that are not read; an FFV1 stream's
+// record parses and every frame's keyframe bit is recorded, frame 0's set; a PNG stream's size is frame 0's IHDR.
+inline void finish_index(Index &V, detail::File &file) {
+    auto fail = [&](const std::string &why) -> void { throw std::runtime_error("Video file " + V.name + ": " + why); };
+    const int64_t file_bytes = file.size();
+    if (file_bytes < 0) fail("truncated frame");
+    for (const Index::RawChunk &c : V.raw)
+        if (c.at + (int64_t)c.size > file_bytes) fail("truncated frame");
+    for (const auto &c : V.coded)
+        if (c.first + (int64_t)c.second > file_bytes) fail("truncated frame");
+    if (V.codec == Codec::ffv1) {
+        ffv1::Record rec;
+        char why[200];
+        if (ffv1::parse_record(V.extradata.data(), (int64_t)V.extradata.size(), V.rows, V.cols, rec, nullptr, nullptr, why, sizeof why))
+            fail(std::string("FFV1 configuration record: ") + why);
+        V.keyframe.resize(V.coded.size());
+        for (size_t i = 0; i < V.coded.size(); ++i) {  // the first two bytes of each chunk hold its keyframe bit
+            uint8_t d[2] = {0, 0};
+            const uint32_t len = std::min<uint32_t>(V.coded[i].second, 2);
+            if (!file.seek(V.coded[i].first) || !file.read(d, len)) fail("truncated frame");
+            V.keyframe[i] = (uint8_t)ffv1::keyframe_bit(d, len);
+        }
+        if (!V.keyframe.empty() && !V.keyframe[0])
+            throw std::runtime_error("Video file " + V.name + ", frame 0: the first FFV1 frame is not a keyframe");
+    } else {
+        V.extradata.clear();
+    }
+    if (V.codec == Codec::png && !V.coded.empty()) {  // the size is frame 0's (IHDR); read_frames checks every other frame against it
+        uint8_t d[45];
+        const uint32_t len = std::min<uint32_t>(V.coded[0].second, sizeof d);
+        V.rows = V.cols = 0;
+        if (!file.seek(V.coded[0].first) || !file.read(d, len)) fail("truncated frame");
+        check_png_frame(d, V.coded[0].second < sizeof d ? V.coded[0].second : sizeof d, V.rows, V.cols, "Video file " + V.name + ", frame 0");
+    }
+    if (V.n == 0) fail("no video frames found");
+}
+
+// What a refusal of a stream this library does not decode ends with.
+inline const char *outside_this_library() {
+    return "Decoding compressed or YUV-planar video is outside this library (convert the video first).";
+}
 
 // The walk over stream 0's frame chunks ('00db' / '00dc') in file order, with the format and record checks.
 inline Index index_avi(const std::string &name) {
@@ -199,8 +245,7 @@ inline Index index_avi(const std::string &name) {
         if (!(grey && bits == 8) && !(rgb && (bits == 8 || bits == 24 || bits == 32))) {
             char fc[5] = {(char)(fourcc & 255), (char)((fourcc >> 8) & 255), (char)((fourcc >> 16) & 255), (char)((fourcc >> 24) & 255), 0};
             fail(std::string("stream 0 is '") + fc + "' with " + std::to_string(bits) +
-                 " bits per pixel; only uncompressed 8-bit grey (Y800) and BI_RGB 8 / 24 / 32-bit frames are read here. Decoding compressed or "
-                 "YUV-planar video is outside this library (convert the video first).");
+                 " bits per pixel; only uncompressed 8-bit grey (Y800) and BI_RGB 8 / 24 / 32-bit frames are read here. " + outside_this_library());
         }
         if (size == 0) continue;  // dropped frame: VideoCapture repeats nothing, it simply has one frame less
         const size_t tight = (size_t)V.cols * (bits / 8), padded = (tight + 3) & ~(size_t)3;
@@ -213,13 +258,6 @@ inline Index index_avi(const std::string &name) {
         V.raw.push_back(Index::RawChunk{(int64_t)ftello(f), size, stride});
         if (!skip((uint64_t)size + (size & 1))) fail("truncated frame");
     }
-    // a chunk must be in the file whole, also the bytes behind the image area that are not read
-    const int64_t file_bytes = file.size();
-    if (file_bytes < 0) fail("truncated frame");
-    for (const Index::RawChunk &c : V.raw)
-        if (c.at + (int64_t)c.size > file_bytes) fail("truncated frame");
-    for (const auto &c : V.coded)
-        if (c.first + (int64_t)c.second > file_bytes) fail("truncated frame");
     V.bpp = bits / 8;
     V.bottom_up = raw_rgb && height_signed > 0;  // BI_RGB DIBs are stored bottom-up unless the height is negative
     if (!V.raw.empty()) {
@@ -229,31 +267,7 @@ inline Index index_avi(const std::string &name) {
     } else {
         V.n = (int)V.coded.size();
     }
-    if (V.codec == Codec::ffv1) {
-        ffv1::Record rec;
-        char why[200];
-        if (ffv1::parse_record(V.extradata.data(), (int64_t)V.extradata.size(), V.rows, V.cols, rec, nullptr, nullptr, why, sizeof why))
-            fail(std::string("FFV1 configuration record: ") + why);
-        V.keyframe.resize(V.coded.size());
-        for (size_t i = 0; i < V.coded.size(); ++i) {  // the first two bytes of each chunk hold its keyframe bit
-            uint8_t d[2] = {0, 0};
-            const uint32_t len = std::min<uint32_t>(V.coded[i].second, 2);
-            if (!file.seek(V.coded[i].first) || !rd(d, len)) fail("truncated frame");
-            V.keyframe[i] = (uint8_t)ffv1::keyframe_bit(d, len);
-        }
-        if (!V.keyframe.empty() && !V.keyframe[0])
-            throw std::runtime_error("Video file " + name + ", frame 0: the first FFV1 frame is not a keyframe");
-    } else {
-        V.extradata.clear();
-    }
-    if (V.codec == Codec::png && !V.coded.empty()) {  // the size is frame 0's (IHDR); read_frames checks every other frame against it
-        uint8_t d[45];
-        const uint32_t len = std::min<uint32_t>(V.coded[0].second, sizeof d);
-        V.rows = V.cols = 0;
-        if (!file.seek(V.coded[0].first) || !rd(d, len)) fail("truncated frame");
-        check_png_frame(d, V.coded[0].second < sizeof d ? V.coded[0].second : sizeof d, V.rows, V.cols, "Video file " + name + ", frame 0");
-    }
-    if (V.n == 0) fail("no video frames found");
+    finish_index(V, file);
     return V;
 }
 
@@ -276,8 +290,23 @@ inline Index index_lmv(const std::string &name) {
     return V;
 }
 
-// An AVI file, or else the LMV1 container.
-inline Index index_video(const std::string &name) { return is_avi(name) ? index_avi(name) : index_lmv(name); }
+// Matroska and QuickTime / MP4 (lm_containers.hpp)
+inline bool is_mkv(const std::string &name);
+inline bool is_mov(const std::string &name);
+inline Index index_mkv(const std::string &name);
+inline Index index_mov(const std::string &name);
+
+// The container is chosen by the file's signature, not its extension: AVI, Matroska, QuickTime / MP4, LMV1.
+inline Index index_video(const std::string &name) {
+    if (is_avi(name)) return index_avi(name);
+    if (is_mkv(name)) return index_mkv(name);
+    if (is_mov(name)) return index_mov(name);
+    const std::vector<uint8_t> h = slurp(name, 4);
+    if (h.size() < 4 || std::memcmp(h.data(), "LMV1", 4))
+        throw std::runtime_error("Video file " + name +
+                                 ": unrecognised container; the videos read here are AVI, Matroska (.mkv), QuickTime / MP4 (.mov, .mp4) and LMV1");
+    return index_lmv(name);
+}
 
 // Frames [first, first + n) of an indexed video.  Uncompressed: channel 0 of each frame, [n][rows][cols]; coded: the frame
 // chunks back to back, with offsets relative to the first of them (PNG frames are checked here against frame 0's size).
@@ -315,7 +344,7 @@ inline Video read_frames(const Index &ix, int first, int n, const Dest &dest = n
                         if (ix.grey) std::memcpy(dst, src, (size_t)V.cols);
                         else for (int x = 0; x < V.cols; ++x) dst[x] = ix.palette_b[src[x]];
                     } else {
-                        for (int x = 0; x < V.cols; ++x) dst[x] = src[(size_t)x * ix.bpp];  // B of BGR(A): channel 0
+                        for (int x = 0; x < V.cols; ++x) dst[x] = src[(size_t)x * ix.bpp + ix.channel0];  // B of BGR(A): channel 0
                     }
                 }
         }
@@ -470,3 +499,5 @@ inline Image read_png_gray(const std::string &name) {
 }
 
 }  // namespace lmmedia
+
+#include "lm_containers.hpp"

@@ -101,11 +101,12 @@ int lmh_read_avi(const char *path, int32_t *dims, uint8_t *out, char *msg, int m
         return 1;
     }
 }
-// PNG-coded AVI: dims = {n, rows, cols, payload bytes}; with payload / offsets NULL only the dimensions are returned,
+// PNG-coded video (any container index_video reads): dims = {n, rows, cols, payload bytes}; with payload / offsets NULL only the dimensions are returned,
 // otherwise payload receives the frame chunks and offsets[n + 1] their bounds.  0 ok, 1 error (msg filled)
 int lmh_read_avi_png(const char *path, int64_t *dims, uint8_t *payload, int64_t *offsets, char *msg, int msg_cap) {
     try {
-        const lmmedia::Video V = lmmedia::read_avi(path);
+        const lmmedia::Index ix = lmmedia::index_video(path);
+        const lmmedia::Video V = lmmedia::read_frames(ix, 0, ix.n);
         if (V.codec != lmmedia::Codec::png) throw std::runtime_error(std::string("Video file ") + path + ": not a PNG-coded stream");
         dims[0] = V.n;
         dims[1] = V.rows;
@@ -119,11 +120,12 @@ int lmh_read_avi_png(const char *path, int64_t *dims, uint8_t *payload, int64_t 
         return 1;
     }
 }
-// FFV1-coded AVI: dims = {n, rows, cols, payload bytes, extradata bytes}; with payload / offsets / extradata NULL only the
+// FFV1-coded video (any container index_video reads): dims = {n, rows, cols, payload bytes, extradata bytes}; with payload / offsets / extradata NULL only the
 // dimensions are returned.  0 ok, 1 error (msg filled)
 int lmh_read_avi_ffv1(const char *path, int64_t *dims, uint8_t *payload, int64_t *offsets, uint8_t *extradata, char *msg, int msg_cap) {
     try {
-        const lmmedia::Video V = lmmedia::read_avi(path);
+        const lmmedia::Index ix = lmmedia::index_video(path);
+        const lmmedia::Video V = lmmedia::read_frames(ix, 0, ix.n);
         if (V.codec != lmmedia::Codec::ffv1) throw std::runtime_error(std::string("Video file ") + path + ": not an FFV1-coded stream");
         dims[0] = V.n;
         dims[1] = V.rows;
@@ -139,7 +141,7 @@ int lmh_read_avi_ffv1(const char *path, int64_t *dims, uint8_t *payload, int64_t
         return 1;
     }
 }
-// Frames [first, first + count) of an AVI or LMV1 video through lmmedia::index_video + read_frames: dims = {n (whole video),
+// Frames [first, first + count) of a video (AVI, Matroska, QuickTime / MP4, LMV1) through lmmedia::index_video + read_frames: dims = {n (whole video),
 // rows, cols, codec (0 raw, 1 PNG, 2 FFV1), bytes of the range}.  out receives the pixels (raw) or the frame chunks (coded, with
 // offsets[count + 1] relative to the first); with out NULL only dims are returned.  0 ok, 1 error (msg filled)
 int lmh_read_avi_range(const char *path, int64_t first, int64_t count, int64_t *dims, uint8_t *out, int64_t *offsets, char *msg, int msg_cap) {
