@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define LM_ABI_VERSION 5  /* 5: lm_bounding_box_tm, and (backward compatible additions) lm_decode_png, lm_decode_ffv1, lm_device_alloc / lm_device_free / lm_device_copy, lm_get_info("ms_decode"), lm_get_info("device_allocs"); 4: lm_bounding_box_base, lm_mouse_box_size; 2: lm_set_option, lm_get_info, lm_debug_nms, lm_bounding_box_tm_de, lm_moving_average; 3: lm_host_alloc / lm_host_free, lm_unary_costs / lm_pairwise_costs, options streams 1..4, screen_layout, screen_priority */
+#define LM_ABI_VERSION 5  /* 5: lm_bounding_box_tm, and (backward compatible additions) lm_decode_png, lm_decode_ffv1, lm_decode_mjpeg, lm_device_alloc / lm_device_free / lm_device_copy, lm_get_info("ms_decode"), lm_get_info("device_allocs"); 4: lm_bounding_box_base, lm_mouse_box_size; 2: lm_set_option, lm_get_info, lm_debug_nms, lm_bounding_box_tm_de, lm_moving_average; 3: lm_host_alloc / lm_host_free, lm_unary_costs / lm_pairwise_costs, options streams 1..4, screen_layout, screen_priority */
 
 /* feature / view indices used in every [2] / [3] array below */
 enum { LM_PAW = 0, LM_SNOUT = 1, LM_TAIL = 2 };
@@ -321,6 +321,15 @@ int lm_decode_png(lm_ctx *ctx, const uint8_t *payload, int payload_on_device, co
  * or the first bad frame and slice.  Needs lm_configure only.  lm_get_info("ms_decode") covers it. */
 int lm_decode_ffv1(lm_ctx *ctx, const uint8_t *extradata, int64_t extradata_len, const uint8_t *payload, int payload_on_device,
                    const int64_t *offsets, int64_t n, uint8_t *frames);
+/* Motion-JPEG frames (AVI 'MJPG', Matroska V_MJPEG, QuickTime 'jpeg'): payload holds n baseline JPEG files, payload / offsets
+ * / frames as for lm_decode_png.  Each frame must be 8-bit, Huffman-coded, sequential (SOF0 / SOF1), one interleaved scan,
+ * of the configured size, grey or YCbCr with Y at 2x2 or 2x1 and an even height.  libavcodec keeps DHT and DQT tables from
+ * frame to frame; here every frame must define its own DQT, and every frame must define by DHT the same tables as frame 0
+ * of the call (tables no frame defines are the JPEG Annex K ones).  The output is channel 0 of the frame cv::VideoCapture delivers through libavcodec's decoder (its integer
+ * simple IDCT and its YCbCr -> BGR conversion), bit-exact.  Each frame's entropy-coded data decodes serially on the
+ * device, the IDCT in parallel over blocks.  LM_ERR_INVALID names the first bad frame and why.  Needs lm_configure only.
+ * lm_get_info("ms_decode") covers it. */
+int lm_decode_mjpeg(lm_ctx *ctx, const uint8_t *payload, int payload_on_device, const int64_t *offsets, int64_t n, uint8_t *frames);
 int lm_device_alloc(lm_ctx *ctx, void **ptr, size_t bytes);   /* on the context's device, for callers without a CUDA runtime */
 int lm_device_free(lm_ctx *ctx, void *ptr);
 /* Copies `bytes` between two device buffers of the context's device on its stream and returns when the copy is done (a

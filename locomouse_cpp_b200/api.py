@@ -27,7 +27,7 @@ EXPORTS = ("lm_abi_version", "lm_create", "lm_destroy", "lm_last_error", "lm_con
            "lm_set_background", "lm_set_calibration", "lm_get_geometry", "lm_detect_batch", "lm_last_timing",
            "lm_debug_fetch", "lm_set_option", "lm_get_info", "lm_debug_nms", "lm_bounding_box_tm_de", "lm_moving_average",
            "lm_host_alloc", "lm_host_free", "lm_unary_costs", "lm_pairwise_costs", "lm_bounding_box_base", "lm_mouse_box_size", "lm_bounding_box_tm",
-           "lm_decode_png", "lm_device_alloc", "lm_device_free", "lm_decode_ffv1",
+           "lm_decode_png", "lm_device_alloc", "lm_device_free", "lm_decode_ffv1", "lm_decode_mjpeg",
            "lm_device_copy")
 
 
@@ -104,6 +104,8 @@ def load_library():
     L.lm_host_free.argtypes = [vp]
     L.lm_decode_png.restype = C.c_int
     L.lm_decode_png.argtypes = [vp, vp, i32, vp, i64, vp]
+    L.lm_decode_mjpeg.restype = C.c_int
+    L.lm_decode_mjpeg.argtypes = [vp, vp, i32, vp, i64, vp]
     L.lm_decode_ffv1.restype = C.c_int
     L.lm_decode_ffv1.argtypes = [vp, vp, i64, vp, i32, vp, i64, vp]
     L.lm_device_alloc.restype = C.c_int
@@ -269,6 +271,13 @@ class Detector:
                                   dtype=np.uint8).reshape(-1)
         return self._decode(lambda ptr, on_dev, offs, n, out_ptr: self._L.lm_decode_ffv1(self._ctx, ex.ctypes.data, ex.size, ptr, on_dev,
                                                                                           offs, n, out_ptr),
+                            payload, offsets, out)
+
+    def decode_mjpeg(self, payload, offsets, out=None):
+        """Motion-JPEG video frames (baseline JPEG files: 'MJPG' AVI chunks, Matroska V_MJPEG / QuickTime 'jpeg' samples)
+        decoded on the device, bit-exact with cv2.VideoCapture's channel 0 (libavcodec's decoder); payload, offsets and out as
+        for decode_png.  A refused or malformed frame raises ValueError naming it and the reason."""
+        return self._decode(lambda ptr, on_dev, offs, n, out_ptr: self._L.lm_decode_mjpeg(self._ctx, ptr, on_dev, offs, n, out_ptr),
                             payload, offsets, out)
 
     def _decode(self, call, payload, offsets, out):

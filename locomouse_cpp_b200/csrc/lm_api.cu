@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "ffv1_format.h"
+#include "mjpeg_format.h"
 #include "lm_internal.h"
 
 namespace {
@@ -60,12 +61,13 @@ struct lm_ctx {
     };
     // Context-lifetime buffers, by role: grow-only (grow()), kept across re-configuration until lm_destroy.  The folded
     // calibration (k_fold_calib: the map with the mirror folded in, the background seen through it, k_prep's run flags) is
-    // rebuilt when fold_dirty is set.  lm_decode_ffv1 shares the PNG staging, offset, status and header buffers; the three
+    // rebuilt when fold_dirty is set.  lm_decode_ffv1 shares the PNG staging, offset, status and header buffers, lm_decode_mjpeg
+    // the PNG scratch (its coefficients), staging, offset and status buffers; the three
     // pass-1 entry points share their scratch, as do the two cost builders.
     enum {
         BKG, CALIB, TMPL, FOLD_CALIB = TMPL + 6, FOLD_BKG, FOLD_RUN,
         PNG_SCRATCH, PNG_STAGE0, PNG_STAGE1, PNG_OFFS, PNG_STATUS, PNG_HDR, FFV1_REC, FFV1_INIT, FFV1_SOFF, FFV1_SLEN, FFV1_CHAINS,
-        FFV1_WORK0, FFV1_WORK1,
+        FFV1_WORK0, FFV1_WORK1, MJPEG_HDR,
         P1_MINMAX, P1_LUT, P1_STAGE, P1_HIST, P1_PRED, P1_DIFF, P1_BITS0, P1_BITS1, P1_CC, P1_VMAP, P1_VMASK, P1_SLOW, P1_RUNS,
         P1_LMASK, P1_DISK, P1_BBX, P1_LIMS,
         COST_CAND, COST_NCAND, COST_PRIOR, COST_OUT, COST_JC, COST_NNZ, COST_OFFS, COST_IR, COST_PR,
@@ -127,7 +129,7 @@ struct lm_ctx {
     std::vector<float> timeline;     // [sub-batch][9]: ms from the start of the last call to its stage events 0..7 and to the end of the screen kernel
     int64_t launches = 0;
     cudaEvent_t ev_png_copy[2] = {}, ev_png_done[2] = {};
-    float ms_decode = 0.f;            // decode kernels of the last lm_decode_png / lm_decode_ffv1 call
+    float ms_decode = 0.f;            // decode kernels of the last lm_decode_png / lm_decode_ffv1 / lm_decode_mjpeg call
     int last_B = 0;                   // size of the last sub-batch (for lm_debug_fetch)
     int last_slot = 0;
     int64_t last_s0 = 0;
@@ -1245,7 +1247,7 @@ int lm_get_info(const lm_ctx *ctx, const char *name, double *value) {
         *value = (double)ctx->timeline[(size_t)sub * 10 + q];
         return LM_OK;
     }
-    if (!strcmp(name, "ms_decode")) {  // device time of the decode kernels in the last lm_decode_png / lm_decode_ffv1 call
+    if (!strcmp(name, "ms_decode")) {  // device time of the decode kernels in the last lm_decode_png / lm_decode_ffv1 / lm_decode_mjpeg call
         *value = (double)ctx->ms_decode;
         return LM_OK;
     }
@@ -2048,6 +2050,102 @@ int decode_ffv1_impl(lm_ctx *ctx, const uint8_t *extradata, int64_t extradata_le
     return LM_OK;
 }
 }  // namespace
+
+// ---- lm_decode_mjpeg ---------------------------------------------------------------------------------------------------
+namespace {
+int decode_mjpeg_impl(lm_ctx *ctx, const uint8_t *payload, int on_dev, const int64_t *offsets, int64_t n, uint8_t *frames) {
+    if (!ctx->configured) return fail(ctx, LM_ERR_STATE, "lm_decode_mjpeg needs lm_configure first");
+    if (n < 0) return fail(ctx, LM_ERR_INVALID, "negative frame count");
+    ctx->ms_decode = 0.f;
+    if (n == 0) return LM_OK;
+    if (!payload || !offsets || !frames) return fail(ctx, LM_ERR_INVALID, "null argument");
+    const int rows = ctx->cfg.vid_rows, cols = ctx->cfg.vid_cols;
+    for (int64_t i = 0; i < n; ++i)
+        if (offsets[i] < 0 || offsets[i + 1] < offsets[i]) return fail(ctx, LM_ERR_INVALID, "frame %lld: offsets must not decrease", (long long)i);
+    if (rows > 65535 || cols > 65535) return fail(ctx, LM_ERR_INVALID, "a JPEG frame is at most 65535 x 65535 pixels");
+    cudaStream_t st = ctx->stream, cp = ctx->copy_stream;
+    auto &B = ctx->buf;
+    using L = lm_ctx;
+    if (int rc = grow(ctx, B[L::PNG_OFFS], (size_t)(n + 1) * sizeof(int64_t))) return rc;
+    if (int rc = grow(ctx, B[L::PNG_STATUS], (size_t)(n + 1) * sizeof(int32_t))) return rc;  // + frame 0's DHT tables
+    int64_t *d_offs = reinterpret_cast<int64_t *>(B[L::PNG_OFFS].p);
+    int32_t *d_status = reinterpret_cast<int32_t *>(B[L::PNG_STATUS].p);
+    CK(cudaMemcpyAsync(d_offs, offsets, (size_t)(n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    CK(cudaMemsetAsync(d_status, 0xff, (size_t)n * sizeof(int32_t), st));  // -1: not decoded
+
+    // Pieces of consecutive frames share the coefficient scratch (the widest layout's blocks per frame) and, from the host,
+    // one of two staging buffers: the copy of piece k + 1 (copy stream) overlaps the decode of piece k.
+    const size_t slot = (size_t)mjpeg::max_blocks(rows, cols) * 64 * sizeof(int16_t);
+    const size_t scratch_budget = (size_t)4 << 30, stage_budget = (size_t)2 << 30;
+    const int64_t max_piece = std::max<int64_t>(1, std::min<int64_t>(on_dev ? 8192 : std::max<int64_t>(1024, (n + 3) / 4), scratch_budget / slot));
+    struct Piece {
+        int64_t s, e;
+    };
+    std::vector<Piece> pieces;
+    size_t stage_need = 0;
+    int64_t piece_max = 0;
+    for (int64_t s = 0; s < n;) {
+        int64_t e = s + 1;
+        while (e < n && e - s < max_piece && (on_dev || (size_t)(offsets[e + 1] - offsets[s]) <= stage_budget)) ++e;
+        pieces.push_back({s, e});
+        stage_need = std::max(stage_need, (size_t)(offsets[e] - offsets[s]));
+        piece_max = std::max(piece_max, e - s);
+        s = e;
+    }
+    if (int rc = grow(ctx, B[L::PNG_SCRATCH], slot * (size_t)piece_max)) return rc;
+    if (int rc = grow(ctx, B[L::MJPEG_HDR], lm_mjpeg_header_bytes() * (size_t)piece_max)) return rc;
+    if (!on_dev) {
+        for (int k = 0; k < 2 && k < (int)pieces.size(); ++k)
+            if (int rc = grow(ctx, B[L::PNG_STAGE0 + k], std::max<size_t>(stage_need, 1))) return rc;
+        for (int k = 0; k < 2; ++k) {
+            if (!ctx->ev_png_copy[k]) CK(cudaEventCreateWithFlags(&ctx->ev_png_copy[k], cudaEventDisableTiming));
+            if (!ctx->ev_png_done[k]) CK(cudaEventCreateWithFlags(&ctx->ev_png_done[k], cudaEventDisableTiming));
+        }
+    }
+    struct Events {  // start / end of each piece's decode launches, for ms_decode
+        std::vector<cudaEvent_t> ev;
+        ~Events() {
+            for (cudaEvent_t e : ev) cudaEventDestroy(e);
+        }
+    } T;
+    T.ev.resize(2 * pieces.size());
+    for (auto &e : T.ev) CK(cudaEventCreate(&e));
+    for (size_t k = 0; k < pieces.size(); ++k) {
+        const Piece &P = pieces[k];
+        const uint8_t *src = payload;
+        int64_t base = 0;
+        if (!on_dev) {
+            uint8_t *stg = B[L::PNG_STAGE0 + (k & 1)].p;
+            if (k >= 2) CK(cudaStreamWaitEvent(cp, ctx->ev_png_done[k & 1], 0));  // piece k - 2 no longer reads this buffer
+            CK(cudaMemcpyAsync(stg, payload + offsets[P.s], (size_t)(offsets[P.e] - offsets[P.s]), cudaMemcpyHostToDevice, cp));
+            CK(cudaEventRecord(ctx->ev_png_copy[k & 1], cp));
+            CK(cudaStreamWaitEvent(st, ctx->ev_png_copy[k & 1], 0));
+            src = stg;
+            base = offsets[P.s];
+        }
+        CK(cudaEventRecord(T.ev[2 * k], st));
+        if (lm_launch_mjpeg_decode(src, d_offs + P.s, base, (int)(P.e - P.s), rows, cols, B[L::MJPEG_HDR].p, B[L::PNG_SCRATCH].as<int16_t>(),
+                                   d_status + P.s, d_status + n, k == 0, frames + P.s * (int64_t)rows * cols, st) < 0)
+            return fail(ctx, LM_ERR_RUNTIME, "Motion-JPEG decode launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        CK(cudaEventRecord(T.ev[2 * k + 1], st));
+        if (!on_dev) CK(cudaEventRecord(ctx->ev_png_done[k & 1], st));
+    }
+    std::vector<int32_t> status((size_t)n);
+    CK(cudaMemcpyAsync(status.data(), d_status, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    for (size_t k = 0; k < pieces.size(); ++k) {
+        float t = 0.f;
+        if (cudaEventElapsedTime(&t, T.ev[2 * k], T.ev[2 * k + 1]) == cudaSuccess) ctx->ms_decode += t;
+    }
+    for (int64_t i = 0; i < n; ++i)
+        if (status[i] != mjpeg::LM_MJPEG_OK) return fail(ctx, LM_ERR_INVALID, "frame %lld: %s", (long long)i, mjpeg::status_text(status[i]));
+    return LM_OK;
+}
+}  // namespace
+
+int lm_decode_mjpeg(lm_ctx *ctx, const uint8_t *payload, int payload_on_device, const int64_t *offsets, int64_t n, uint8_t *frames) {
+    return entry(ctx, [&] { return decode_mjpeg_impl(ctx, payload, payload_on_device, offsets, n, frames); });
+}
 
 int lm_decode_ffv1(lm_ctx *ctx, const uint8_t *extradata, int64_t extradata_len, const uint8_t *payload, int payload_on_device,
                    const int64_t *offsets, int64_t n, uint8_t *frames) {

@@ -238,6 +238,16 @@ int lm_launch_ffv1_decode(const ffv1::Record *rec, int ac, const uint8_t *initia
                           const int32_t *slen, int32_t *status, uint8_t *out, int rows, int cols, const LmFfv1Chain *chains, int nchains,
                           uint8_t *work, int64_t work_bytes, int work_in_smem, cudaStream_t s);
 
+// Motion-JPEG frame decode (k_mjpeg.cu, format in mjpeg_format.h).  Frame j of the launch is payload[offs[j] - base,
+// offs[j + 1] - base); its header goes to hdr + j * lm_mjpeg_header_bytes(), its coefficients to coef + j *
+// mjpeg::max_blocks(rows, cols) * 64, its pixels to out + j * rows * cols, its LM_MJPEG_* code to status[j].  *dht0 holds the
+// Huffman tables the call's frame 0 defines (written by the launch with first_piece set), which every frame must match.
+// A CTA of the entropy kernel takes 8 frames (4 kB of lookahead tables each), so several CTAs share an SM.
+constexpr int LM_MJPEG_FRAMES_PER_CTA = 8;
+size_t lm_mjpeg_header_bytes();
+int lm_launch_mjpeg_decode(const uint8_t *payload, const int64_t *offs, int64_t base, int n, int rows, int cols, uint8_t *hdr, int16_t *coef,
+                           int32_t *status, int32_t *dht0, int first_piece, uint8_t *out, cudaStream_t s);
+
 // pick the padded kernel-row width the correlation kernel is instantiated for (>= kw), or -1
 int lm_corr_kwp(int kw);
 // dynamic shared memory the correlation kernel needs for a view/template (for capability checks)

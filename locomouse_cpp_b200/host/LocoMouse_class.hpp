@@ -96,7 +96,7 @@ struct LocoMouse_Media {
     std::vector<uint8_t> bkg;           // rows x cols
     // loadVideo + loadBackground (LocoMouse_class.cpp:367-417): the video's index and its first window (the whole video when
     // it fits in max_resident_bytes); throws std::runtime_error as the reference's constructor does
-    void load(const std::string &video_file, const std::string &bkg_file, size_t max_resident_bytes, int batch_frames);
+    void load(const std::string &video_file, const std::string &bkg_file, size_t max_resident_bytes, int batch_frames, bool decode_mjpeg = false);
     void read_window(int k, PinnedArray<uint8_t> &to, std::vector<int64_t> &to_offsets) const;
 };
 
@@ -163,6 +163,7 @@ public:
     // page-locked bytes of frames held at a time: a longer video is read, decoded and tracked in windows of this many bytes
     // (a multiple of batch_frames frames), each read on a reader thread while the device works on the one before
     int64_t max_resident_bytes = (int64_t)8 << 30;
+    int decode_mjpeg = 0;  // 1: Motion-JPEG video is decoded (bit-exact with libavcodec's decoder, lm_decode_mjpeg), 0: refused
     int fma_mode = 1;
     int cand_cap = 64, det_cap = 8192, match_cap = 256;
 

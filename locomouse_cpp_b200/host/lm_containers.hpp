@@ -137,7 +137,7 @@ inline bool is_mkv(const std::string &name) {
     return h.size() >= 4 && h[0] == 0x1A && h[1] == 0x45 && h[2] == 0xDF && h[3] == 0xA3;
 }
 
-inline Index index_mkv(const std::string &name) {
+inline Index index_mkv(const std::string &name, const Options &opt) {
     enum : uint32_t {
         EBML = 0x1A45DFA3, DocType = 0x4282, Segment = 0x18538067, Info = 0x1549A966, TimecodeScale = 0x2AD7B1, Duration = 0x4489,
         Tracks = 0x1654AE6B, TrackEntry = 0xAE, TrackNumber = 0xD7, TrackType = 0x83, CodecID = 0x86, CodecPrivate = 0x63A2,
@@ -285,6 +285,8 @@ inline Index index_mkv(const std::string &name) {
     if (vt->codec == "V_FFV1") {
         V.codec = Codec::ffv1;
         V.extradata = vt->priv;
+    } else if (vt->codec == "V_MJPEG" && opt.decode_mjpeg) {
+        V.codec = Codec::mjpeg;
     } else if (vt->codec == "V_MS/VFW/FOURCC") {
         // a BITMAPINFOHEADER, as in an AVI's 'strf'
         const std::vector<uint8_t> &b = vt->priv;
@@ -298,6 +300,8 @@ inline Index index_mkv(const std::string &name) {
         } else if (fourcc == cc("FFV1")) {
             V.codec = Codec::ffv1;
             V.extradata.assign(b.begin() + 40, b.end());
+        } else if (opt.decode_mjpeg && (fourcc == cc("MJPG") || fourcc == cc("mjpg"))) {
+            V.codec = Codec::mjpeg;
         } else if ((fourcc == cc("Y800") || fourcc == cc("GREY") || fourcc == cc("Y8  ")) && bits == 8) {
             raw = true;
         } else if (fourcc == 0 && (bits == 24 || bits == 32)) {  // BI_RGB: BGR(A), rows top-down as libavformat reads them from Matroska (no AVI bottom-up flip)
@@ -386,7 +390,7 @@ void boxes(Span s, const Fail &fail, const Fn &fn) {
 }
 }  // namespace detail
 
-inline Index index_mov(const std::string &name) {
+inline Index index_mov(const std::string &name, const Options &opt) {
     using detail::Span;
     detail::File file(name);
     auto fail = [&](const std::string &why) -> void { throw std::runtime_error("Video file " + name + ": " + why); };
@@ -516,6 +520,8 @@ inline Index index_mov(const std::string &name) {
     bool raw = false;
     if (type == "png " || type == "MPNG") {
         V.codec = Codec::png;
+    } else if (type == "jpeg" && opt.decode_mjpeg) {
+        V.codec = Codec::mjpeg;
     } else if (type == "FFV1") {
         V.codec = Codec::ffv1;
         bool glbl = false;
@@ -555,8 +561,9 @@ inline Index index_mov(const std::string &name) {
             if (flags & 0x20) p += 2;
             if (descr(4) && p < b.n) oti = b.d[p];
         });
-        if (oti != 0x6D) outside("'mp4v' with object type " + std::to_string(oti) + " (not PNG)");
-        V.codec = Codec::png;
+        if (oti == 0x6C && opt.decode_mjpeg) V.codec = Codec::mjpeg;  // libavformat: 0x6C is MJPEG
+        else if (oti != 0x6D) outside("'mp4v' with object type " + std::to_string(oti) + " (not PNG)");
+        else V.codec = Codec::png;
     } else if (type == "raw ") {
         outside("'raw ' with depth " + std::to_string(depth));
     } else {

@@ -5,7 +5,8 @@
 // 'GREY' / 'Y8  ', what cv2.VideoWriter(fourcc = 0, isColor = False) writes), BI_RGB 8-bit with a palette, BI_RGB 24- / 32-bit
 // (channel 0 = blue, as extractChannel takes it).  PNG-coded streams ('MPNG' / 'png ', lossless, what cv2.VideoWriter writes
 // with those fourccs) are not decoded here: their frame chunks -- each a complete PNG file -- are returned as one payload with
-// offsets, for lm_decode_png to decode on the device.  FFV1-coded streams ('FFV1', lossless, version 3 as libavcodec writes
+// offsets, for lm_decode_png to decode on the device.  Motion-JPEG streams are returned the same way for lm_decode_mjpeg when
+// the caller opts in (Options::decode_mjpeg); otherwise they are refused like every other lossy codec.  FFV1-coded streams ('FFV1', lossless, version 3 as libavcodec writes
 // it) are returned the same way, with the configuration record from 'strf' as extradata, for lm_decode_ffv1; the record is
 // checked here (ffv1_format.h) and so is every frame's keyframe bit.  Other compressed or YUV-planar streams need a decoder
 // that is outside this library: they are refused with a message that says so.  The same frames in Matroska and QuickTime / MP4
@@ -29,6 +30,7 @@
 #include <vector>
 
 #include "../csrc/ffv1_format.h"
+#include "../csrc/mjpeg_format.h"
 
 namespace lmmedia {
 
@@ -62,7 +64,13 @@ inline bool is_png(const std::string &name) {
 // into memory the upload runs from at the PCIe rate).  Without one they go to Video::frames / a malloc'ed Video::payload.
 using Dest = std::function<uint8_t *(size_t bytes)>;
 
-enum class Codec { raw, png, ffv1 };
+enum class Codec { raw, png, ffv1, mjpeg };
+
+// What the index functions accept beyond the lossless codecs.  Motion-JPEG is decoded bit-exactly with the libavcodec
+// decoder OpenCV calls (mjpeg_format.h), so a caller whose reference reads it through another decoder turns it on knowingly.
+struct Options {
+    bool decode_mjpeg = false;  // Motion-JPEG (AVI 'MJPG', Matroska V_MJPEG, QuickTime 'jpeg', MP4 object type 0x6C) instead of a refusal
+};
 
 struct Video {
     int n = 0, rows = 0, cols = 0;
@@ -92,6 +100,22 @@ inline void check_png_frame(const uint8_t *d, size_t len, int &rows, int &cols, 
         fail(std::to_string(w) + " x " + std::to_string(h) + " pixels, frame 0 has " + std::to_string(cols) + " x " + std::to_string(rows));
 }
 
+// Header segments of one Motion-JPEG frame up to its SOS: what lm_decode_mjpeg decodes.  Its SOF size must be the video's
+// rows x cols (rows = 0: any, and it becomes the video's), and its DHT must define the tables the video's first frame
+// defines (dht < 0: any, and its set becomes the video's), because libavcodec carries tables from one frame to the next.
+inline void check_mjpeg_frame(const uint8_t *d, size_t len, int &rows, int &cols, int &dht, const std::string &where) {
+    std::unique_ptr<mjpeg::Header> h(new mjpeg::Header);
+    const int st = mjpeg::parse(d, (int64_t)len, 0, 0, *h);
+    if (st != mjpeg::LM_MJPEG_OK) throw std::runtime_error(where + ": " + mjpeg::status_text(st));
+    if (rows && (h->rows != rows || h->cols != cols))
+        throw std::runtime_error(where + ": " + mjpeg::status_text(mjpeg::LM_MJPEG_SIZE) + ": the frame is " + std::to_string(h->cols) + " x " +
+                                 std::to_string(h->rows) + " pixels (SOF), the video " + std::to_string(cols) + " x " + std::to_string(rows));
+    if (dht >= 0 && h->dht_mask != dht) throw std::runtime_error(where + ": " + mjpeg::status_text(mjpeg::LM_MJPEG_DHT_CHANGE));
+    rows = h->rows;
+    cols = h->cols;
+    dht = h->dht_mask;
+}
+
 // Where every frame of a video lies in its file: the result of one walk over the chunk headers (index_avi, or index_lmv for
 // the LMV1 container of lm_files.hpp), from which read_frames reads any range of frames.  Every chunk is checked against the
 // file size here, so a truncated chunk is refused before any frame is used, wherever it lies.
@@ -112,6 +136,7 @@ struct Index {
     // coded frames: file offset and size of every frame chunk; FFV1: every frame's keyframe bit and the configuration record
     std::vector<std::pair<int64_t, uint32_t>> coded;
     std::vector<uint8_t> keyframe, extradata;
+    int mjpeg_dht = -1;  // Motion-JPEG: the tables frame 0's DHT defines (mjpeg::Header::dht_mask), which every frame must match
 };
 
 namespace detail {
@@ -162,6 +187,15 @@ inline void finish_index(Index &V, detail::File &file) {
         if (!file.seek(V.coded[0].first) || !file.read(d, len)) fail("truncated frame");
         check_png_frame(d, V.coded[0].second < sizeof d ? V.coded[0].second : sizeof d, V.rows, V.cols, "Video file " + V.name + ", frame 0");
     }
+    if (V.codec == Codec::mjpeg && !V.coded.empty()) {
+        // Frame 0's SOF must give the container's frame size (where the container states one): libavcodec weaves a frame
+        // whose SOF height is below 3/4 of the container's as an interlaced field pair, and this decoder does not.  read_frames
+        // checks every other frame against the size and frame 0's DHT tables.
+        std::vector<uint8_t> d(V.coded[0].second);
+        if (V.rows <= 0 || V.cols <= 0) V.rows = V.cols = 0;
+        if (!file.seek(V.coded[0].first) || !file.read(d.data(), d.size())) fail("truncated frame");
+        check_mjpeg_frame(d.data(), d.size(), V.rows, V.cols, V.mjpeg_dht, "Video file " + V.name + ", frame 0");
+    }
     if (V.n == 0) fail("no video frames found");
 }
 
@@ -171,7 +205,7 @@ inline const char *outside_this_library() {
 }
 
 // The walk over stream 0's frame chunks ('00db' / '00dc') in file order, with the format and record checks.
-inline Index index_avi(const std::string &name) {
+inline Index index_avi(const std::string &name, const Options &opt = {}) {
     detail::File file(name);
     FILE *f = file.f;
     auto fail = [&](const std::string &why) -> void { throw std::runtime_error("Video file " + name + ": " + why); };
@@ -234,9 +268,10 @@ inline Index index_avi(const std::string &name) {
         const bool grey = fourcc == cc("Y800") || fourcc == cc("GREY") || fourcc == cc("Y8  ") || fourcc == cc("Y8\0\0");
         const bool rgb = fourcc == 0 || fourcc == cc("DIB ") || fourcc == cc("RGB ") || fourcc == cc("RAW ");
         const bool png = fourcc == cc("MPNG") || fourcc == cc("png ");
-        if (png || fourcc == cc("FFV1")) {
+        const bool mjpg = opt.decode_mjpeg && (fourcc == cc("MJPG") || fourcc == cc("mjpg"));
+        if (png || mjpg || fourcc == cc("FFV1")) {
             if (size == 0) continue;
-            V.codec = png ? Codec::png : Codec::ffv1;
+            V.codec = png ? Codec::png : mjpg ? Codec::mjpeg : Codec::ffv1;
             const off_t at = ftello(f);
             V.coded.emplace_back((int64_t)at, size);
             if (!skip((uint64_t)size + (size & 1))) fail("truncated frame");
@@ -293,14 +328,14 @@ inline Index index_lmv(const std::string &name) {
 // Matroska and QuickTime / MP4 (lm_containers.hpp)
 inline bool is_mkv(const std::string &name);
 inline bool is_mov(const std::string &name);
-inline Index index_mkv(const std::string &name);
-inline Index index_mov(const std::string &name);
+inline Index index_mkv(const std::string &name, const Options &opt = {});
+inline Index index_mov(const std::string &name, const Options &opt = {});
 
 // The container is chosen by the file's signature, not its extension: AVI, Matroska, QuickTime / MP4, LMV1.
-inline Index index_video(const std::string &name) {
-    if (is_avi(name)) return index_avi(name);
-    if (is_mkv(name)) return index_mkv(name);
-    if (is_mov(name)) return index_mov(name);
+inline Index index_video(const std::string &name, const Options &opt = {}) {
+    if (is_avi(name)) return index_avi(name, opt);
+    if (is_mkv(name)) return index_mkv(name, opt);
+    if (is_mov(name)) return index_mov(name, opt);
     const std::vector<uint8_t> h = slurp(name, 4);
     if (h.size() < 4 || std::memcmp(h.data(), "LMV1", 4))
         throw std::runtime_error("Video file " + name +
@@ -358,11 +393,13 @@ inline Video read_frames(const Index &ix, int first, int n, const Dest &dest = n
     if (dest) V.payload = std::shared_ptr<uint8_t>(buf, [](uint8_t *) {});  // owned by the caller
     else V.payload = std::shared_ptr<uint8_t>(buf, [](uint8_t *q) { std::free(q); });
     V.offsets.push_back(0);
+    int dht = ix.mjpeg_dht;
     for (int i = 0; i < n; ++i) {
         const auto &c = ix.coded[(size_t)(first + i)];
         uint8_t *d = buf + V.offsets.back();
         if (!file.seek(c.first) || !file.read(d, c.second)) fail("truncated frame");
         if (ix.codec == Codec::png) check_png_frame(d, c.second, V.rows, V.cols, "Video file " + ix.name + ", frame " + std::to_string(first + i));
+        if (ix.codec == Codec::mjpeg) check_mjpeg_frame(d, c.second, V.rows, V.cols, dht, "Video file " + ix.name + ", frame " + std::to_string(first + i));
         V.offsets.push_back(V.offsets.back() + c.second);
     }
     V.n = n;

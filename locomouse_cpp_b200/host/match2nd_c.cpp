@@ -234,6 +234,80 @@ int lmh_decode_ffv1(const uint8_t *extradata, int64_t extradata_len, const uint8
         }
     return 0;
 }
+// Motion-JPEG video (any container index_video reads) with decode_mjpeg on: dims = {n, rows, cols, payload bytes}; with
+// payload / offsets NULL only the dimensions are returned.  0 ok, 1 error (msg filled)
+int lmh_read_video_mjpeg(const char *path, int64_t *dims, uint8_t *payload, int64_t *offsets, char *msg, int msg_cap) {
+    try {
+        lmmedia::Options opt;
+        opt.decode_mjpeg = true;
+        const lmmedia::Index ix = lmmedia::index_video(path, opt);
+        const lmmedia::Video V = lmmedia::read_frames(ix, 0, ix.n);
+        if (V.codec != lmmedia::Codec::mjpeg) throw std::runtime_error(std::string("Video file ") + path + ": not a Motion-JPEG stream");
+        dims[0] = V.n;
+        dims[1] = V.rows;
+        dims[2] = V.cols;
+        dims[3] = V.offsets.back();
+        if (payload) std::memcpy(payload, V.payload.get(), (size_t)V.offsets.back());
+        if (offsets) std::memcpy(offsets, V.offsets.data(), V.offsets.size() * sizeof(int64_t));
+        return 0;
+    } catch (const std::exception &e) {
+        if (msg && msg_cap > 0) std::snprintf(msg, (size_t)msg_cap, "%s", e.what());
+        return 1;
+    }
+}
+// lmh_read_avi_range with decode_mjpeg on (codec 3 = Motion-JPEG)
+int lmh_read_avi_range_mjpeg(const char *path, int64_t first, int64_t count, int64_t *dims, uint8_t *out, int64_t *offsets, char *msg,
+                             int msg_cap) {
+    try {
+        lmmedia::Options opt;
+        opt.decode_mjpeg = true;
+        const lmmedia::Index ix = lmmedia::index_video(path, opt);
+        dims[0] = ix.n;
+        dims[1] = ix.rows;
+        dims[2] = ix.cols;
+        dims[3] = (int64_t)ix.codec;
+        dims[4] = 0;
+        if (count <= 0) return 0;
+        const lmmedia::Video V = lmmedia::read_frames(ix, (int)first, (int)count);
+        dims[4] = V.codec == lmmedia::Codec::raw ? (int64_t)V.frames.size() : V.offsets.back();
+        if (out) std::memcpy(out, V.codec == lmmedia::Codec::raw ? V.frames.data() : V.payload.get(), (size_t)dims[4]);
+        if (offsets && V.codec != lmmedia::Codec::raw) std::memcpy(offsets, V.offsets.data(), V.offsets.size() * sizeof(int64_t));
+        return 0;
+    } catch (const std::exception &e) {
+        if (msg && msg_cap > 0) std::snprintf(msg, (size_t)msg_cap, "%s", e.what());
+        return 1;
+    }
+}
+// mjpeg_format.h run serially on the CPU: the header parse, entropy decode and IDCT that k_mjpeg.cu runs on the device, for
+// the CPU tests.  out: [n][rows][cols].  0 ok, 1 error (msg names the first bad frame and why)
+int lmh_decode_mjpeg(const uint8_t *payload, const int64_t *offsets, int64_t n, int rows, int cols, uint8_t *out, char *msg, int msg_cap) {
+    std::unique_ptr<mjpeg::Header> hold(new mjpeg::Header);
+    mjpeg::Header &h = *hold;
+    std::vector<uint16_t> fast((size_t)4 << mjpeg::FAST_BITS);
+    std::vector<int16_t> coef;
+    int dht0 = -1;  // the tables frame 0's DHT defines: every frame must define the same (libavcodec carries them over)
+    for (int64_t f = 0; f < n; ++f) {
+        const uint8_t *fr = payload + offsets[f];
+        const int64_t len = offsets[f + 1] - offsets[f];
+        int st = mjpeg::parse(fr, len, rows, cols, h);
+        for (int t = 0; t < 4 && st == mjpeg::LM_MJPEG_OK; ++t)
+            if (!mjpeg::build_fast(h.tab[t], fast.data() + ((size_t)t << mjpeg::FAST_BITS))) st = mjpeg::LM_MJPEG_TABLE;
+        if (st == mjpeg::LM_MJPEG_OK && f == 0) dht0 = h.dht_mask;
+        if (st == mjpeg::LM_MJPEG_OK && h.dht_mask != dht0) st = mjpeg::LM_MJPEG_DHT_CHANGE;
+        if (st == mjpeg::LM_MJPEG_OK) {
+            coef.assign((size_t)h.blocks() * 64, 0);
+            st = mjpeg::decode_scan(h, fr + h.ecs, fr + len, fast.data(),
+                                    [&](int64_t b, const int16_t *blk) { std::memcpy(&coef[(size_t)b * 64], blk, 64 * sizeof(int16_t)); });
+        }
+        if (st != mjpeg::LM_MJPEG_OK) {
+            std::snprintf(msg, (size_t)msg_cap, "frame %lld: %s", (long long)f, mjpeg::status_text(st));
+            return 1;
+        }
+        for (int by = 0; by < h.y_blocks_y(); ++by)
+            for (int bx = 0; bx < h.y_blocks_x(); ++bx) mjpeg::put_y_block(h, coef.data(), by, bx, out + f * (int64_t)rows * cols);
+    }
+    return 0;
+}
 int lmh_read_png(const char *path, int32_t *dims, uint8_t *out, char *msg, int msg_cap) {
     try {
         const lmmedia::Image I = lmmedia::read_png_gray(path);
