@@ -347,7 +347,19 @@ int lm_last_timing(const lm_ctx *ctx, float ms[7], int64_t *launches);
 /* Copies an intermediate of the LAST sub-batch back to the host for parity debugging.
  * what: 0 = pre-processed bottom window (u8), 1 = side window (u8), 2 = bottom tail mask (u8 0/255,
  * bb_h_bottom x tail_w), 3 = per-frame min/max (2 x int32). frame is relative to the last call.
+ * Items of the last pass-1 call (lm_bounding_box_tm / _base / _tm_de; backward-compatible additions, they need no
+ * lm_detect_batch): frame is the index within that call and must lie in its last chunk (256 frames for TM and the base
+ * class, 1024 for TM_DE), LM_ERR_INVALID otherwise.  dims = rows, 32-bit words per row, width in pixels, method (LM_P1_*);
+ * the item is rows x words int32 / uint32.
+ *   4 = bit image A: TM the filtered image (filter2D output >= 1), base the binary image (normalised value >= 3) of the
+ *       whole calibrated image;
+ *   5 = bit image B: TM the opened image (bwAreaOpen output), base the median image (median >= 3);
+ *       (bit x of a row is word x / 32, bit x % 32; bits at and beyond `width` are 0; not available for TM_DE)
+ *   6 = the per-frame sums, one row: TM the CV_32S column sums of the filled image [side_w]; base Row_side [side_w] |
+ *       Row_bottom [bottom_w] | Col_side [side_h] | Col_bottom [bottom_h] (255 per pixel of the view's largest
+ *       component); TM_DE the per-column count of thresholded pixels inside the bands [side_w].
  * Returns the number of bytes written or a negative lm_status. */
+enum { LM_P1_TM_DE = 1, LM_P1_BASE = 2, LM_P1_TM = 3 };
 int64_t lm_debug_fetch(lm_ctx *ctx, int what, int64_t frame, void *dst, int64_t dst_bytes,
                        int32_t dims[4]);
 

@@ -378,17 +378,28 @@ class Detector:
         return dict(zip(self.STAGES, map(float, ms))), int(n.value)
 
     def debug_fetch(self, what: int, frame: int):
+        """An intermediate and its dims (include/locomouse_b200.h, lm_debug_fetch).  0 / 1 / 2: a u8 image; 3: min / max;
+        4 / 5 (after a bounding_box_tm / _base call; frame = index within that call): the bit image unpacked to a 0 / 1 uint8
+        [rows, width]; 6: the frame's int32 sums."""
         dims = np.zeros(4, np.int32)
         need = self._L.lm_debug_fetch(self._ctx, what, frame, None, 0, dims.ctypes.data)
-        nbytes = {0: int(dims[0]) * int(dims[1]), 1: int(dims[0]) * int(dims[1]), 2: int(dims[0]) * int(dims[1]), 3: 8}[what]
-        del need
-        buf = np.zeros(nbytes, np.uint8)
+        if need < 0 and what in (4, 5, 6) and need != LM_ERR_INVALID:
+            self._check(int(need))   # no pass-1 call yet
+        words = what in (4, 5, 6)
+        nbytes = 8 if what == 3 else int(dims[0]) * int(dims[1]) * (4 if words else 1)
+        buf = np.zeros(max(nbytes, 1), np.uint8)
         got = self._L.lm_debug_fetch(self._ctx, what, frame, buf.ctypes.data, nbytes, dims.ctypes.data)
         if got < 0:
             self._check(int(got))
         if what == 3:
             mm = buf.view(np.int32)
             return np.array([255 - mm[0], mm[1]], np.int32), dims
+        if what == 6:
+            return buf[:nbytes].view(np.int32).copy(), dims
+        if words:
+            w = buf[:nbytes].view("<u4").reshape(int(dims[0]), int(dims[1]))
+            bits = np.unpackbits(w.view(np.uint8), axis=1, bitorder="little")
+            return bits[:, :int(dims[2])].copy(), dims
         return buf.reshape(int(dims[0]), int(dims[1])), dims
 
     def close(self):

@@ -13,7 +13,7 @@
 //   k_bb_pred   one thread replays imadjust_default's float cumulative scan (order matters), all threads then build
 //               pred[d] = ( imadjust_default( normalise(d) ) > threshold )
 //   k_bb_cols   column sums of pred over the rows / columns that survive the zeroed bands (streamed from the kept
-//               differences), first / last, bb_x
+//               differences), stored per frame (lm_debug_fetch item 6), first / last, bb_x
 // The whole-video moving average that follows is sequential and stays on the host (lm_moving_average).
 #include <cstdlib>
 
@@ -36,6 +36,7 @@ struct BBoxDev {
     uint8_t *diff;        // [B][side_h * side_w] raw difference sat(F - BKG) of every side-view pixel, written by k_bb_hist (may be null)
     double *bb_x;         // [B]
     int32_t *lims;        // [B][2]
+    int32_t *sums;        // [B][side_w] column sums (null: not kept)
 };
 
 __global__ void __launch_bounds__(256) k_bb_hist(const __grid_constant__ BBoxDev P) {
@@ -287,6 +288,7 @@ __global__ void __launch_bounds__(256) k_bb_cols(const __grid_constant__ BBoxDev
                     if (d[q] > -1000) sum += pred[d[q] < 0 ? 0 : d[q]];
             }
         }
+        if (P.sums) P.sums[(int64_t)f * P.p.side_w + x] = sum;
         if (sum >= P.p.min_count) {  // firstLastOverT: p[i] >= th
             atomicMin(&s_first, x);
             atomicMax(&s_last, x);
@@ -308,7 +310,8 @@ __global__ void __launch_bounds__(256) k_bb_cols(const __grid_constant__ BBoxDev
 
 }  // namespace
 
-static BBoxDev bbox_dev(const LmBatch &b, const lm_bb_de_params &p, uint32_t *hist, uint8_t *pred, double *bb_x, int32_t *lims, uint8_t *diff) {
+static BBoxDev bbox_dev(const LmBatch &b, const lm_bb_de_params &p, uint32_t *hist, uint8_t *pred, double *bb_x, int32_t *lims, int32_t *sums,
+                        uint8_t *diff) {
     BBoxDev P{};
     P.frames = b.frames;
     P.frame_bytes = b.frame_bytes;
@@ -327,6 +330,7 @@ static BBoxDev bbox_dev(const LmBatch &b, const lm_bb_de_params &p, uint32_t *hi
     P.diff = diff;
     P.bb_x = bb_x;
     P.lims = lims;
+    P.sums = sums;
     return P;
 }
 
@@ -339,7 +343,7 @@ int lm_launch_bbox_pred(const LmBatch &b, const lm_bb_de_params &p, uint32_t *hi
     int nl = lm_launch_minmax(b, s);
     if (nl < 0) return -1;
     launches += nl;
-    const BBoxDev P = bbox_dev(b, p, hist, pred, nullptr, nullptr, diff);
+    const BBoxDev P = bbox_dev(b, p, hist, pred, nullptr, nullptr, nullptr, diff);
     const int npx = p.side_w * p.side_h;
     int gx = (npx + 256 * 16 - 1) / (256 * 16);
     gx = gx < 1 ? 1 : (gx > 64 ? 64 : gx);
@@ -359,10 +363,10 @@ int lm_launch_bbox_pred(const LmBatch &b, const lm_bb_de_params &p, uint32_t *hi
 
 // b: frames / bkg / calib / minmax / lut / n_cols / flip / B filled in by the caller (imadjust must be 0)
 int lm_launch_bbox_tm_de(const LmBatch &b, const lm_bb_de_params &p, uint32_t *hist, uint8_t *pred, double *bb_x, int32_t *lims,
-                         cudaStream_t s, uint8_t *diff) {
+                         int32_t *sums, cudaStream_t s, uint8_t *diff) {
     int launches = lm_launch_bbox_pred(b, p, hist, pred, s, diff);
     if (launches < 0) return -1;
-    const BBoxDev P = bbox_dev(b, p, hist, pred, bb_x, lims, diff);
+    const BBoxDev P = bbox_dev(b, p, hist, pred, bb_x, lims, sums, diff);
     k_bb_cols<<<b.B, 256, 0, s>>>(P);
     launches += 1;
     return cudaGetLastError() == cudaSuccess ? launches : -1;

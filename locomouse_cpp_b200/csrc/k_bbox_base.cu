@@ -13,7 +13,8 @@
 //   k_bbb_major  median >= 3  <=>  at least (k*k+1)/2 of the zero-extended k x k window are set: window popcounts on the
 //                bit image
 //   k_bbb_cc     per (frame, view): the view's bits -> shared memory -> run-based largest component (cc_runs.cuh) ->
-//                per-column / per-row counts -> the four (first, last) pairs
+//                per-column / per-row counts -> the four sum vectors (stored per frame, lm_debug_fetch item 6) -> the four
+//                (first, last) pairs
 //   k_bbb_cc_slow  the same through the pixel union-find in global memory, for views with more runs than fit
 // The six per-frame numbers and the whole-video post-processing (computeMouseBoxSize, vecmovingaverage) are host work.
 #include <algorithm>
@@ -36,6 +37,7 @@ struct BBaseDev {
     uint32_t *bits, *major;  // [B][n_rows][wpr]
     lm_bb_base_params p;
     int32_t *lims;           // [B][4][2]: Row_side, Row_bottom, Col_side, Col_bottom
+    int32_t *sums;           // [B][lm_bbox_base_sums(p)]: the same four vectors (255 per pixel; null: not kept)
     int *need_slow;          // [B][2]
     int runcap;
     // slow path scratch: SLOW_SLOTS x (3 ints per pixel of the larger view + its u8 map and mask)
@@ -150,6 +152,13 @@ __device__ void first_last(const int *sums, int L, int scale, int th, int as_flo
     __syncthreads();
 }
 
+// the frame's Row_* (view v, L entries) or Col_* (rows entries) vector in P.sums
+__device__ __forceinline__ int32_t *base_sums(const BBaseDev &P, int f, int v, bool col) {
+    const lm_bb_base_params &p = P.p;
+    int32_t *o = P.sums + (int64_t)f * (p.side_w + p.bottom_w + p.side_h + p.bottom_h);
+    return col ? o + p.side_w + p.bottom_w + (v ? p.side_h : 0) : o + (v ? p.side_w : 0);
+}
+
 __global__ void __launch_bounds__(TAIL_THREADS) k_bbb_cc(const __grid_constant__ BBaseDev P) {
     extern __shared__ __align__(16) unsigned char raw[];
     const int f = blockIdx.x, v = blockIdx.y, tid = threadIdx.x;
@@ -191,6 +200,11 @@ __global__ void __launch_bounds__(TAIL_THREADS) k_bbb_cc(const __grid_constant__
     }
     int32_t *lim = P.lims + (int64_t)f * 8;
     // Row_* = per-column sums (scanned over min(N_COLS, view width) entries), Col_* = per-row sums; 255 per pixel
+    if (P.sums) {
+        int32_t *rs = base_sums(P, f, v, false), *cs = base_sums(P, f, v, true);
+        for (int i = tid; i < min(P.n_cols, cols); i += TAIL_THREADS) rs[i] = S.cnt[i] * 255;
+        for (int i = tid; i < rows; i += TAIL_THREADS) cs[i] = S.rowcnt[i] * 255;
+    }
     first_last(S.cnt, min(P.n_cols, cols), 255, P.p.min_pixel_visible, P.p.sums_as_float, lim + (v ? 2 : 0), s_acc);
     first_last(S.rowcnt, rows, 255, P.p.min_pixel_visible, P.p.sums_as_float, lim + (v ? 6 : 4), s_acc);
 }
@@ -227,6 +241,10 @@ __global__ void __launch_bounds__(SLOW_THREADS) k_bbb_cc_slow(const __grid_const
         for (int pass = 0; pass < 2; ++pass) {
             const int *sums = pass ? rowcnt : colcnt;
             const int Lc = pass ? rows : min(P.n_cols, cols);
+            if (P.sums) {
+                int32_t *out = base_sums(P, f, v, pass != 0);
+                for (int i = tid; i < Lc; i += SLOW_THREADS) out[i] = sums[i] * 255;
+            }
             __syncthreads();
             if (tid == 0) {
                 s_acc[0] = 0x7fffffff;
@@ -273,7 +291,7 @@ size_t lm_bbox_base_slow_ints(const lm_bb_base_params &p) {
 // bits / major: lm_bbox_base_bits_bytes each; cc: BB_SLOW_SLOTS * 3 * lm_bbox_base_slow_ints ints; vmap / vmask: BB_SLOW_SLOTS *
 // lm_bbox_base_slow_ints bytes each; need_slow: [B][2]; lims: [B][4][2].
 int lm_launch_bbox_base(const LmBatch &b, const lm_bb_base_params &p, uint32_t *bits, uint32_t *major, int32_t *cc, uint8_t *vmap, uint8_t *vmask,
-                        int *need_slow, int32_t *lims, cudaStream_t s) {
+                        int *need_slow, int32_t *lims, int32_t *sums, cudaStream_t s) {
     int launches = 0;
     if (cudaMemsetAsync(b.minmax, 0, (size_t)(b.B + 1) * 2 * sizeof(int32_t), s) != cudaSuccess) return -1;
     int nl = lm_launch_minmax(b, s);
@@ -295,6 +313,7 @@ int lm_launch_bbox_base(const LmBatch &b, const lm_bb_base_params &p, uint32_t *
     P.major = major;
     P.p = p;
     P.lims = lims;
+    P.sums = sums;
     P.need_slow = need_slow;
     P.cc = cc;
     P.vmap = vmap;

@@ -14,7 +14,7 @@
 //                 pixels are counted per distinct kernel weight (popcounts) and only sums within the rounding margin of 0.5
 //                 replay OpenCV's float adds in row-major tap order
 //   k_bbtm_fill   per frame: 4-connected labelling of the seed-valued pixels, the component of pixel (0, 0) = the flood
-//                 fill; column sums via a difference array; first / last; bb_x
+//                 fill; column sums via a difference array, stored per frame (lm_debug_fetch item 6); first / last; bb_x
 // Frames whose run count exceeds the shared-memory capacity set a flag and are redone by the same code with its run arrays
 // in global memory (k_bbtm_open / k_bbtm_fill instantiated with GLOBAL = true, one CTA per flagged frame).
 #include <algorithm>
@@ -48,6 +48,7 @@ struct BBTmDev {
     int64_t g_stride;        // runs per slot
     double *bb_x;            // [B]
     int32_t *lims;           // [B][2]
+    int32_t *sums;           // [B][W] column sums of the filled image (null: not kept)
 };
 
 __global__ void __launch_bounds__(256) k_bbtm_bin(const __grid_constant__ BBTmDev P) {
@@ -393,6 +394,7 @@ __global__ void __launch_bounds__(TAIL_THREADS) k_bbtm_fill(const __grid_constan
             for (int c = c0; c < c1; ++c) {
                 run += diff[c];
                 const int sum = (int)seed * run + 255 * (P.H - run);
+                if (P.sums) P.sums[(int64_t)f * P.W + c] = sum;
                 const float v = P.as_float ? __int_as_float(sum) : (float)sum;
                 if (v >= (float)P.min_pixel_visible) {   // firstLastOverT: p[i] >= th
                     atomicMin(&s_first, c);
@@ -426,7 +428,7 @@ size_t lm_bbox_tm_slow_runs(const lm_bb_tm_params &p) { return (size_t)p.side_h 
 // hist / pred: [B][256]; bits_a / bits_b: lm_bbox_tm_bits_bytes each; need_slow: [B][2]; g_runs: chunk capacity x
 // lm_bbox_tm_slow_runs x 14 bytes (slots: the frames of a chunk); disk: the kernel on the device.
 int lm_launch_bbox_tm(const LmBatch &b, const lm_bb_tm_params &p, const float *d_disk, uint32_t *hist, uint8_t *pred, uint32_t *bits_a,
-                      uint32_t *bits_b, int *need_slow, unsigned char *g_runs, int g_slots, uint32_t *level_mask, double *bb_x, int32_t *lims, cudaStream_t s) {
+                      uint32_t *bits_b, int *need_slow, unsigned char *g_runs, int g_slots, uint32_t *level_mask, double *bb_x, int32_t *lims, int32_t *sums, cudaStream_t s) {
     // 1. pred[d]: the front end shared with LocoMouse_TM_DE (normalisation LUT, histogram, imadjust_default, threshold)
     lm_bb_de_params q{};
     q.side_x = p.side_x;
@@ -465,6 +467,7 @@ int lm_launch_bbox_tm(const LmBatch &b, const lm_bb_tm_params &p, const float *d
     P.need_slow = need_slow;
     P.bb_x = bb_x;
     P.lims = lims;
+    P.sums = sums;
     const size_t runs = lm_bbox_tm_slow_runs(p);
     P.g_stride = (int64_t)runs;
     {

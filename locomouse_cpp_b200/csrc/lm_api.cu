@@ -69,7 +69,7 @@ struct lm_ctx {
         PNG_SCRATCH, PNG_STAGE0, PNG_STAGE1, PNG_OFFS, PNG_STATUS, PNG_HDR, FFV1_REC, FFV1_INIT, FFV1_SOFF, FFV1_SLEN, FFV1_CHAINS,
         FFV1_WORK0, FFV1_WORK1, MJPEG_HDR,
         P1_MINMAX, P1_LUT, P1_STAGE, P1_HIST, P1_PRED, P1_DIFF, P1_BITS0, P1_BITS1, P1_CC, P1_VMAP, P1_VMASK, P1_SLOW, P1_RUNS,
-        P1_LMASK, P1_DISK, P1_BBX, P1_LIMS,
+        P1_LMASK, P1_DISK, P1_BBX, P1_LIMS, P1_SUMS,
         COST_CAND, COST_NCAND, COST_PRIOR, COST_OUT, COST_JC, COST_NNZ, COST_OFFS, COST_IR, COST_PR,
         GUARD_COUNT, NBUF
     };
@@ -133,6 +133,12 @@ struct lm_ctx {
     int last_B = 0;                   // size of the last sub-batch (for lm_debug_fetch)
     int last_slot = 0;
     int64_t last_s0 = 0;
+    // the last chunk of the last pass-1 call (lm_debug_fetch items 4 .. 6): method (LM_P1_*, 0: none), its frames
+    // [p1_s0, p1_s0 + p1_B) of the call, bit-image rows / words per row / width, int32 sums per frame
+    struct {
+        int method = 0, B = 0, rows = 0, wpr = 0, width = 0, nsums = 0;
+        int64_t s0 = 0;
+    } p1;
 };
 
 namespace {
@@ -1348,6 +1354,7 @@ int grow_bufs(lm_ctx *ctx, std::initializer_list<std::pair<int, size_t>> want) {
 // memory, the staging buffer.
 int pass1_scratch(lm_ctx *ctx, int cap, int frames_on_device) {
     using L = lm_ctx;
+    ctx->p1.method = 0;  // the buffers are about to be overwritten: nothing to fetch until this call finishes
     const int64_t fsz = (int64_t)ctx->cfg.vid_rows * ctx->cfg.vid_cols;
     if (int rc = grow_bufs(ctx, {{L::P1_MINMAX, (size_t)(cap + 1) * 2 * sizeof(int32_t)}, {L::P1_LUT, (size_t)(cap + 1) * 256}})) return rc;
     return frames_on_device ? LM_OK : grow(ctx, ctx->buf[L::P1_STAGE], (size_t)cap * fsz);
@@ -1382,6 +1389,22 @@ int pass1_chunk(lm_ctx *ctx, const uint8_t *frames, int frames_on_device, int64_
     }
     return LM_OK;
 }
+
+// The per-frame sums only lm_debug_fetch reads: kept for the last chunk of a call (the only one it can address), so the
+// earlier chunks of a long video skip the stores (measured on a B200: storing every chunk cost pass 1 about 0.7 %).
+int32_t *last_chunk_sums(lm_ctx *ctx, int64_t s0, int cap, int64_t n) { return s0 + cap >= n ? ctx->buf[lm_ctx::P1_SUMS].as<int32_t>() : nullptr; }
+
+// Records the last chunk of a finished pass-1 call of n frames in chunks of `cap` for lm_debug_fetch items 4 .. 6.
+void set_p1(lm_ctx *ctx, int method, int64_t n, int cap, int rows, int wpr, int width, int nsums) {
+    auto &q = ctx->p1;
+    q.method = method;
+    q.s0 = (n - 1) / cap * cap;
+    q.B = (int)(n - q.s0);
+    q.rows = rows;
+    q.wpr = wpr;
+    q.width = width;
+    q.nsums = nsums;
+}
 }  // namespace
 
 int lm_bounding_box_tm_de(lm_ctx *ctx, const uint8_t *frames, int frames_on_device, int64_t n, const lm_bb_de_params *p,
@@ -1408,7 +1431,7 @@ int lm_bounding_box_tm_de(lm_ctx *ctx, const uint8_t *frames, int frames_on_devi
         // call stay on the device until the end: chunks run back to back without a host sync
         if ((rc = grow_bufs(ctx, {{L::P1_PRED, (size_t)cap * 256}, {L::P1_HIST, (size_t)cap * 256 * sizeof(uint32_t)},
                                   {L::P1_DIFF, (size_t)cap * p->side_w * p->side_h}, {L::P1_BBX, (size_t)n * sizeof(double)},
-                                  {L::P1_LIMS, (size_t)n * 2 * sizeof(int32_t)}})))
+                                  {L::P1_LIMS, (size_t)n * 2 * sizeof(int32_t)}, {L::P1_SUMS, (size_t)cap * p->side_w * sizeof(int32_t)}})))
             return rc;
         if ((rc = fold_calib(ctx))) return rc;  // k_prep's vector tier, used by k_bb_hist16
         cudaStream_t st = ctx->stream;
@@ -1419,7 +1442,8 @@ int lm_bounding_box_tm_de(lm_ctx *ctx, const uint8_t *frames, int frames_on_devi
             LmBatch b;
             if ((rc = pass1_chunk(ctx, frames, frames_on_device, s0, B, b))) return rc;
             use_fold(ctx, b);
-            if (lm_launch_bbox_tm_de(b, *p, S[L::P1_HIST].as<uint32_t>(), S[L::P1_PRED].p, d_bbx + s0, d_lims + s0 * 2, st, S[L::P1_DIFF].p) < 0)
+            if (lm_launch_bbox_tm_de(b, *p, S[L::P1_HIST].as<uint32_t>(), S[L::P1_PRED].p, d_bbx + s0, d_lims + s0 * 2, last_chunk_sums(ctx, s0, cap, n), st,
+                                     S[L::P1_DIFF].p) < 0)
                 return fail(ctx, LM_ERR_RUNTIME, "bounding-box launch failed: %s", cudaGetErrorString(cudaGetLastError()));
         }
         if (cudaMemcpyAsync(bb_x_raw, d_bbx, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st) != cudaSuccess)
@@ -1428,6 +1452,7 @@ int lm_bounding_box_tm_de(lm_ctx *ctx, const uint8_t *frames, int frames_on_devi
             return fail(ctx, LM_ERR_RUNTIME, "D2H copy failed");
         if (cudaStreamSynchronize(st) != cudaSuccess)
             return fail(ctx, LM_ERR_RUNTIME, "pass 1 failed on the device: %s", cudaGetErrorString(cudaGetLastError()));
+        set_p1(ctx, LM_P1_TM_DE, n, cap, 0, 0, p->side_w, p->side_w);
         return LM_OK;
     });
 }
@@ -1458,7 +1483,8 @@ int lm_bounding_box_base(lm_ctx *ctx, const uint8_t *frames, int frames_on_devic
         if ((rc = pass1_scratch(ctx, cap, frames_on_device))) return rc;
         if ((rc = grow_bufs(ctx, {{L::P1_BITS0, bits}, {L::P1_BITS1, bits}, {L::P1_CC, (size_t)LM_BBOX_SLOW_SLOTS * 3 * slow * sizeof(int32_t)},
                                   {L::P1_VMAP, (size_t)LM_BBOX_SLOW_SLOTS * slow}, {L::P1_VMASK, (size_t)LM_BBOX_SLOW_SLOTS * slow},
-                                  {L::P1_SLOW, (size_t)cap * 2 * sizeof(int)}, {L::P1_LIMS, (size_t)n * 8 * sizeof(int32_t)}})))
+                                  {L::P1_SLOW, (size_t)cap * 2 * sizeof(int)}, {L::P1_LIMS, (size_t)n * 8 * sizeof(int32_t)},
+                                  {L::P1_SUMS, (size_t)cap * lm_bbox_base_sums(*p) * sizeof(int32_t)}})))
             return rc;
         cudaStream_t st = ctx->stream;
         int32_t *d_lims = S[L::P1_LIMS].as<int32_t>();
@@ -1467,12 +1493,13 @@ int lm_bounding_box_base(lm_ctx *ctx, const uint8_t *frames, int frames_on_devic
             LmBatch b;
             if ((rc = pass1_chunk(ctx, frames, frames_on_device, s0, B, b))) return rc;
             if (lm_launch_bbox_base(b, *p, S[L::P1_BITS0].as<uint32_t>(), S[L::P1_BITS1].as<uint32_t>(), S[L::P1_CC].as<int32_t>(), S[L::P1_VMAP].p,
-                                    S[L::P1_VMASK].p, S[L::P1_SLOW].as<int>(), d_lims + s0 * 8, st) < 0)
+                                    S[L::P1_VMASK].p, S[L::P1_SLOW].as<int>(), d_lims + s0 * 8, last_chunk_sums(ctx, s0, cap, n), st) < 0)
                 return fail(ctx, LM_ERR_RUNTIME, "bounding-box launch failed: %s", cudaGetErrorString(cudaGetLastError()));
         }
         std::vector<int32_t> h_lims((size_t)n * 8);
         CK(cudaMemcpyAsync(h_lims.data(), d_lims, h_lims.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
+        set_p1(ctx, LM_P1_BASE, n, cap, k.n_rows, (k.n_cols + 31) / 32, k.n_cols, lm_bbox_base_sums(*p));
         for (int64_t f = 0; f < n; ++f) {  // computeMouseBox's last lines (class.cpp:981-993) + the caller's offset (628)
             const int32_t *rs = &h_lims[(size_t)f * 8], *rb = rs + 2, *cs = rs + 4, *cb = rs + 6;
             double *o = box + f * 6;
@@ -1529,7 +1556,8 @@ int lm_bounding_box_tm(lm_ctx *ctx, const uint8_t *frames, int frames_on_device,
         if ((rc = grow_bufs(ctx, {{L::P1_HIST, (size_t)cap * 256 * sizeof(uint32_t)}, {L::P1_PRED, (size_t)cap * 256}, {L::P1_BITS0, bits},
                                   {L::P1_BITS1, bits}, {L::P1_SLOW, (size_t)cap * 2 * sizeof(int)},
                                   {L::P1_RUNS, (size_t)cap_tm * lm_bbox_tm_slow_runs(*p) * 14 + 64}, {L::P1_LMASK, 512 * sizeof(uint32_t)},
-                                  {L::P1_DISK, disk}, {L::P1_BBX, (size_t)n * sizeof(double)}, {L::P1_LIMS, (size_t)n * 2 * sizeof(int32_t)}})))
+                                  {L::P1_DISK, disk}, {L::P1_BBX, (size_t)n * sizeof(double)}, {L::P1_LIMS, (size_t)n * 2 * sizeof(int32_t)},
+                                  {L::P1_SUMS, (size_t)cap * p->side_w * sizeof(int32_t)}})))
             return rc;
         cudaStream_t st = ctx->stream;
         double *d_bbx = S[L::P1_BBX].as<double>();
@@ -1541,13 +1569,14 @@ int lm_bounding_box_tm(lm_ctx *ctx, const uint8_t *frames, int frames_on_device,
             if ((rc = pass1_chunk(ctx, frames, frames_on_device, s0, B, b))) return rc;
             rc = lm_launch_bbox_tm(b, *p, S[L::P1_DISK].as<float>(), S[L::P1_HIST].as<uint32_t>(), S[L::P1_PRED].p, S[L::P1_BITS0].as<uint32_t>(),
                                    S[L::P1_BITS1].as<uint32_t>(), S[L::P1_SLOW].as<int>(), S[L::P1_RUNS].as<unsigned char>(), cap_tm,
-                                   S[L::P1_LMASK].as<uint32_t>(), d_bbx + s0, d_lims + s0 * 2, st);
+                                   S[L::P1_LMASK].as<uint32_t>(), d_bbx + s0, d_lims + s0 * 2, last_chunk_sums(ctx, s0, cap, n), st);
             if (rc == -2) return fail(ctx, LM_ERR_INVALID, "side view of %d x %d pixels does not fit the shared-memory bit image", p->side_w, p->side_h);
             if (rc < 0) return fail(ctx, LM_ERR_RUNTIME, "bounding-box launch failed: %s", cudaGetErrorString(cudaGetLastError()));
         }
         CK(cudaMemcpyAsync(bb_x_raw, d_bbx, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st));
         if (lims) CK(cudaMemcpyAsync(lims, d_lims, (size_t)n * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
+        set_p1(ctx, LM_P1_TM, n, cap, p->side_h, (p->side_w + 31) / 32, p->side_w, p->side_w);
         return LM_OK;
     });
 }
@@ -2163,7 +2192,28 @@ int lm_last_timing(const lm_ctx *ctx, float ms[7], int64_t *launches) {
     return LM_OK;
 }
 
+// items 4 .. 6: the last chunk of the last pass-1 call
+static int64_t debug_fetch_p1(lm_ctx *ctx, int what, int64_t frame, void *dst, int64_t dst_bytes, int32_t dims[4]) {
+    const auto &q = ctx->p1;
+    if (!q.method) return fail(ctx, LM_ERR_STATE, "no pass-1 call has finished on this context");
+    const int64_t i = frame - q.s0;
+    if (i < 0 || i >= q.B) return fail(ctx, LM_ERR_INVALID, "frame %lld is not in the last chunk of the last pass-1 call", (long long)frame);
+    if (what != 6 && q.method == LM_P1_TM_DE) return fail(ctx, LM_ERR_INVALID, "lm_bounding_box_tm_de keeps no bit images");
+    int32_t d[4] = {q.rows, q.wpr, q.width, q.method};
+    if (what == 6) d[0] = 1, d[1] = q.nsums;
+    const int64_t bytes = (int64_t)d[0] * d[1] * 4;
+    const auto &b = ctx->buf[what == 4 ? lm_ctx::P1_BITS0 : what == 5 ? lm_ctx::P1_BITS1 : lm_ctx::P1_SUMS];
+    if (dims) memcpy(dims, d, sizeof d);
+    if (!dst || dst_bytes < bytes) return fail(ctx, LM_ERR_INVALID, "debug buffer too small (%lld needed)", (long long)bytes);
+    DeviceGuard guard(ctx->device);
+    cudaError_t e = cudaMemcpyAsync(dst, b.p + i * bytes, (size_t)bytes, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) return fail(ctx, LM_ERR_RUNTIME, "cudaMemcpy: %s", cudaGetErrorString(e));
+    return bytes;
+}
+
 int64_t lm_debug_fetch(lm_ctx *ctx, int what, int64_t frame, void *dst, int64_t dst_bytes, int32_t dims[4]) {
+    if (ctx && what >= 4 && what <= 6) return debug_fetch_p1(ctx, what, frame, dst, dst_bytes, dims);
     if (!ctx || !ctx->Bcap) return LM_ERR_STATE;
     const int64_t i = frame - ctx->last_s0;
     if (i < 0 || i >= ctx->last_B) return fail(ctx, LM_ERR_INVALID, "frame %lld is not in the last sub-batch", (long long)frame);

@@ -149,23 +149,27 @@ int lm_launch_nms(const LmBatch &b, cudaStream_t s);
 // bytes of nms_scratch per list: 8 + 8 + 4 bytes per entry (two key arrays, one link array), 16-byte aligned slices
 __host__ __device__ inline size_t lm_nms_scratch_bytes(int det_cap) { return ((size_t)det_cap * 20 + 15) & ~(size_t)15; }
 int lm_launch_pair(const LmBatch &b, cudaStream_t s);
+// sums (may be null): [B][side_w] per-column counts of the thresholded side view
 int lm_launch_bbox_tm_de(const LmBatch &b, const lm_bb_de_params &p, uint32_t *hist, uint8_t *pred, double *bb_x, int32_t *lims,
-                         cudaStream_t s, uint8_t *diff = nullptr);
+                         int32_t *sums, cudaStream_t s, uint8_t *diff = nullptr);
 
 // pass 1 of the base class (k_bbox_base.cu)
 int lm_launch_bbox_pred(const LmBatch &b, const lm_bb_de_params &p, uint32_t *hist, uint8_t *pred, cudaStream_t s, uint8_t *diff = nullptr);
 // pass 1 of LocoMouse_TM (k_bbox_tm.cu); returns the number of launches, -1 on a launch error, -2 when the side view's bit
-// image does not fit into shared memory
+// image does not fit into shared memory.  sums (may be null): [B][side_w] CV_32S column sums of the filled image.
 size_t lm_bbox_tm_bits_bytes(const lm_bb_tm_params &p, int B);
 size_t lm_bbox_tm_slow_runs(const lm_bb_tm_params &p);
 int lm_launch_bbox_tm(const LmBatch &b, const lm_bb_tm_params &p, const float *d_disk, uint32_t *hist, uint8_t *pred, uint32_t *bits_a,
                       uint32_t *bits_b, int *need_slow, unsigned char *g_runs, int g_slots, uint32_t *level_mask /* 512 words */, double *bb_x, int32_t *lims,
-                      cudaStream_t s);
+                      int32_t *sums, cudaStream_t s);
 size_t lm_bbox_base_bits_bytes(int n_rows, int n_cols, int B);
 size_t lm_bbox_base_slow_ints(const lm_bb_base_params &p);
 constexpr int LM_BBOX_SLOW_SLOTS = 8;
+// sums (may be null): [B][lm_bbox_base_sums(p)] = Row_side[side_w] | Row_bottom[bottom_w] | Col_side[side_h] | Col_bottom[bottom_h], 255 per
+// pixel of each view's largest component
+inline int lm_bbox_base_sums(const lm_bb_base_params &p) { return p.side_w + p.bottom_w + p.side_h + p.bottom_h; }
 int lm_launch_bbox_base(const LmBatch &b, const lm_bb_base_params &p, uint32_t *bits, uint32_t *major, int32_t *cc, uint8_t *vmap, uint8_t *vmask,
-                        int *need_slow, int32_t *lims, cudaStream_t s);
+                        int *need_slow, int32_t *lims, int32_t *sums, cudaStream_t s);
 
 // cost builders (k_cost.cu); all pointers are device memory.  Pairwise: phase 0 = count + scan (fills jc, nnz, offs),
 // phase 1 = fill (ir, pr)
