@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define LM_ABI_VERSION 5  /* 5: lm_bounding_box_tm, and (backward compatible additions) lm_decode_png, lm_decode_ffv1, lm_decode_mjpeg, lm_device_alloc / lm_device_free / lm_device_copy, lm_get_info("ms_decode"), lm_get_info("device_allocs"); 4: lm_bounding_box_base, lm_mouse_box_size; 2: lm_set_option, lm_get_info, lm_debug_nms, lm_bounding_box_tm_de, lm_moving_average; 3: lm_host_alloc / lm_host_free, lm_unary_costs / lm_pairwise_costs, options streams 1..4, screen_layout, screen_priority */
+#define LM_ABI_VERSION 5  /* 5: lm_bounding_box_tm, and (backward compatible additions) lm_decode_png, lm_decode_ffv1, lm_decode_mjpeg, lm_decode_mpeg4, lm_device_alloc / lm_device_free / lm_device_copy, lm_get_info("ms_decode"), lm_get_info("device_allocs"); 4: lm_bounding_box_base, lm_mouse_box_size; 2: lm_set_option, lm_get_info, lm_debug_nms, lm_bounding_box_tm_de, lm_moving_average; 3: lm_host_alloc / lm_host_free, lm_unary_costs / lm_pairwise_costs, options streams 1..4, screen_layout, screen_priority */
 
 /* feature / view indices used in every [2] / [3] array below */
 enum { LM_PAW = 0, LM_SNOUT = 1, LM_TAIL = 2 };
@@ -330,6 +330,18 @@ int lm_decode_ffv1(lm_ctx *ctx, const uint8_t *extradata, int64_t extradata_len,
  * device, the IDCT in parallel over blocks.  LM_ERR_INVALID names the first bad frame and why.  Needs lm_configure only.
  * lm_get_info("ms_decode") covers it. */
 int lm_decode_mjpeg(lm_ctx *ctx, const uint8_t *payload, int payload_on_device, const int64_t *offsets, int64_t n, uint8_t *frames);
+/* MPEG-4 Part 2 video (AVI 'XVID' / 'DIVX' / 'FMP4' / 'MP4V', Matroska V_MPEG4/ISO/SP / ASP, MP4 'mp4v'; what cv2.VideoWriter
+ * writes with 'mp4v' and 'XVID'): payload holds n frames (one VOP each, possibly behind VOS / VOL / GOV headers), payload /
+ * offsets / frames as for lm_decode_png; extradata (may be NULL with length 0) holds the VOL when the container keeps it
+ * out of the frames (MP4 esds DecoderSpecificInfo, Matroska CodecPrivate).  Frame 0 must be an I-VOP; I- and P-VOPs are
+ * decoded (a not-coded VOP has no frame in VideoCapture and is refused; the readers leave it out): rectangular,
+ * progressive, 8-bit, H.263 quantisation, 1MV, half-pel, no resync markers, of the configured size; everything else is
+ * refused (B-VOPs, GMC, quarter-pel, 4MV, interlace, data partitioning, short header, XviD / DivX user data).  The output is channel 0 of the frame cv::VideoCapture delivers through libavcodec's mpeg4 decoder and
+ * libswscale, bit-exact.  Entropy decoding runs one device thread per frame; reconstruction is parallel over macroblocks,
+ * one launch per frame position after each I-VOP.  LM_ERR_INVALID names the first bad frame and why.  Needs lm_configure
+ * only.  lm_get_info("ms_decode") covers it. */
+int lm_decode_mpeg4(lm_ctx *ctx, const uint8_t *extradata, int64_t extradata_len, const uint8_t *payload, int payload_on_device,
+                    const int64_t *offsets, int64_t n, uint8_t *frames);
 int lm_device_alloc(lm_ctx *ctx, void **ptr, size_t bytes);   /* on the context's device, for callers without a CUDA runtime */
 int lm_device_free(lm_ctx *ctx, void *ptr);
 /* Copies `bytes` between two device buffers of the context's device on its stream and returns when the copy is done (a

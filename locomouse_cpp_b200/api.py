@@ -28,6 +28,7 @@ EXPORTS = ("lm_abi_version", "lm_create", "lm_destroy", "lm_last_error", "lm_con
            "lm_debug_fetch", "lm_set_option", "lm_get_info", "lm_debug_nms", "lm_bounding_box_tm_de", "lm_moving_average",
            "lm_host_alloc", "lm_host_free", "lm_unary_costs", "lm_pairwise_costs", "lm_bounding_box_base", "lm_mouse_box_size", "lm_bounding_box_tm",
            "lm_decode_png", "lm_device_alloc", "lm_device_free", "lm_decode_ffv1", "lm_decode_mjpeg",
+           "lm_decode_mpeg4",
            "lm_device_copy")
 
 
@@ -108,6 +109,8 @@ def load_library():
     L.lm_decode_mjpeg.argtypes = [vp, vp, i32, vp, i64, vp]
     L.lm_decode_ffv1.restype = C.c_int
     L.lm_decode_ffv1.argtypes = [vp, vp, i64, vp, i32, vp, i64, vp]
+    L.lm_decode_mpeg4.restype = C.c_int
+    L.lm_decode_mpeg4.argtypes = [vp, vp, i64, vp, i32, vp, i64, vp]
     L.lm_device_alloc.restype = C.c_int
     L.lm_device_alloc.argtypes = [vp, C.POINTER(vp), C.c_size_t]
     L.lm_device_free.restype = C.c_int
@@ -278,6 +281,18 @@ class Detector:
         decoded on the device, bit-exact with cv2.VideoCapture's channel 0 (libavcodec's decoder); payload, offsets and out as
         for decode_png.  A refused or malformed frame raises ValueError naming it and the reason."""
         return self._decode(lambda ptr, on_dev, offs, n, out_ptr: self._L.lm_decode_mjpeg(self._ctx, ptr, on_dev, offs, n, out_ptr),
+                            payload, offsets, out)
+
+    def decode_mpeg4(self, extradata, payload, offsets, out=None):
+        """MPEG-4 Part 2 video frames (cv2.VideoWriter 'mp4v' / 'XVID': AVI chunks, Matroska V_MPEG4/ISO/* or MP4 'mp4v'
+        samples) decoded on the device, bit-exact with cv2.VideoCapture's channel 0 (libavcodec's decoder).  extradata: the VOL
+        the container keeps out of the frames (MP4 DecoderSpecificInfo, Matroska CodecPrivate; b"" when the frames carry it);
+        payload, offsets and out as for decode_png; frame 0 must be an I-VOP.  A refused or malformed frame raises ValueError
+        naming it and the reason."""
+        ex = np.ascontiguousarray(np.frombuffer(bytes(extradata), np.uint8) if isinstance(extradata, (bytes, bytearray)) else extradata,
+                                  dtype=np.uint8).reshape(-1)
+        return self._decode(lambda ptr, on_dev, offs, n, out_ptr: self._L.lm_decode_mpeg4(self._ctx, ex.ctypes.data if ex.size else None, ex.size,
+                                                                                           ptr, on_dev, offs, n, out_ptr),
                             payload, offsets, out)
 
     def _decode(self, call, payload, offsets, out):

@@ -15,6 +15,7 @@
 
 #include "ffv1_format.h"
 #include "mjpeg_format.h"
+#include "mpeg4_format.h"
 #include "lm_internal.h"
 
 namespace {
@@ -62,12 +63,12 @@ struct lm_ctx {
     // Context-lifetime buffers, by role: grow-only (grow()), kept across re-configuration until lm_destroy.  The folded
     // calibration (k_fold_calib: the map with the mirror folded in, the background seen through it, k_prep's run flags) is
     // rebuilt when fold_dirty is set.  lm_decode_ffv1 shares the PNG staging, offset, status and header buffers, lm_decode_mjpeg
-    // the PNG scratch (its coefficients), staging, offset and status buffers; the three
+    // and lm_decode_mpeg4 the PNG scratch (their coefficients), staging, offset and status buffers; the three
     // pass-1 entry points share their scratch, as do the two cost builders.
     enum {
         BKG, CALIB, TMPL, FOLD_CALIB = TMPL + 6, FOLD_BKG, FOLD_RUN,
         PNG_SCRATCH, PNG_STAGE0, PNG_STAGE1, PNG_OFFS, PNG_STATUS, PNG_HDR, FFV1_REC, FFV1_INIT, FFV1_SOFF, FFV1_SLEN, FFV1_CHAINS,
-        FFV1_WORK0, FFV1_WORK1, MJPEG_HDR,
+        FFV1_WORK0, FFV1_WORK1, MJPEG_HDR, MPEG4_VOP, MPEG4_INFO, MPEG4_LINES, MPEG4_PLANES, MPEG4_SEGS,
         P1_MINMAX, P1_LUT, P1_STAGE, P1_HIST, P1_PRED, P1_DIFF, P1_BITS0, P1_BITS1, P1_CC, P1_VMAP, P1_VMASK, P1_SLOW, P1_RUNS,
         P1_LMASK, P1_DISK, P1_BBX, P1_LIMS, P1_SUMS,
         COST_CAND, COST_NCAND, COST_PRIOR, COST_OUT, COST_JC, COST_NNZ, COST_OFFS, COST_IR, COST_PR,
@@ -129,7 +130,7 @@ struct lm_ctx {
     std::vector<float> timeline;     // [sub-batch][9]: ms from the start of the last call to its stage events 0..7 and to the end of the screen kernel
     int64_t launches = 0;
     cudaEvent_t ev_png_copy[2] = {}, ev_png_done[2] = {};
-    float ms_decode = 0.f;            // decode kernels of the last lm_decode_png / lm_decode_ffv1 / lm_decode_mjpeg call
+    float ms_decode = 0.f;            // decode kernels of the last lm_decode_png / lm_decode_ffv1 / lm_decode_mjpeg / lm_decode_mpeg4 call
     int last_B = 0;                   // size of the last sub-batch (for lm_debug_fetch)
     int last_slot = 0;
     int64_t last_s0 = 0;
@@ -1253,7 +1254,7 @@ int lm_get_info(const lm_ctx *ctx, const char *name, double *value) {
         *value = (double)ctx->timeline[(size_t)sub * 10 + q];
         return LM_OK;
     }
-    if (!strcmp(name, "ms_decode")) {  // device time of the decode kernels in the last lm_decode_png / lm_decode_ffv1 / lm_decode_mjpeg call
+    if (!strcmp(name, "ms_decode")) {  // device time of the decode kernels in the last lm_decode_png / ffv1 / mjpeg / mpeg4 call
         *value = (double)ctx->ms_decode;
         return LM_OK;
     }
@@ -2174,6 +2175,164 @@ int decode_mjpeg_impl(lm_ctx *ctx, const uint8_t *payload, int on_dev, const int
 
 int lm_decode_mjpeg(lm_ctx *ctx, const uint8_t *payload, int payload_on_device, const int64_t *offsets, int64_t n, uint8_t *frames) {
     return entry(ctx, [&] { return decode_mjpeg_impl(ctx, payload, payload_on_device, offsets, n, frames); });
+}
+
+// ---- lm_decode_mpeg4 ---------------------------------------------------------------------------------------------------
+namespace {
+int decode_mpeg4_impl(lm_ctx *ctx, const uint8_t *extradata, int64_t extradata_len, const uint8_t *payload, int on_dev, const int64_t *offsets,
+                      int64_t n, uint8_t *frames) {
+    if (!ctx->configured) return fail(ctx, LM_ERR_STATE, "lm_decode_mpeg4 needs lm_configure first");
+    if (n < 0) return fail(ctx, LM_ERR_INVALID, "negative frame count");
+    ctx->ms_decode = 0.f;
+    if (n == 0) return LM_OK;
+    if (!payload || !offsets || !frames || extradata_len < 0 || (extradata_len > 0 && !extradata)) return fail(ctx, LM_ERR_INVALID, "null argument");
+    if (n > INT32_MAX) return fail(ctx, LM_ERR_INVALID, "too many frames in one call");
+    const int rows = ctx->cfg.vid_rows, cols = ctx->cfg.vid_cols;
+    for (int64_t i = 0; i < n; ++i)
+        if (offsets[i] < 0 || offsets[i + 1] < offsets[i]) return fail(ctx, LM_ERR_INVALID, "frame %lld: offsets must not decrease", (long long)i);
+    if (rows > 8191 || cols > 8191) return fail(ctx, LM_ERR_INVALID, "an MPEG-4 frame is at most 8191 x 8191 pixels");
+    mpeg4::Vol vol{};
+    mpeg4::Vop vop0{};
+    if (extradata_len > 0)
+        if (int st = mpeg4::parse(extradata, extradata_len, rows, cols, false, vol, vop0))
+            return fail(ctx, LM_ERR_INVALID, "MPEG-4 extradata: %s", mpeg4::status_text(st));
+    cudaStream_t st = ctx->stream, cp = ctx->copy_stream;
+    auto &B = ctx->buf;
+    using L = lm_ctx;
+    if (int rc = grow(ctx, B[L::PNG_OFFS], (size_t)(n + 1) * sizeof(int64_t))) return rc;
+    if (int rc = grow(ctx, B[L::PNG_STATUS], (size_t)n * sizeof(int32_t))) return rc;
+    if (int rc = grow(ctx, B[L::MPEG4_VOP], (size_t)n * lm_mpeg4_vop_bytes() + lm_mpeg4_vol_bytes())) return rc;
+    int64_t *d_offs = reinterpret_cast<int64_t *>(B[L::PNG_OFFS].p);
+    int32_t *d_status = reinterpret_cast<int32_t *>(B[L::PNG_STATUS].p);
+    uint8_t *d_vop = B[L::MPEG4_VOP].p, *d_vol = d_vop + (size_t)n * lm_mpeg4_vop_bytes();
+    CK(cudaMemcpyAsync(d_offs, offsets, (size_t)(n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+
+    // Every frame's VOP header, in order: parsed here from a host payload, by k_mpeg4_locate from a device payload
+    std::vector<mpeg4::Vop> vops((size_t)n);
+    std::vector<int32_t> status((size_t)n, 0);
+    if (!on_dev) {
+        for (int64_t f = 0; f < n; ++f) {
+            int s = mpeg4::parse(payload + offsets[f], offsets[f + 1] - offsets[f], rows, cols, true, vol, vops[(size_t)f]);
+            if (s == mpeg4::LM_MPEG4_OK && vops[(size_t)f].type == mpeg4::VOP_N) s = mpeg4::LM_MPEG4_NOT_CODED;
+            if (s == mpeg4::LM_MPEG4_OK && f == 0 && vops[0].type != mpeg4::VOP_I) s = mpeg4::LM_MPEG4_FIRST_NOT_I;
+            if (s) return fail(ctx, LM_ERR_INVALID, "frame %lld: %s", (long long)f, mpeg4::status_text(s));
+        }
+        CK(cudaMemcpyAsync(d_vop, vops.data(), (size_t)n * sizeof(mpeg4::Vop), cudaMemcpyHostToDevice, st));
+        CK(cudaMemsetAsync(d_status, 0, (size_t)n * sizeof(int32_t), st));
+    } else {
+        CK(cudaMemcpyAsync(d_vol, &vol, sizeof vol, cudaMemcpyHostToDevice, st));
+        if (lm_launch_mpeg4_locate(payload, d_offs, (int)n, rows, cols, d_vol, !vol.valid, d_vop, d_status, st) < 0)
+            return fail(ctx, LM_ERR_RUNTIME, "MPEG-4 locate launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        CK(cudaMemcpyAsync(vops.data(), d_vop, (size_t)n * sizeof(mpeg4::Vop), cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(status.data(), d_status, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        for (int64_t f = 0; f < n; ++f)
+            if (status[(size_t)f]) return fail(ctx, LM_ERR_INVALID, "frame %lld: %s", (long long)f, mpeg4::status_text(status[(size_t)f]));
+    }
+
+    // Pieces of consecutive frames share the scratch (coefficients, macroblock records, prediction state) and, from the host,
+    // one of two staging buffers: the copy of piece k + 1 (copy stream) overlaps the decode of piece k.  A piece's segments
+    // start at its first frame and at each I-VOP; every segment has two reference planes.
+    const int mbw = (cols + 15) / 16, mbh = (rows + 15) / 16;
+    const int64_t nmb = (int64_t)mbw * mbh, plane = lm_mpeg4_plane_bytes(rows, cols), lines = lm_mpeg4_lines_bytes(cols);
+    const size_t per_frame = (size_t)nmb * (mpeg4::BLOCKS_PER_MB * 64 * sizeof(int16_t) + lm_mpeg4_info_bytes()) + (size_t)lines;
+    const size_t scratch_budget = (size_t)4 << 30, stage_budget = (size_t)2 << 30;
+    constexpr int max_segs = 256;
+    const int64_t max_piece = std::max<int64_t>(1, std::min<int64_t>(on_dev ? 2048 : std::max<int64_t>(512, (n + 3) / 4), scratch_budget / per_frame));
+    struct Piece {
+        int64_t s, e;
+        int seg0, nseg, seg_len;  // its segments: entries seg0 .. seg0 + nseg - 1 of segs
+    };
+    std::vector<Piece> pieces;
+    std::vector<int32_t> segs;  // (first frame in the piece, frames) per segment
+    size_t stage_need = 0;
+    int64_t piece_max = 0;
+    int segs_max = 0;
+    for (int64_t s = 0; s < n;) {
+        Piece P{s, s, (int)(segs.size() / 2), 0, 0};
+        for (int64_t e = s; e < n; ++e) {
+            const bool starts = e == s || vops[(size_t)e].type == mpeg4::VOP_I;
+            if (e > s && (e - s >= max_piece || (starts && P.nseg == max_segs) ||
+                          (!on_dev && (size_t)(offsets[e + 1] - offsets[s]) > stage_budget)))
+                break;
+            if (starts) {
+                segs.push_back((int32_t)(e - s));
+                segs.push_back(0);
+                ++P.nseg;
+            }
+            ++segs.back();
+            P.seg_len = std::max<int>(P.seg_len, segs.back());
+            P.e = e + 1;
+        }
+        pieces.push_back(P);
+        stage_need = std::max(stage_need, (size_t)(offsets[P.e] - offsets[P.s]));
+        piece_max = std::max(piece_max, P.e - P.s);
+        segs_max = std::max(segs_max, P.nseg);
+        s = P.e;
+    }
+    if (int rc = grow(ctx, B[L::PNG_SCRATCH], (size_t)piece_max * nmb * mpeg4::BLOCKS_PER_MB * 64 * sizeof(int16_t))) return rc;
+    if (int rc = grow(ctx, B[L::MPEG4_INFO], (size_t)piece_max * nmb * lm_mpeg4_info_bytes())) return rc;
+    if (int rc = grow(ctx, B[L::MPEG4_LINES], (size_t)piece_max * lines)) return rc;
+    if (int rc = grow(ctx, B[L::MPEG4_PLANES], (size_t)(2 * segs_max + 1) * plane)) return rc;  // + the carried plane
+    if (int rc = grow(ctx, B[L::MPEG4_SEGS], segs.size() * sizeof(int32_t))) return rc;
+    uint8_t *planes = B[L::MPEG4_PLANES].p, *carry = planes + (size_t)2 * segs_max * plane;
+    int32_t *d_segs = reinterpret_cast<int32_t *>(B[L::MPEG4_SEGS].p);
+    CK(cudaMemcpyAsync(d_segs, segs.data(), segs.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    if (!on_dev) {
+        for (int k = 0; k < 2 && k < (int)pieces.size(); ++k)
+            if (int rc = grow(ctx, B[L::PNG_STAGE0 + k], std::max<size_t>(stage_need, 1))) return rc;
+        for (int k = 0; k < 2; ++k) {
+            if (!ctx->ev_png_copy[k]) CK(cudaEventCreateWithFlags(&ctx->ev_png_copy[k], cudaEventDisableTiming));
+            if (!ctx->ev_png_done[k]) CK(cudaEventCreateWithFlags(&ctx->ev_png_done[k], cudaEventDisableTiming));
+        }
+    }
+    struct Events {  // start / end of each piece's decode launches, for ms_decode
+        std::vector<cudaEvent_t> ev;
+        ~Events() {
+            for (cudaEvent_t e : ev) cudaEventDestroy(e);
+        }
+    } T;
+    T.ev.resize(2 * pieces.size());
+    for (auto &e : T.ev) CK(cudaEventCreate(&e));
+    for (size_t k = 0; k < pieces.size(); ++k) {
+        const Piece &P = pieces[k];
+        const uint8_t *src = payload;
+        int64_t base = 0;
+        if (!on_dev) {
+            uint8_t *stg = B[L::PNG_STAGE0 + (k & 1)].p;
+            if (k >= 2) CK(cudaStreamWaitEvent(cp, ctx->ev_png_done[k & 1], 0));  // piece k - 2 no longer reads this buffer
+            CK(cudaMemcpyAsync(stg, payload + offsets[P.s], (size_t)(offsets[P.e] - offsets[P.s]), cudaMemcpyHostToDevice, cp));
+            CK(cudaEventRecord(ctx->ev_png_copy[k & 1], cp));
+            CK(cudaStreamWaitEvent(st, ctx->ev_png_copy[k & 1], 0));
+            src = stg;
+            base = offsets[P.s];
+        }
+        CK(cudaEventRecord(T.ev[2 * k], st));
+        if (lm_launch_mpeg4_decode(src, d_offs + P.s, base, (int)(P.e - P.s), d_vop + P.s * (int64_t)lm_mpeg4_vop_bytes(), rows, cols,
+                                   B[L::MPEG4_INFO].p, B[L::PNG_SCRATCH].as<int16_t>(), B[L::MPEG4_LINES].p, d_segs + 2 * P.seg0, P.nseg,
+                                   P.seg_len, planes, carry, d_status + P.s, frames + P.s * (int64_t)rows * cols, st) < 0)
+            return fail(ctx, LM_ERR_RUNTIME, "MPEG-4 decode launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        // the piece's last frame, which the next piece's first segment may continue
+        const int32_t last_len = segs[(size_t)2 * (P.seg0 + P.nseg - 1) + 1];
+        CK(cudaMemcpyAsync(carry, planes + (size_t)(2 * (P.nseg - 1) + ((last_len - 1) & 1)) * plane, (size_t)plane, cudaMemcpyDeviceToDevice, st));
+        CK(cudaEventRecord(T.ev[2 * k + 1], st));
+        if (!on_dev) CK(cudaEventRecord(ctx->ev_png_done[k & 1], st));
+    }
+    CK(cudaMemcpyAsync(status.data(), d_status, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    for (size_t k = 0; k < pieces.size(); ++k) {
+        float t = 0.f;
+        if (cudaEventElapsedTime(&t, T.ev[2 * k], T.ev[2 * k + 1]) == cudaSuccess) ctx->ms_decode += t;
+    }
+    for (int64_t i = 0; i < n; ++i)
+        if (status[(size_t)i] != mpeg4::LM_MPEG4_OK) return fail(ctx, LM_ERR_INVALID, "frame %lld: %s", (long long)i, mpeg4::status_text(status[(size_t)i]));
+    return LM_OK;
+}
+}  // namespace
+
+int lm_decode_mpeg4(lm_ctx *ctx, const uint8_t *extradata, int64_t extradata_len, const uint8_t *payload, int payload_on_device,
+                    const int64_t *offsets, int64_t n, uint8_t *frames) {
+    return entry(ctx, [&] { return decode_mpeg4_impl(ctx, extradata, extradata_len, payload, payload_on_device, offsets, n, frames); });
 }
 
 int lm_decode_ffv1(lm_ctx *ctx, const uint8_t *extradata, int64_t extradata_len, const uint8_t *payload, int payload_on_device,

@@ -252,6 +252,26 @@ size_t lm_mjpeg_header_bytes();
 int lm_launch_mjpeg_decode(const uint8_t *payload, const int64_t *offs, int64_t base, int n, int rows, int cols, uint8_t *hdr, int16_t *coef,
                            int32_t *status, int32_t *dht0, int first_piece, uint8_t *out, cudaStream_t s);
 
+// MPEG-4 Part 2 decode (k_mpeg4.cu, format in mpeg4_format.h).  Frame j of a launch is payload[offs[j] - base, offs[j + 1] -
+// base) with its VOP header at vop + j * lm_mpeg4_vop_bytes() and its LM_MPEG4_* code in status[j] (0 on entry: headers
+// good); its macroblock records go to info + j * nmb * lm_mpeg4_info_bytes(), its coefficients to coef + j * nmb * 320, its
+// prediction state to lines + j * lm_mpeg4_lines_bytes(cols), its pixels to out + j * rows * cols.  seg: nseg pairs (first
+// frame, frames) of the launch's segments, each reconstructed in the planes 2 s, 2 s + 1 (lm_mpeg4_plane_bytes each); a
+// segment that starts with a P-VOP predicts its first frame from `carry`.  Entropy CTAs take 8 frames and 44 kB of
+// shared lookahead tables.  lm_launch_mpeg4_locate fills vop / status of n frames already on the device (need_vol: *vol is
+// invalid and becomes frame 0's VOL).
+constexpr int LM_MPEG4_FRAMES_PER_CTA = 8;
+size_t lm_mpeg4_vol_bytes();
+size_t lm_mpeg4_vop_bytes();
+size_t lm_mpeg4_info_bytes();
+int64_t lm_mpeg4_lines_bytes(int cols);
+inline int64_t lm_mpeg4_plane_bytes(int rows, int cols) { return (int64_t)((cols + 15) / 16) * ((rows + 15) / 16) * 320; }
+int lm_launch_mpeg4_locate(const uint8_t *payload, const int64_t *offs, int n, int rows, int cols, uint8_t *vol, int need_vol, uint8_t *vop,
+                           int32_t *status, cudaStream_t s);
+int lm_launch_mpeg4_decode(const uint8_t *payload, const int64_t *offs, int64_t base, int n, const uint8_t *vop, int rows, int cols, uint8_t *info,
+                           int16_t *coef, uint8_t *lines, const int32_t *seg, int nseg, int seg_len, uint8_t *planes, const uint8_t *carry,
+                           int32_t *status, uint8_t *out, cudaStream_t s);
+
 // pick the padded kernel-row width the correlation kernel is instantiated for (>= kw), or -1
 int lm_corr_kwp(int kw);
 // dynamic shared memory the correlation kernel needs for a view/template (for capability checks)

@@ -186,7 +186,8 @@ void worker(Shared &S, int dev, lm_ctx *ctx) {
         Load r;
         const auto t0 = clk::now();
         try {
-            m->load(S.E[i].video, S.E[i].bkg, (size_t)S.params.max_resident_bytes, S.params.batch_frames, S.params.decode_mjpeg != 0);
+            m->load(S.E[i].video, S.E[i].bkg, (size_t)S.params.max_resident_bytes, S.params.batch_frames, S.params.decode_mjpeg != 0,
+                    S.params.decode_mpeg4 != 0);
         } catch (const std::invalid_argument &e) {
             r.status = "invalid", r.message = std::string("Invalid inputs: ") + e.what();
         } catch (const std::exception &e) {

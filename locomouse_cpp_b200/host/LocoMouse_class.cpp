@@ -120,6 +120,7 @@ LocoMouse_Parameters::LocoMouse_Parameters(const std::string &config_file_name) 
             else if (key == "batch_frames") batch_frames = std::stoi(val);
             else if (key == "max_resident_bytes") max_resident_bytes = std::stoll(val);
             else if (key == "decode_mjpeg") decode_mjpeg = std::stoi(val);
+            else if (key == "decode_mpeg4") decode_mpeg4 = std::stoi(val);
             else if (key == "fma_mode") fma_mode = std::stoi(val);
             else if (key == "cand_cap") cand_cap = std::stoi(val);
             else if (key == "det_cap") det_cap = std::stoi(val);
@@ -172,6 +173,7 @@ LocoMouse_Parameters::LocoMouse_Parameters(const std::string &config_file_name) 
     if (batch_frames <= 0) throw std::invalid_argument("batch_frames must be positive.");
     if (max_resident_bytes <= 0) throw std::invalid_argument("max_resident_bytes must be positive.");
     if (decode_mjpeg != 0 && decode_mjpeg != 1) throw std::invalid_argument("decode_mjpeg must be 0 or 1.");
+    if (decode_mpeg4 != 0 && decode_mpeg4 != 1) throw std::invalid_argument("decode_mpeg4 must be 0 or 1.");
     if (batch_workers_per_gpu <= 0) throw std::invalid_argument("batch_workers_per_gpu must be positive.");
     if (max_displacement_side < 0) throw std::invalid_argument("max_displacement_side must be non-negative. Was " + std::to_string(max_displacement_side) + ".");
     if (occlusion_grid_spacing_pixels_side <= 0 || occlusion_grid_spacing_pixels_bottom <= 0)
@@ -297,10 +299,11 @@ void LocoMouse::initializePaths(const LocoMouse_ParseInputs &INPUT) {
 }
 
 void LocoMouse_Media::load(const std::string &video_file, const std::string &bkg_file, size_t max_resident_bytes, int batch_frames,
-                           bool decode_mjpeg) {
+                           bool decode_mjpeg, bool decode_mpeg4) {
     // AVI, the reference's input (VideoCapture + extractChannel(0), class.cpp:367-400, 1282-1293), or the LMV1 container
     lmmedia::Options opt;
     opt.decode_mjpeg = decode_mjpeg;
+    opt.decode_mpeg4 = decode_mpeg4;
     index = lmmedia::index_video(video_file, opt);
     n_frames = (unsigned int)index.n;
     rows = index.rows;
@@ -403,7 +406,8 @@ LocoMouse::LocoMouse(LocoMouse_ParseInputs INPUTS) {
     initializePaths(INPUTS);
     LM_PARAMS = LocoMouse_Parameters(CONFIG_FILE);
     OWN_MEDIA.reset(new LocoMouse_Media());
-    OWN_MEDIA->load(VIDEO_FILE, BKG_FILE, (size_t)LM_PARAMS.max_resident_bytes, LM_PARAMS.batch_frames, LM_PARAMS.decode_mjpeg != 0);
+    OWN_MEDIA->load(VIDEO_FILE, BKG_FILE, (size_t)LM_PARAMS.max_resident_bytes, LM_PARAMS.batch_frames, LM_PARAMS.decode_mjpeg != 0,
+                    LM_PARAMS.decode_mpeg4 != 0);
     OWN_POOL.reset(new LocoMouse_WindowPool());
     initializeInputs(*OWN_MEDIA, OWN_POOL.get());
     const int rc = lm_create(&CTX, LM_PARAMS.device);
@@ -489,6 +493,9 @@ void LocoMouse::useWindow(int k, int next) {
             check(lm_decode_png(CTX, MEDIA->data.data(), 0, MEDIA->offsets.data(), n, POOL->decoded.p));
         else if (MEDIA->codec == lmmedia::Codec::mjpeg)
             check(lm_decode_mjpeg(CTX, MEDIA->data.data(), 0, MEDIA->offsets.data(), n, POOL->decoded.p));
+        else if (MEDIA->codec == lmmedia::Codec::mpeg4)  // every window starts at an I-VOP; extradata holds the VOL
+            check(lm_decode_mpeg4(CTX, MEDIA->extradata.data(), (int64_t)MEDIA->extradata.size(), MEDIA->data.data(), 0, MEDIA->offsets.data(), n,
+                                  POOL->decoded.p));
         else
             check(lm_decode_ffv1(CTX, MEDIA->extradata.data(), (int64_t)MEDIA->extradata.size(), MEDIA->data.data(), 0, MEDIA->offsets.data(), n,
                                  POOL->decoded.p));

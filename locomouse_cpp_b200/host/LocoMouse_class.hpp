@@ -92,11 +92,12 @@ struct LocoMouse_Media {
     int window = 0;                     // the window in data / offsets
     PinnedArray<uint8_t> data;          // raw: channel 0 of the window's frames, [count][rows][cols]; coded: its frame chunks
     std::vector<int64_t> offsets;       // coded: frame first + i = data[offsets[i], offsets[i + 1])
-    std::vector<uint8_t> extradata;     // FFV1: the configuration record
+    std::vector<uint8_t> extradata;     // FFV1: the configuration record; MPEG-4: the VOL
     std::vector<uint8_t> bkg;           // rows x cols
     // loadVideo + loadBackground (LocoMouse_class.cpp:367-417): the video's index and its first window (the whole video when
     // it fits in max_resident_bytes); throws std::runtime_error as the reference's constructor does
-    void load(const std::string &video_file, const std::string &bkg_file, size_t max_resident_bytes, int batch_frames, bool decode_mjpeg = false);
+    void load(const std::string &video_file, const std::string &bkg_file, size_t max_resident_bytes, int batch_frames, bool decode_mjpeg = false,
+              bool decode_mpeg4 = false);
     void read_window(int k, PinnedArray<uint8_t> &to, std::vector<int64_t> &to_offsets) const;
 };
 
@@ -164,6 +165,7 @@ public:
     // (a multiple of batch_frames frames), each read on a reader thread while the device works on the one before
     int64_t max_resident_bytes = (int64_t)8 << 30;
     int decode_mjpeg = 0;  // 1: Motion-JPEG video is decoded (bit-exact with libavcodec's decoder, lm_decode_mjpeg), 0: refused
+    int decode_mpeg4 = 0;  // 1: MPEG-4 Part 2 video is decoded (bit-exact with libavcodec's decoder, lm_decode_mpeg4), 0: refused
     int fma_mode = 1;
     int cand_cap = 64, det_cap = 8192, match_cap = 256;
 

@@ -287,6 +287,9 @@ inline Index index_mkv(const std::string &name, const Options &opt) {
         V.extradata = vt->priv;
     } else if (vt->codec == "V_MJPEG" && opt.decode_mjpeg) {
         V.codec = Codec::mjpeg;
+    } else if ((vt->codec == "V_MPEG4/ISO/SP" || vt->codec == "V_MPEG4/ISO/ASP") && opt.decode_mpeg4) {
+        V.codec = Codec::mpeg4;
+        V.extradata = vt->priv;  // the VOL, where the writer put it there
     } else if (vt->codec == "V_MS/VFW/FOURCC") {
         // a BITMAPINFOHEADER, as in an AVI's 'strf'
         const std::vector<uint8_t> &b = vt->priv;
@@ -302,6 +305,10 @@ inline Index index_mkv(const std::string &name, const Options &opt) {
             V.extradata.assign(b.begin() + 40, b.end());
         } else if (opt.decode_mjpeg && (fourcc == cc("MJPG") || fourcc == cc("mjpg"))) {
             V.codec = Codec::mjpeg;
+        } else if (opt.decode_mpeg4 && mpeg4_fourcc(fourcc)) {
+            V.codec = Codec::mpeg4;
+            V.fourcc = fourcc;
+            V.extradata.assign(b.begin() + 40, b.end());
         } else if ((fourcc == cc("Y800") || fourcc == cc("GREY") || fourcc == cc("Y8  ")) && bits == 8) {
             raw = true;
         } else if (fourcc == 0 && (bits == 24 || bits == 32)) {  // BI_RGB: BGR(A), rows top-down as libavformat reads them from Matroska (no AVI bottom-up flip)
@@ -309,7 +316,7 @@ inline Index index_mkv(const std::string &name, const Options &opt) {
             V.grey = false;
             V.bpp = bits / 8;
         } else {
-            outside("'" + fc + "' with " + std::to_string(bits) + " bits per pixel");
+            outside("'" + fc + "' with " + std::to_string(bits) + " bits per pixel" + (mpeg4_fourcc(fourcc) ? mpeg4_opt_in() : ""));
         }
     } else if (vt->codec == "V_UNCOMPRESSED") {
         const std::string cs = vt->has_colour ? detail::fourcc_text(vt->colour) : "";
@@ -324,7 +331,7 @@ inline Index index_mkv(const std::string &name, const Options &opt) {
             outside("uncompressed with ColourSpace '" + cs + "'");
         }
     } else {
-        outside("'" + vt->codec + "'");
+        outside("'" + vt->codec + "'" + (vt->codec.rfind("V_MPEG4/ISO/", 0) == 0 ? mpeg4_opt_in() : ""));
     }
     if ((raw || V.codec == Codec::ffv1) && (V.rows <= 0 || V.cols <= 0)) fail("the video track has no frame size");
     for (const Blk &b : blocks) {
@@ -543,14 +550,18 @@ inline Index index_mov(const std::string &name, const Options &opt) {
     } else if (type == "mp4v") {
         // esds: ES_Descriptor (tag 3) -> DecoderConfigDescriptor (tag 4) -> objectTypeIndication; libavformat maps 0x6D to PNG
         int oti = -1;
+        std::vector<uint8_t> dsi;  // DecoderSpecificInfo (tag 5): an MPEG-4 stream's VOL
         detail::boxes(children, fail, [&](const uint8_t *t, Span b) {
             if (!is(t, "esds") || b.n < 4) return;
-            size_t p = 4;
+            size_t p = 4, len = 0;
             auto descr = [&](int tag) -> bool {
                 if (p >= b.n || b.d[p] != tag) return false;
                 ++p;
-                for (int k = 0; k < 4 && p < b.n; ++k)
+                len = 0;
+                for (int k = 0; k < 4 && p < b.n; ++k) {
+                    len = (len << 7) | (b.d[p] & 0x7F);
                     if (!(b.d[p++] & 0x80)) break;
+                }
                 return true;
             };
             if (!descr(3) || p + 3 > b.n) return;
@@ -559,10 +570,15 @@ inline Index index_mov(const std::string &name, const Options &opt) {
             if (flags & 0x80) p += 2;
             if ((flags & 0x40) && p < b.n) p += 1 + b.d[p];
             if (flags & 0x20) p += 2;
-            if (descr(4) && p < b.n) oti = b.d[p];
+            if (descr(4) && p < b.n) {
+                oti = b.d[p];
+                p += 13;  // objectTypeIndication, streamType, bufferSizeDB, maxBitrate, avgBitrate
+                if (descr(5)) dsi.assign(b.d + p, b.d + std::min<size_t>(b.n, p + len));
+            }
         });
         if (oti == 0x6C && opt.decode_mjpeg) V.codec = Codec::mjpeg;  // libavformat: 0x6C is MJPEG
-        else if (oti != 0x6D) outside("'mp4v' with object type " + std::to_string(oti) + " (not PNG)");
+        else if (oti == 0x20 && opt.decode_mpeg4) V.codec = Codec::mpeg4, V.extradata = dsi;  // 0x20: MPEG-4 Part 2 visual
+        else if (oti != 0x6D) outside("'mp4v' with object type " + std::to_string(oti) + " (not PNG)" + (oti == 0x20 ? mpeg4_opt_in() : ""));
         else V.codec = Codec::png;
     } else if (type == "raw ") {
         outside("'raw ' with depth " + std::to_string(depth));

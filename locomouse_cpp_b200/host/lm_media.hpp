@@ -6,7 +6,9 @@
 // (channel 0 = blue, as extractChannel takes it).  PNG-coded streams ('MPNG' / 'png ', lossless, what cv2.VideoWriter writes
 // with those fourccs) are not decoded here: their frame chunks -- each a complete PNG file -- are returned as one payload with
 // offsets, for lm_decode_png to decode on the device.  Motion-JPEG streams are returned the same way for lm_decode_mjpeg when
-// the caller opts in (Options::decode_mjpeg); otherwise they are refused like every other lossy codec.  FFV1-coded streams ('FFV1', lossless, version 3 as libavcodec writes
+// the caller opts in (Options::decode_mjpeg), and MPEG-4 Part 2 streams for lm_decode_mpeg4 with their VOL as extradata
+// (Options::decode_mpeg4; every frame's VOP header is checked and its I-VOP bit recorded); otherwise they are refused like
+// every other lossy codec.  FFV1-coded streams ('FFV1', lossless, version 3 as libavcodec writes
 // it) are returned the same way, with the configuration record from 'strf' as extradata, for lm_decode_ffv1; the record is
 // checked here (ffv1_format.h) and so is every frame's keyframe bit.  Other compressed or YUV-planar streams need a decoder
 // that is outside this library: they are refused with a message that says so.  The same frames in Matroska and QuickTime / MP4
@@ -31,6 +33,7 @@
 
 #include "../csrc/ffv1_format.h"
 #include "../csrc/mjpeg_format.h"
+#include "../csrc/mpeg4_format.h"
 
 namespace lmmedia {
 
@@ -64,13 +67,28 @@ inline bool is_png(const std::string &name) {
 // into memory the upload runs from at the PCIe rate).  Without one they go to Video::frames / a malloc'ed Video::payload.
 using Dest = std::function<uint8_t *(size_t bytes)>;
 
-enum class Codec { raw, png, ffv1, mjpeg };
+enum class Codec { raw, png, ffv1, mjpeg, mpeg4 };
 
 // What the index functions accept beyond the lossless codecs.  Motion-JPEG is decoded bit-exactly with the libavcodec
 // decoder OpenCV calls (mjpeg_format.h), so a caller whose reference reads it through another decoder turns it on knowingly.
 struct Options {
     bool decode_mjpeg = false;  // Motion-JPEG (AVI 'MJPG', Matroska V_MJPEG, QuickTime 'jpeg', MP4 object type 0x6C) instead of a refusal
+    // MPEG-4 Part 2 (AVI 'XVID' / 'DIVX' / 'DX50' / 'FMP4' / 'MP4V', Matroska V_MPEG4/ISO/SP and ASP, MP4 'mp4v' object type
+    // 0x20) decoded bit-exactly with libavcodec's mpeg4 decoder (mpeg4_format.h), instead of a refusal
+    bool decode_mpeg4 = false;
 };
+
+// AVI / VfW fourccs of MPEG-4 Part 2 video
+inline bool mpeg4_fourcc(uint32_t fourcc) {
+    for (const char *s : {"XVID", "xvid", "DIVX", "DX50", "FMP4", "MP4V", "mp4v"})
+        if (fourcc == le32(reinterpret_cast<const uint8_t *>(s))) return true;
+    return false;
+}
+
+// What a refusal of MPEG-4 Part 2 video without decode_mpeg4 adds
+inline const char *mpeg4_opt_in() {
+    return " MPEG-4 Part 2 video is decoded with the configuration key decode_mpeg4: 1 (bit-exact with libavcodec's decoder).";
+}
 
 struct Video {
     int n = 0, rows = 0, cols = 0;
@@ -137,6 +155,9 @@ struct Index {
     std::vector<std::pair<int64_t, uint32_t>> coded;
     std::vector<uint8_t> keyframe, extradata;
     int mjpeg_dht = -1;  // Motion-JPEG: the tables frame 0's DHT defines (mjpeg::Header::dht_mask), which every frame must match
+    // MPEG-4 Part 2: the container's fourcc (AVI / VfW, 0 elsewhere); keyframe holds every frame's I-VOP bit and extradata
+    // the VOL (the container's, or the headers in front of frame 0's VOP)
+    uint32_t fourcc = 0;
 };
 
 namespace detail {
@@ -151,6 +172,73 @@ struct File {
     int64_t size() { return fseeko(f, 0, SEEK_END) == 0 ? (int64_t)ftello(f) : -1; }
 };
 }  // namespace detail
+
+// Every MPEG-4 frame's headers up to its VOP header: the VOL (the container's extradata, else the frame's) is the one
+// mpeg4_format.h decodes, of the container's size, the same in every frame; the VOP is I or P, frame 0 an I-VOP.  A
+// not-coded VOP is left out, as a zero-size AVI chunk is: libavcodec returns no frame for it, so VideoCapture reads one frame
+// less.  Records the I-VOP bits (windows end before one) and, where the container has no extradata, the headers in front of
+// frame 0's VOP as extradata, so that every window's decode has the VOL.  libavcodec decodes an 'XVID' or 'DIVX' stream without
+// libavcodec's user data with XviD's IDCT and bug workarounds, so such streams are refused.
+inline void index_mpeg4(Index &V, detail::File &file) {
+    auto fail = [&](const std::string &why) -> void { throw std::runtime_error("Video file " + V.name + ": " + why); };
+    if (V.rows <= 0 || V.cols <= 0) fail("the video track has no frame size");
+    mpeg4::Vol vol{};
+    mpeg4::Vop vop{};
+    if (!V.extradata.empty())
+        if (int st = mpeg4::parse(V.extradata.data(), (int64_t)V.extradata.size(), V.rows, V.cols, false, vol, vop))
+            fail(std::string("MPEG-4 extradata: ") + mpeg4::status_text(st));
+    auto lavc = [](const uint8_t *d, size_t n) {
+        for (size_t i = 0; i + 8 <= n; ++i)
+            if (d[i] == 0 && d[i + 1] == 0 && d[i + 2] == 1 && d[i + 3] == 0xB2 && !std::memcmp(d + i + 4, "Lavc", 4)) return true;
+        return false;
+    };
+    bool lavc_seen = lavc(V.extradata.data(), V.extradata.size());
+    V.keyframe.clear();
+    std::vector<std::pair<int64_t, uint32_t>> kept;
+    std::vector<uint8_t> d;
+    for (size_t i = 0; i < V.coded.size(); ++i) {
+        // the headers in front of the VOP's macroblocks: a prefix of the frame, or all of it when the prefix ends too soon
+        const std::string where = "Video file " + V.name + ", frame " + std::to_string(i);
+        size_t len = std::min<size_t>(V.coded[i].second, 512);
+        for (int pass = 0; pass < 2; ++pass) {
+            d.resize(len);
+            if (!file.seek(V.coded[i].first) || !file.read(d.data(), len)) fail("truncated frame");
+            const int st = mpeg4::parse(d.data(), (int64_t)len, V.rows, V.cols, true, vol, vop);
+            if (st == mpeg4::LM_MPEG4_OK && (vop.data_bit >> 3) + 8 <= (int64_t)len) break;
+            if (len == V.coded[i].second) {
+                if (st) throw std::runtime_error(where + ": " + mpeg4::status_text(st));
+                break;
+            }
+            len = V.coded[i].second;
+        }
+        if (vop.type == mpeg4::VOP_N) continue;
+        V.keyframe.push_back(vop.type == mpeg4::VOP_I);
+        kept.push_back(V.coded[i]);
+        if (kept.size() == 1) {
+            if (vop.type != mpeg4::VOP_I) throw std::runtime_error(where + ": " + mpeg4::status_text(mpeg4::LM_MPEG4_FIRST_NOT_I));
+            lavc_seen = lavc_seen || lavc(d.data(), d.size());
+            if (V.extradata.empty()) {  // everything in front of the VOP start code
+                const int64_t vop_at = (vop.data_bit >> 3);
+                int64_t e = 0;
+                for (int64_t p = 0; p + 3 < vop_at; ++p)
+                    if (d[p] == 0 && d[p + 1] == 0 && d[p + 2] == 1 && d[p + 3] == 0xB6) e = p;
+                V.extradata.assign(d.begin(), d.begin() + e);
+            }
+        }
+    }
+    V.coded.swap(kept);
+    V.n = (int)V.coded.size();
+    auto cc = [](const char *s) { return le32(reinterpret_cast<const uint8_t *>(s)); };
+    uint32_t upper = V.fourcc;  // libavcodec compares the codec tag upper-cased (ff_toupper4)
+    for (int k = 0; k < 4; ++k) {
+        const uint32_t c = (upper >> (8 * k)) & 255;
+        if (c >= 'a' && c <= 'z') upper -= (uint32_t)('a' - 'A') << (8 * k);
+    }
+    if ((upper == cc("XVID") || upper == cc("DIVX")) && !lavc_seen)
+        fail("'" + std::string(reinterpret_cast<const char *>(&V.fourcc), 4) +
+             "' MPEG-4 video without libavcodec's user data: libavcodec decodes it with XviD's IDCT and bug workarounds, which "
+             "are not restated here");
+}
 
 // The checks every container's index ends with (index_avi, index_mkv, index_mov), once V.n, the codec, the chunks and the
 // record are set: every chunk lies inside the file, also the bytes behind the image area that are not read; an FFV1 stream's
@@ -177,6 +265,8 @@ inline void finish_index(Index &V, detail::File &file) {
         }
         if (!V.keyframe.empty() && !V.keyframe[0])
             throw std::runtime_error("Video file " + V.name + ", frame 0: the first FFV1 frame is not a keyframe");
+    } else if (V.codec == Codec::mpeg4) {
+        index_mpeg4(V, file);
     } else {
         V.extradata.clear();
     }
@@ -269,9 +359,11 @@ inline Index index_avi(const std::string &name, const Options &opt = {}) {
         const bool rgb = fourcc == 0 || fourcc == cc("DIB ") || fourcc == cc("RGB ") || fourcc == cc("RAW ");
         const bool png = fourcc == cc("MPNG") || fourcc == cc("png ");
         const bool mjpg = opt.decode_mjpeg && (fourcc == cc("MJPG") || fourcc == cc("mjpg"));
-        if (png || mjpg || fourcc == cc("FFV1")) {
+        const bool mp4v = opt.decode_mpeg4 && mpeg4_fourcc(fourcc);
+        if (png || mjpg || mp4v || fourcc == cc("FFV1")) {
             if (size == 0) continue;
-            V.codec = png ? Codec::png : mjpg ? Codec::mjpeg : Codec::ffv1;
+            V.codec = png ? Codec::png : mjpg ? Codec::mjpeg : mp4v ? Codec::mpeg4 : Codec::ffv1;
+            V.fourcc = fourcc;
             const off_t at = ftello(f);
             V.coded.emplace_back((int64_t)at, size);
             if (!skip((uint64_t)size + (size & 1))) fail("truncated frame");
@@ -280,7 +372,8 @@ inline Index index_avi(const std::string &name, const Options &opt = {}) {
         if (!(grey && bits == 8) && !(rgb && (bits == 8 || bits == 24 || bits == 32))) {
             char fc[5] = {(char)(fourcc & 255), (char)((fourcc >> 8) & 255), (char)((fourcc >> 16) & 255), (char)((fourcc >> 24) & 255), 0};
             fail(std::string("stream 0 is '") + fc + "' with " + std::to_string(bits) +
-                 " bits per pixel; only uncompressed 8-bit grey (Y800) and BI_RGB 8 / 24 / 32-bit frames are read here. " + outside_this_library());
+                 " bits per pixel; only uncompressed 8-bit grey (Y800) and BI_RGB 8 / 24 / 32-bit frames are read here. " + outside_this_library() +
+                 (mpeg4_fourcc(fourcc) ? mpeg4_opt_in() : ""));
         }
         if (size == 0) continue;  // dropped frame: VideoCapture repeats nothing, it simply has one frame less
         const size_t tight = (size_t)V.cols * (bits / 8), padded = (tight + 3) & ~(size_t)3;

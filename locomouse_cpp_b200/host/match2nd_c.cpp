@@ -308,6 +308,116 @@ int lmh_decode_mjpeg(const uint8_t *payload, const int64_t *offsets, int64_t n, 
     }
     return 0;
 }
+// MPEG-4 Part 2 video (any container index_video reads) with decode_mpeg4 on: dims = {n, rows, cols, payload bytes,
+// extradata bytes}; with payload / offsets / extradata NULL only the dimensions are returned; ivop (optional, n bytes):
+// each frame's I-VOP bit.  0 ok, 1 error (msg filled)
+int lmh_read_video_mpeg4(const char *path, int64_t *dims, uint8_t *payload, int64_t *offsets, uint8_t *extradata, uint8_t *ivop, char *msg,
+                         int msg_cap) {
+    try {
+        lmmedia::Options opt;
+        opt.decode_mpeg4 = true;
+        const lmmedia::Index ix = lmmedia::index_video(path, opt);
+        const lmmedia::Video V = lmmedia::read_frames(ix, 0, ix.n);
+        if (V.codec != lmmedia::Codec::mpeg4) throw std::runtime_error(std::string("Video file ") + path + ": not an MPEG-4 Part 2 stream");
+        dims[0] = V.n;
+        dims[1] = V.rows;
+        dims[2] = V.cols;
+        dims[3] = V.offsets.back();
+        dims[4] = (int64_t)ix.extradata.size();
+        if (payload) std::memcpy(payload, V.payload.get(), (size_t)V.offsets.back());
+        if (offsets) std::memcpy(offsets, V.offsets.data(), V.offsets.size() * sizeof(int64_t));
+        if (extradata && !ix.extradata.empty()) std::memcpy(extradata, ix.extradata.data(), ix.extradata.size());
+        if (ivop) std::memcpy(ivop, ix.keyframe.data(), ix.keyframe.size());
+        return 0;
+    } catch (const std::exception &e) {
+        if (msg && msg_cap > 0) std::snprintf(msg, (size_t)msg_cap, "%s", e.what());
+        return 1;
+    }
+}
+// mpeg4_format.h run serially on the CPU: the header parse, macroblock decode and reconstruction that k_mpeg4.cu runs on the
+// device, for the CPU tests.  out: [n][rows][cols].  0 ok, 1 error (msg names the first bad frame and why)
+int lmh_decode_mpeg4(const uint8_t *extradata, int64_t extradata_len, const uint8_t *payload, const int64_t *offsets, int64_t n, int rows,
+                     int cols, uint8_t *out, char *msg, int msg_cap) {
+    static const std::unique_ptr<mpeg4::Tables> tables = [] {
+        std::unique_ptr<mpeg4::Tables> t(new mpeg4::Tables);
+        mpeg4::build_tables(*t, 0, 0, 1);
+        mpeg4::build_tables(*t, 1, 0, 1);
+        return t;
+    }();
+    const int mbw = (cols + 15) / 16, mbh = (rows + 15) / 16;
+    auto fail = [&](int64_t f, int st) {
+        std::snprintf(msg, (size_t)msg_cap, "frame %lld: %s", (long long)f, mpeg4::status_text(st));
+        return 1;
+    };
+    mpeg4::Vol vol{};
+    mpeg4::Vop vop{};
+    if (extradata_len > 0)
+        if (int st = mpeg4::parse(extradata, extradata_len, rows, cols, false, vol, vop)) {
+            std::snprintf(msg, (size_t)msg_cap, "extradata: %s", mpeg4::status_text(st));
+            return 1;
+        }
+    std::vector<uint8_t> ref((size_t)mbw * mbh * 320), cur(ref.size()), lines((size_t)mpeg4::lines_bytes(mbw));
+    std::vector<mpeg4::MbInfo> info((size_t)mbw * mbh);
+    std::vector<int16_t> coef((size_t)mbw * mbh * mpeg4::BLOCKS_PER_MB * 64);
+    for (int64_t f = 0; f < n; ++f) {
+        const uint8_t *fr = payload + offsets[f];
+        const int64_t len = offsets[f + 1] - offsets[f];
+        int st = mpeg4::parse(fr, len, rows, cols, true, vol, vop);
+        if (st == mpeg4::LM_MPEG4_OK && vop.type == mpeg4::VOP_N) st = mpeg4::LM_MPEG4_NOT_CODED;
+        if (st == mpeg4::LM_MPEG4_OK && f == 0 && vop.type != mpeg4::VOP_I) st = mpeg4::LM_MPEG4_FIRST_NOT_I;
+        if (st == mpeg4::LM_MPEG4_OK)
+            st = mpeg4::decode_vop(
+                *tables, vop, mbw, mbh, fr, len, mpeg4::lines_at(lines.data(), mbw), [&](int mb, const mpeg4::MbInfo &mi) { info[(size_t)mb] = mi; },
+                [&](int mb, int b, const int16_t *blk) { std::memcpy(&coef[((size_t)mb * mpeg4::BLOCKS_PER_MB + b) * 64], blk, 64 * sizeof(int16_t)); });
+        if (st != mpeg4::LM_MPEG4_OK) return fail(f, st);
+        uint8_t *cy = cur.data(), *cc = cy + (size_t)mbw * mbh * 256;
+        for (int my = 0; my < mbh; ++my)
+            for (int mx = 0; mx < mbw; ++mx)
+                mpeg4::build_mb(mbw, mbh, mx, my, info[(size_t)(my * mbw + mx)], &coef[(size_t)(my * mbw + mx) * mpeg4::BLOCKS_PER_MB * 64],
+                                vop.rounding, ref.data(), ref.data() + (size_t)mbw * mbh * 256, cy, cc);
+        for (int my = 0; my < mbh; ++my)
+            for (int mx = 0; mx < mbw; ++mx) mpeg4::put_mb(mbw, mx, my, cy, cc, rows, cols, out + f * (int64_t)rows * cols);
+        std::swap(ref, cur);
+    }
+    return 0;
+}
+// lmh_plan_windows with decode_mpeg4 on: MPEG-4 windows end before an I-VOP
+int lmh_plan_windows_mpeg4(const char *path, int64_t max_bytes, int batch_frames, int32_t *starts, int cap, char *msg, int msg_cap) {
+    try {
+        lmmedia::Options opt;
+        opt.decode_mpeg4 = true;
+        const lmmedia::Index ix = lmmedia::index_video(path, opt);
+        const int W = lmmedia::window_frames((size_t)max_bytes, (size_t)ix.rows * ix.cols, batch_frames);
+        const std::vector<int> s = lmmedia::plan_windows(ix.n, W, ix.keyframe);
+        for (size_t i = 0; i < s.size() && (int)i < cap; ++i) starts[i] = s[i];
+        return (int)s.size() - 1;
+    } catch (const std::exception &e) {
+        if (msg && msg_cap > 0) std::snprintf(msg, (size_t)msg_cap, "%s", e.what());
+        return -1;
+    }
+}
+// mpeg4::blue for every (Y, Cb): table[Y * 256 + Cb]
+void lmh_mpeg4_blue(uint8_t *table) {
+    for (int y = 0; y < 256; ++y)
+        for (int c = 0; c < 256; ++c) table[y * 256 + c] = mpeg4::blue(y, c);
+}
+// (last, run, level) of TCOEF symbol s (< 102) of the intra (intra = 1) or inter table, for the tests' encoder
+void lmh_mpeg4_tcoef_event(int intra, int s, int32_t *lrl) {
+    int last, run, level;
+    mpeg4::tcoef_event(intra, s, last, run, level);
+    lrl[0] = last, lrl[1] = run, lrl[2] = level;
+}
+// {code, length} of every symbol of VLC table t of mpeg4_format.h (codes, lens: mpeg4::count(t) entries); returns the count
+int lmh_mpeg4_vlc(int t, int32_t *codes, int32_t *lens) {
+    if (t < 0 || t >= mpeg4::T_COUNT) return 0;
+    for (int s = 0; s < mpeg4::count(t); ++s) {
+        int c, l;
+        mpeg4::code(t, s, c, l);
+        codes[s] = c;
+        lens[s] = l;
+    }
+    return mpeg4::count(t);
+}
 int lmh_read_png(const char *path, int32_t *dims, uint8_t *out, char *msg, int msg_cap) {
     try {
         const lmmedia::Image I = lmmedia::read_png_gray(path);
